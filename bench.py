@@ -70,7 +70,7 @@ BYTES_PROJ_BWD_PER_VISIBLE = 48.0 + 12.0 + 192.0  # packed grads + conic + SH re
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the measured window (>= 1)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--gaussians", type=int, default=1_000_000)
@@ -91,7 +91,64 @@ def parse_args():
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--repeats", type=int, default=5, help="extra timed windows of K steps after the measured one (spread: median / p10 / p90)")
     ap.add_argument("--no-multi-gpu-check", action="store_true", help="N>1: skip the N-rank == 1-rank gradient / replica-identity check")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last step of the measured window returned (loss, gradients, radii, render, alphas, strategy "
+                         "statistics; a fixed seeded sample of Gaussians and pixels) as DIR/<name>.npy, for comparing two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
+    return args
+
+
+# ------------------------------------------------------------------------------------------------
+# --dump-outputs
+# ------------------------------------------------------------------------------------------------
+DUMP_GAUSSIANS = 1 << 16  # sampled Gaussians: 59 gradient floats + radii + 3 statistics each
+DUMP_PIXELS = 1 << 18     # sampled pixels: render (4) + alpha
+DUMP_MAX_BYTES = 64 << 20
+
+
+def _dump_sample(n: int, k: int, seed: int):
+    """Sorted indices of a fixed seeded sample of k of range(n) (all of them when n <= k)."""
+    import torch
+
+    if n <= k:
+        return torch.arange(n)
+    return torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:k].sort().values
+
+
+def collect_outputs(out, stats) -> dict:
+    """Host copies (float32, float64 indices) of a fused step's StepOutput + the strategy statistics, sampled so that
+    the whole dump stays under DUMP_MAX_BYTES.  Same arguments -> same inputs -> same sample."""
+    import torch
+
+    N = out.radii.shape[-1]
+    gi = _dump_sample(N, DUMP_GAUSSIANS, seed=1)
+    gd = gi.to(out.radii.device)
+    res = {"loss": out.loss.float().cpu(), "gaussian_index": gi.double()}
+    for k, g in out.grads.items():
+        res["grad_" + k] = g.reshape(N, -1).index_select(0, gd).float().cpu()
+    res["radii"] = out.radii.reshape(-1, N).index_select(1, gd).float().cpu()
+    res["strategy_stats"] = stats.index_select(1, gd).float().cpu()  # grad2d, count, radii_max
+    C, H, W = out.render.shape[:3]
+    pi = _dump_sample(C * H * W, DUMP_PIXELS, seed=2)
+    pd = pi.to(out.render.device)
+    res["pixel_index"] = pi.double()
+    res["render"] = out.render.reshape(C * H * W, -1).index_select(0, pd).float().cpu()
+    res["alphas"] = out.alphas.reshape(C * H * W).index_select(0, pd).float().cpu()
+    total = sum(t.numel() * t.element_size() for t in res.values())
+    assert total <= DUMP_MAX_BYTES, f"output dump of {total} B exceeds {DUMP_MAX_BYTES} B"
+    return res
+
+
+def write_outputs(dump_dir: str, res: dict) -> None:
+    import numpy as np
+
+    os.makedirs(dump_dir, exist_ok=True)
+    for k, t in res.items():
+        np.save(os.path.join(dump_dir, k + ".npy"), t.numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -537,11 +594,17 @@ def main_ours(args):
     for _ in range(W_):
         out = step()
     barrier()
+    last = {}
+
+    def measured_step():
+        last["out"] = step()
+
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
     # THE measurement (contract): exactly K steps, one window
-    ms_total = timed_window(step, K)
+    ms_total = timed_window(measured_step, K)
+    dumped = collect_outputs(last["out"], stats) if args.dump_outputs and rank == 0 else None
     ms_per_step = ms_total / K
     value = world * width * height / (ms_per_step * 1e-3) / 1e6
     # R more windows of K steps: run-to-run spread (median / p10 / p90), and enough wall time for >= 10 clock samples
@@ -788,6 +851,8 @@ def main_ours(args):
             line["cpu_baseline"] = {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample", "cpu_seconds_spent", "steps")}
         else:
             line["cpu_baseline"] = None
+        if dumped is not None:
+            write_outputs(args.dump_outputs, dumped)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()

@@ -1,12 +1,13 @@
 """GPU: the CUDA path against outputs of the REFERENCE'S OWN CODE.
 
 1. `test_cuda_paths_match_reference_model_fixture`: tests/golden/ref_model_*.npz hold what the unmodified
-   /root/reference/qed_splatter/model.py (QEDSplatterModel.get_outputs + get_loss_dict + backward, model.py:73-118,
-   199-321) produced in the build container (scripts/make_golden_reference_model.py; rasterization = the CPU oracle).
+   qed_splatter/model.py (QEDSplatterModel.get_outputs + get_loss_dict + backward, model.py:73-118, 199-321) produced
+   (scripts/make_golden_reference_model.py; rasterization = the CPU oracle).
    Both product paths must reproduce them on the B200: the gsplat-surface `rasterization()` + `depth_supervised_loss()`
-   and the fused `FusedSplatStep.step()` (folded activations, fused loss, `mask`).
-2. `test_unmodified_reference_model_runs_on_the_cuda_shim`: when the reference package travelled to this machine
-   (baseline/_ref, see tests/reference_model.py) the UNMODIFIED model.py itself runs on the GPU with
+   and the fused `FusedSplatStep.step()` (folded activations, fused loss, `mask`); the get_viewmat kernel must
+   reproduce the viewmat model.py built.
+2. `test_unmodified_reference_model_runs_on_the_cuda_shim`: when the reference package is available
+   (see tests/reference_model.py) the UNMODIFIED model.py itself runs on the GPU with
    `from gsplat.rendering import rasterization` resolved to the product's shim, and must give the same outputs, loss dict
    and parameter gradients -- with and without batch["mask"], and `info["means2d"]` must behave as gsplat's strategy
    expects (.grad after retain_grad(), .absgrad)."""
@@ -93,7 +94,20 @@ def test_cuda_paths_match_reference_model_fixture(cuda, name):
     _check_grads(fused, z, "FusedSplatStep")
 
 
-@pytest.mark.skipif(rm.reference_root() is None, reason="reference package not on this machine (baseline/_ref not built)")
+@pytest.mark.parametrize("name", CASES)
+def test_get_viewmat_kernel_matches_reference_model_fixture(cuda, name):
+    """The one-launch get_viewmat kernel on the model's camera against the viewmat the reference's own function built
+    (model.py:22-38, stored in the fixture): rotation block and last row exact, translation to 1 ulp of the sum."""
+    from qed_splatter_b200 import get_viewmat
+
+    z = np.load(os.path.join(GOLDEN, name + ".npz"))
+    ref_vm = torch.from_numpy(z["viewmat"])
+    got_vm = get_viewmat(torch.from_numpy(z["c2w"]).to(cuda)).cpu()
+    assert torch.equal(got_vm[:, :3, :3], ref_vm[:, :3, :3]) and torch.equal(got_vm[:, 3], ref_vm[:, 3])
+    torch.testing.assert_close(got_vm, ref_vm, rtol=0, atol=2e-6)
+
+
+@pytest.mark.skipif(rm.reference_root() is None, reason="reference package not available (see tests/reference_model.py)")
 @pytest.mark.parametrize("name", CASES)
 def test_unmodified_reference_model_runs_on_the_cuda_shim(cuda, name):
     z, s, cam, step, mask = _load(name)
@@ -102,7 +116,7 @@ def test_unmodified_reference_model_runs_on_the_cuda_shim(cuda, name):
         model = rm.build_model(mod, s, cuda, step=step)
         model.train()
         camera = rm.make_camera(s, cam, cuda)
-        out = model.get_outputs(camera)  # /root/reference/qed_splatter/model.py:199-321, unmodified
+        out = model.get_outputs(camera)  # qed_splatter/model.py:199-321, unmodified
         batch = {"image": s.gt_rgb[cam].to(cuda), "depth_image": s.gt_depth[cam].to(cuda)}
         if mask is not None:
             batch["mask"] = mask.to(cuda)
@@ -122,7 +136,7 @@ def test_unmodified_reference_model_runs_on_the_cuda_shim(cuda, name):
         assert model.info["width"] == s.width and model.info["n_cameras"] == 1
 
 
-@pytest.mark.skipif(rm.reference_root() is None, reason="reference package not on this machine (baseline/_ref not built)")
+@pytest.mark.skipif(rm.reference_root() is None, reason="reference package not available (see tests/reference_model.py)")
 def test_reference_model_with_get_viewmat_rebound_to_the_kernel(cuda):
     """Row a1: `qed_splatter.model.get_viewmat = qed_splatter_b200.get_viewmat` (INTEGRATION.md 2b) -- the unmodified model
     then builds its viewmat (model.py:246) with the one-launch kernel; the kernel must agree with the reference's own

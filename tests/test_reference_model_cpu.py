@@ -3,15 +3,20 @@
 `QEDSplatterModel.get_outputs` + `get_loss_dict` are executed from the reference package with `gsplat` resolved to the
 CPU oracle's rasterization; the result must equal the oracle-only formulation of the same step
 (oracle.get_viewmat <- model.py:22-38, composite_and_fill <- :295-306, depth_l1_loss(mask) <- :87-116), i.e. these
-restatements are pinned by reference-held code, with and without `batch["mask"]`.  Skipped when no reference package
-is available (the driver's container has /root/reference; the GPU box gets baseline/_ref)."""
+restatements are pinned by reference-held code, with and without `batch["mask"]`.  Those tests skip when no reference
+package is available (tests/reference_model.py); the stored outputs of the same step of the reference
+(tests/golden/ref_model_*.npz, scripts/make_golden_reference_model.py) pin the restatement without it."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
 from qed_splatter_b200.scenes import scene_s0
 import reference_model as rm
 
-pytestmark = pytest.mark.skipif(rm.reference_root() is None, reason="reference package not available")
+needs_reference = pytest.mark.skipif(rm.reference_root() is None, reason="reference package not available (see tests/reference_model.py)")
+GOLDEN = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _batch(s, cam, mask):
@@ -21,6 +26,7 @@ def _batch(s, cam, mask):
     return b
 
 
+@needs_reference
 @pytest.mark.parametrize("mask_kind,down", [(None, 1), ("float", 1), ("bool", 1), (None, 2)])
 def test_reference_model_lines_equal_oracle_restatement(mask_kind, down):
     s = scene_s0(N=1500, C=2, size=48)
@@ -55,6 +61,36 @@ def test_reference_model_lines_equal_oracle_restatement(mask_kind, down):
         torch.testing.assert_close(got_grads[k], gref.grad, rtol=1e-5, atol=1e-9, msg=lambda m: f"{k}: {m}")
 
 
+@pytest.mark.parametrize("name", ["ref_model_plain", "ref_model_mask", "ref_model_boolmask_sh1"])
+def test_oracle_restatement_matches_reference_model_fixture(name):
+    """The oracle-only formulation of the step reproduces what the unmodified model.py computed (stored fixture):
+    viewmat (model.py:22-38, also the data side's pinned float32 restatement), radii, outputs, loss terms, gradients."""
+    import oracle
+    from oracle import pointcloud as opc
+
+    z = np.load(os.path.join(GOLDEN, name + ".npz"))
+    s = scene_s0(N=int(z["scene_N"]), C=int(z["scene_C"]), size=int(z["scene_size"]), seed=int(z["scene_seed"]))
+    cam, step, kind = int(z["cam"]), int(z["step"]), str(z["mask_kind"])
+    mask = None
+    if kind != "None":
+        mask = torch.rand(s.height, s.width, 1, generator=torch.Generator().manual_seed(5)) > 0.3
+        mask = mask.float() if kind == "float" else mask
+    c2w = torch.from_numpy(z["c2w"])
+    assert torch.equal(c2w, rm.c2w_from_viewmat(s.viewmats[cam:cam + 1]))
+    assert torch.equal(oracle.get_viewmat(c2w), torch.from_numpy(z["viewmat"]))
+    assert np.array_equal(opc.get_viewmat_pinned(z["c2w"]), z["viewmat"])
+    out, loss, leaves = rm.oracle_reference_step(s, cam, c2w, torch.from_numpy(z["background"]), step=step, mask=mask)
+    sum(loss.values()).backward()
+    assert torch.equal(out["info"]["radii"][0], torch.from_numpy(z["radii"]))
+    for k in ("rgb", "depth", "accumulation"):
+        assert torch.equal(out[k].detach(), torch.from_numpy(z[k])), k
+    for k in ("main_loss", "depth_loss"):
+        assert float(loss[k]) == float(z[k]), k
+    for k, v in leaves.items():
+        assert torch.equal(v.grad, torch.from_numpy(z["grad_" + k])), f"grad {k}"
+
+
+@needs_reference
 def test_reference_model_eval_path_and_empty_depth_mask():
     """Eval render (model.py:213-214, 256-257, 313-314) and the all-invalid depth branch (model.py:111-114)."""
     s = scene_s0(N=800, C=1, size=40)

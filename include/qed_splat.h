@@ -104,6 +104,26 @@ int qed_project_bwd(int C, int N, const float* means, const float* quats, const 
                     float* v_means, float* v_quats, float* v_scales, float* v_opacities,
                     float* v_colors_in, qed_stream_t stream);
 
+/* qed_project_bwd that also returns the gradient with respect to the camera poses (gsplat's v_viewmats; splatfacto's
+ * camera optimizer, whose poses enter through qed_splatter/model.py:212,246).
+ *  Same arguments and outputs as qed_project_bwd, plus
+ *  v_viewmats[C,4,4] (overwritten): d loss / d viewmats over every visible (view, Gaussian): the camera-space mean
+ *      (p = W mu + t), the camera-space covariance (W Sigma W^T, incl. the antialiasing compensation) and, with SH colours,
+ *      the view direction mu - campos with campos = -W^-1 t (general inverse).  Row 3 is zero.
+ *  workspace: device memory of at least qed_project_bwd_pose_workspace_bytes(C, N) bytes, 16-byte aligned (per-warp partial
+ *      sums; may be NULL when N == 0).
+ *  Deterministic: no atomics; partials are summed in a fixed order in float64.  C <= 1024 as for qed_project_bwd. */
+size_t qed_project_bwd_pose_workspace_bytes(int C, int N);
+int qed_project_bwd_pose(int C, int N, const float* means, const float* quats, const float* scales,
+                         const float* opacities, int activations, const float* colors_in, int K, int sh_degree,
+                         int colors_per_camera, const float* viewmats, const float* Ks, int width, int height,
+                         float eps2d, int calc_compensations, int n_color, int append_depth,
+                         const int32_t* radii, const float* conics, const float* compensations,
+                         const float* v_means2d, const float* v_depths, const float* v_conics,
+                         const float* v_colors, const float* v_opacities_cn, const float* packed_grads,
+                         float* v_means, float* v_quats, float* v_scales, float* v_opacities,
+                         float* v_colors_in, float* v_viewmats, void* workspace, size_t workspace_bytes, qed_stream_t stream);
+
 /* Pack separate arrays into the compositor's geom record (op-level entry for callers that did not
  * come through qed_project_fwd, e.g. gsplat-style rasterize_to_pixels(means2d, conics, ..)). */
 int qed_pack_geom(int CN, const float* means2d, const float* conics, const float* opacities,
@@ -297,6 +317,11 @@ int qed_arena_gather(int64_t n_new, const int32_t* src, const uint8_t* fresh, co
  * -> gsplat world-to-camera viewmats [C,4,4]: flip the y and z columns of R, analytic rigid inverse [R^T | -R^T T].
  * Called once per step by the model (model.py:246) on the optimised camera pose. */
 int qed_viewmat_from_c2w(int C, int rows, const float* camera_to_worlds, float* viewmats, qed_stream_t stream);
+/* Backward of qed_viewmat_from_c2w: v_viewmats [C,4,4] -> v_camera_to_worlds [C, rows, 4] (overwritten; row 3 of a 4-row
+ * input gets zero, row 3 of v_viewmats is ignored).  With Rf = c2w[:3,:3] diag(1,-1,-1), T = c2w[:3,3]:
+ * v_Rf = v_rot^T - T v_trans^T, v_T = -Rf v_trans, v_c2w[:3,:3] = v_Rf diag(1,-1,-1), v_c2w[:3,3] = v_T. */
+int qed_viewmat_from_c2w_bwd(int C, int rows, const float* camera_to_worlds, const float* v_viewmats, float* v_camera_to_worlds,
+                             qed_stream_t stream);
 
 /* qed_splatter/create_init_pointcloud.py:148-196 `backproject_frame` (Open3D PointCloud.create_from_depth_image, :176-185):
  * depth [height,width] float32 or raw uint16 (depth_is_u16), metres = value * depth_unit_scale (float32 product, :165);

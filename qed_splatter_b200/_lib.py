@@ -26,6 +26,9 @@ SIGNATURES = {
                                 P, P, P, P, P, P, P, P, P, P, P]),
     "qed_project_bwd": (c_int, [c_int, c_int, P, P, P, P, c_int, P, c_int, c_int, c_int, P, P, c_int, c_int,
                                 c_float, c_int, c_int, c_int, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P]),
+    "qed_project_bwd_pose_workspace_bytes": (c_size_t, [c_int, c_int]),
+    "qed_project_bwd_pose": (c_int, [c_int, c_int, P, P, P, P, c_int, P, c_int, c_int, c_int, P, P, c_int, c_int,
+                                     c_float, c_int, c_int, c_int, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, P, c_size_t, P]),
     "qed_pack_geom": (c_int, [c_int, P, P, P, P, P, P]),
     "qed_isect_count": (c_int, [c_int, c_int, P, P, c_int, c_int, c_int, P, P]),
     "qed_isect_scan_workspace_bytes": (c_size_t, [c_int64]),
@@ -57,6 +60,7 @@ SIGNATURES = {
     "qed_comm_allreduce_f32": (c_int, [P, P, P, c_int, c_int, c_int64, c_int64, ctypes.c_uint32, c_int, P]),
     "qed_arena_gather": (c_int, [c_int64, P, P, P, P, P, P, P, P, P, P, P, P, P, P]),
     "qed_viewmat_from_c2w": (c_int, [c_int, c_int, P, P, P]),
+    "qed_viewmat_from_c2w_bwd": (c_int, [c_int, c_int, P, P, P, P]),
     "qed_backproject_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "qed_backproject_depth": (c_int, [c_int, c_int, P, c_int, c_double, c_float, c_int, P, P, P, P, P, c_size_t, P]),
     "qed_voxel_downsample_workspace_bytes": (c_size_t, [c_int64]),

@@ -42,7 +42,30 @@ struct ProjBwdParams {
     float4* xch_peer[16];          // else: its unicast address on every rank
     int xch_world, xch_slot0, xch_total_slots;
     float xch_tag;
+    // camera pose gradient (POSE, see qed_project_bwd_pose): per-warp partial sums of the 15 per-view values
+    // {v_W (9, row-major), v_t (3), sum of the SH direction gradient (3), 0}, 4 float4 at (c * warps + warp) * 4
+    float4* pose_ws;
 };
+
+constexpr int kPoseVals = 15;
+
+// Sums the 15 per-view pose values of the warp's 32 Gaussians (butterfly: a fixed order, every lane ends with the same
+// bits) and stores them as the warp's partial of view c.  The values live in shared memory, [kPoseVals][kProjBwdThreads],
+// each thread touching only its own column (registers would spill in the degree-3 kernels); the column is cleared for
+// the next view.  Every lane of the warp must call it at the same point.
+__device__ __forceinline__ void pose_flush(const ProjBwdParams& p, int c, float* pose_s) {
+    float* dst = reinterpret_cast<float*>(p.pose_ws + ((int64_t)c * gridDim.x * (kProjBwdThreads / 32) + blockIdx.x * (kProjBwdThreads / 32) +
+                                                       (threadIdx.x >> 5)) * 4);
+#pragma unroll
+    for (int k = 0; k < kPoseVals; ++k) {
+        float v = pose_s[k * kProjBwdThreads + threadIdx.x];
+        pose_s[k * kProjBwdThreads + threadIdx.x] = 0.0f;
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+        if ((threadIdx.x & 31) == 0) dst[k] = v;
+    }
+    if ((threadIdx.x & 31) == 0) dst[kPoseVals] = 0.0f;
+}
 
 __device__ __forceinline__ void xch_store(const ProjBwdParams& p, int64_t i, float4 v) {
     if (p.xch_mc) {
@@ -163,7 +186,12 @@ __device__ __forceinline__ void quat_to_rotmat(float qw, float qx, float qy, flo
 // views, so it overwrites the staged coefficient row in place: half the shared memory, and with it 5 resident blocks per SM
 // instead of 4 (the kernel is latency-bound: 35 % issue-active at 16 warps per SM).  ONE = resident blocks asked of ptxas (5: 96
 // registers, 6: 80 registers).
-template <int DEG, bool VEC, bool XCH = false, int ONE = 0>
+// POSE (not with XCH): also the gradient with respect to each view's world-to-camera matrix [W | t].  For every visible
+// (view, Gaussian) the values below are already in registers: the camera-space mean gradient v_p, the camera-space
+// covariance gradient vSc with A = W Sigma, and the SH direction gradient v_d.  v_W += v_p mu^T + 2 vSc A, v_t += v_p,
+// and sum v_d is kept for the camera-position term, which pose_finish_kernel applies once per view.  Per-warp partials
+// (pose_flush) at the end for ONE, after every view otherwise: the view loop then runs in every lane of the warp.
+template <int DEG, bool VEC, bool XCH = false, int ONE = 0, bool POSE = false>
 __global__ void __launch_bounds__(kProjBwdThreads, ONE ? ONE : 4) project_bwd_kernel(const ProjBwdParams p) {
     extern __shared__ float4 smem4[];
     pdl_enter();
@@ -171,7 +199,8 @@ __global__ void __launch_bounds__(kProjBwdThreads, ONE ? ONE : 4) project_bwd_ke
     CamB* cams = reinterpret_cast<CamB*>(smem4);
     constexpr int DG = DEG < 0 ? 0 : DEG;
     using Sh = ShShapeB<DG>;
-    float4* coefbuf = smem4 + nC * (kCamFloatsB / 4);
+    float* pose_s = reinterpret_cast<float*>(smem4 + nC * (kCamFloatsB / 4));  // POSE: [kPoseVals][kProjBwdThreads]
+    float4* coefbuf = smem4 + nC * (kCamFloatsB / 4) + (POSE ? kPoseVals * kProjBwdThreads / 4 : 0);
     float4* vcoefbuf = ONE ? coefbuf : coefbuf + kProjBwdThreads * Sh::kStrideVec;
 
     for (int c = threadIdx.x; c < nC; c += kProjBwdThreads) load_camera_b(p.viewmats + c * 16, p.Ks + c * 9, p.width, p.height, cams[c]);
@@ -291,15 +320,21 @@ __global__ void __launch_bounds__(kProjBwdThreads, ONE ? ONE : 4) project_bwd_ke
 
     float vS00 = 0, vS01 = 0, vS02 = 0, vS11 = 0, vS12 = 0, vS22 = 0;  // full symmetric matrix gradient (off-diag = one side)
     float vm0 = 0, vm1 = 0, vm2 = 0, vopac = 0;
+    constexpr bool kWarpViews = POSE && !ONE;  // every lane runs the view loop (a warp reduction per view)
+    if (POSE) {
+#pragma unroll
+        for (int k = 0; k < kPoseVals; ++k) pose_s[k * kProjBwdThreads + threadIdx.x] = 0.0f;
+    }
 
-    if (in_range && anyvis) {
+    if (kWarpViews || (in_range && anyvis)) {
         int rad_c = rad0;
         for (int c = 0; c < nC; ++c) {
+            if (kWarpViews && c > 0) pose_flush(p, c - 1, pose_s);
             const int64_t idx = (int64_t)c * p.N + n;
             const bool vis = rad_c > 0;
             const float4 r0 = pf0, r1 = pf1, r2 = pf2;
             const float ca = pfa, cb = pfb, cc = pfc;  // conic of the blurred covariance (stored by the forward)
-            if (c + 1 < nC) {  // next view: radius, upstream gradients, conic
+            if (c + 1 < nC && (!kWarpViews || in_range)) {  // next view: radius, upstream gradients, conic
                 const int64_t nx = idx + p.N;
                 rad_c = p.radii[nx];
                 if (rad_c > 0) {
@@ -427,6 +462,18 @@ __global__ void __launch_bounds__(kProjBwdThreads, ONE ? ONE : 4) project_bwd_ke
             } else {
                 vz += cam.fy * ty * rz3 * vJ12;
             }
+            if (POSE) {  // p = W mu + t and Sc = W Sigma W^T (vSc symmetric): v_W = v_p mu^T + 2 vSc A, v_t = v_p
+                const float vp[3] = {vx, vy, vz}, mu[3] = {m0, m1, m2};
+                const float vS[9] = {vSc00, vSc01, vSc02, vSc01, vSc11, vSc12, vSc02, vSc12, vSc22};
+                float* ps = pose_s + threadIdx.x;
+#pragma unroll
+                for (int i = 0; i < 3; ++i) {
+#pragma unroll
+                    for (int j = 0; j < 3; ++j)
+                        ps[(i * 3 + j) * kProjBwdThreads] = vp[i] * mu[j] + 2.0f * (vS[i * 3] * A[j] + vS[i * 3 + 1] * A[3 + j] + vS[i * 3 + 2] * A[6 + j]);
+                    ps[(9 + i) * kProjBwdThreads] = vp[i];
+                }
+            }
             // ---- back to world: v_mu = W^T v_p ; vSigma = W^T vSc W ----
             vm0 += W[0] * vx + W[3] * vy + W[6] * vz;
             vm1 += W[1] * vx + W[4] * vy + W[7] * vz;
@@ -535,13 +582,20 @@ __global__ void __launch_bounds__(kProjBwdThreads, ONE ? ONE : 4) project_bwd_ke
                     float vux, vuy, vuz;
                     sh_bases_vjp<DG>(ux, uy, uz, vb, vux, vuy, vuz);
                     float dotp = vux * ux + vuy * uy + vuz * uz;
-                    vm0 += (vux - dotp * ux) * rdn;
-                    vm1 += (vuy - dotp * uy) * rdn;
-                    vm2 += (vuz - dotp * uz) * rdn;
+                    const float vdx = (vux - dotp * ux) * rdn, vdy = (vuy - dotp * uy) * rdn, vdz = (vuz - dotp * uz) * rdn;
+                    vm0 += vdx;
+                    vm1 += vdy;
+                    vm2 += vdz;
+                    if (POSE) {  // d = mu - campos: the view's campos gets -sum v_d (pose_finish_kernel)
+                        pose_s[12 * kProjBwdThreads + threadIdx.x] = vdx;
+                        pose_s[13 * kProjBwdThreads + threadIdx.x] = vdy;
+                        pose_s[14 * kProjBwdThreads + threadIdx.x] = vdz;
+                    }
                 }
             }
         }
     }
+    if (POSE) pose_flush(p, nC - 1, pose_s);  // ONE: the only view; else the last one
 
     if (in_range) {
         // ---- Sigma = M M^T ; M = R diag(s) ----
@@ -629,16 +683,103 @@ __global__ void __launch_bounds__(kProjBwdThreads, ONE ? ONE : 4) project_bwd_ke
     }
 }
 
-template <int DEG, bool VEC, bool XCH = false, int ONE = 0>
+template <int DEG, bool VEC, bool XCH = false, int ONE = 0, bool POSE = false>
 static int launch_project_bwd(const ProjBwdParams& p, cudaStream_t stream) {
     using Sh = ShShapeB<(DEG < 0 ? 0 : DEG)>;
-    size_t smem = (size_t)p.C * kCamFloatsB * 4;
+    size_t smem = (size_t)p.C * kCamFloatsB * 4 + (POSE ? (size_t)kPoseVals * kProjBwdThreads * 4 : 0);
     if (DEG >= 0 && p.n_color > 0) smem += (size_t)((XCH || ONE) ? 1 : 2) * kProjBwdThreads * Sh::kStrideVec * 16;
-    auto kern = project_bwd_kernel<DEG, VEC, XCH, ONE>;
+    auto kern = project_bwd_kernel<DEG, VEC, XCH, ONE, POSE>;
     if (smem > 48 * 1024) QED_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int blocks = (p.N + kProjBwdThreads - 1) / kProjBwdThreads;
     QED_CUDA_TRY(launch_pdl(kern, dim3(blocks), dim3(kProjBwdThreads), smem, stream, p));
     return QED_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// Pose gradient, second pass: one block per view sums the per-warp partials of project_bwd_kernel<POSE> in a fixed order
+// (float64), then applies the camera-position term of the SH direction.  campos = -W^-1 t with the GENERAL inverse (what
+// the oracle's adjugate form and gsplat differentiate; it equals W^T only for an exactly orthonormal W), d = mu - campos:
+//   g = W^-T sum_n v_d,   v_t += g,   v_W += g campos^T.
+// v_viewmats[c] is overwritten; its row 3 is zero.
+// ------------------------------------------------------------------------------------------------
+constexpr int kPoseFinishThreads = 256;
+
+__global__ void __launch_bounds__(kPoseFinishThreads) pose_finish_kernel(int warps, const float4* __restrict__ ws,
+                                                                         const float* __restrict__ viewmats, float* __restrict__ v_viewmats) {
+    __shared__ double part[kPoseFinishThreads / 32][kPoseVals];
+    pdl_enter();
+    const int c = blockIdx.x;
+    double acc[kPoseVals];
+#pragma unroll
+    for (int k = 0; k < kPoseVals; ++k) acc[k] = 0.0;
+    for (int w = threadIdx.x; w < warps; w += kPoseFinishThreads) {
+        const float4* r = ws + ((int64_t)c * warps + w) * 4;
+        const float4 a = r[0], b = r[1], d = r[2], e = r[3];
+        const float v[kPoseVals] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, d.x, d.y, d.z, d.w, e.x, e.y, e.z};
+#pragma unroll
+        for (int k = 0; k < kPoseVals; ++k) acc[k] += (double)v[k];
+    }
+#pragma unroll
+    for (int k = 0; k < kPoseVals; ++k) {
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) acc[k] += __shfl_xor_sync(0xffffffffu, acc[k], off);
+    }
+    if ((threadIdx.x & 31) == 0) {
+#pragma unroll
+        for (int k = 0; k < kPoseVals; ++k) part[threadIdx.x >> 5][k] = acc[k];
+    }
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    double s[kPoseVals];
+    for (int k = 0; k < kPoseVals; ++k) {
+        s[k] = part[0][k];
+        for (int w = 1; w < kPoseFinishThreads / 32; ++w) s[k] += part[w][k];
+    }
+    const float* V = viewmats + (int64_t)c * 16;
+    double vW[9], vt[3];
+    for (int k = 0; k < 9; ++k) vW[k] = s[k];
+    for (int i = 0; i < 3; ++i) vt[i] = s[9 + i];
+    if (s[12] != 0.0 || s[13] != 0.0 || s[14] != 0.0) {
+        double a[3][3], t[3];
+        for (int i = 0; i < 3; ++i) {
+            for (int j = 0; j < 3; ++j) a[i][j] = V[i * 4 + j];
+            t[i] = V[i * 4 + 3];
+        }
+        // inverse = adjugate / det, the cofactors of load_camera_b
+        double inv[3][3];
+        inv[0][0] = a[1][1] * a[2][2] - a[1][2] * a[2][1];
+        inv[0][1] = a[0][2] * a[2][1] - a[0][1] * a[2][2];
+        inv[0][2] = a[0][1] * a[1][2] - a[0][2] * a[1][1];
+        inv[1][0] = a[1][2] * a[2][0] - a[1][0] * a[2][2];
+        inv[1][1] = a[0][0] * a[2][2] - a[0][2] * a[2][0];
+        inv[1][2] = a[0][2] * a[1][0] - a[0][0] * a[1][2];
+        inv[2][0] = a[1][0] * a[2][1] - a[1][1] * a[2][0];
+        inv[2][1] = a[0][1] * a[2][0] - a[0][0] * a[2][1];
+        inv[2][2] = a[0][0] * a[1][1] - a[0][1] * a[1][0];
+        const double rdet = 1.0 / (a[0][0] * inv[0][0] + a[0][1] * inv[1][0] + a[0][2] * inv[2][0]);
+        for (int i = 0; i < 3; ++i)
+            for (int j = 0; j < 3; ++j) inv[i][j] *= rdet;
+        double campos[3], g[3];
+        for (int i = 0; i < 3; ++i) campos[i] = -(inv[i][0] * t[0] + inv[i][1] * t[1] + inv[i][2] * t[2]);
+        for (int i = 0; i < 3; ++i) g[i] = inv[0][i] * s[12] + inv[1][i] * s[13] + inv[2][i] * s[14];  // W^-T sum v_d
+        for (int i = 0; i < 3; ++i) {
+            vt[i] += g[i];
+            for (int j = 0; j < 3; ++j) vW[i * 3 + j] += g[i] * campos[j];
+        }
+    }
+    float* out = v_viewmats + (int64_t)c * 16;
+    for (int i = 0; i < 3; ++i) {
+        for (int j = 0; j < 3; ++j) out[i * 4 + j] = (float)vW[i * 3 + j];
+        out[i * 4 + 3] = (float)vt[i];
+    }
+    for (int j = 12; j < 16; ++j) out[j] = 0.0f;
+}
+
+// bytes of the per-warp partials of qed_project_bwd_pose
+static size_t pose_workspace_bytes(int C, int N) {
+    if (C <= 0 || N <= 0) return 0;
+    const size_t warps = (size_t)((N + kProjBwdThreads - 1) / kProjBwdThreads) * (kProjBwdThreads / 32);
+    return (size_t)C * warps * 4 * sizeof(float4);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -730,6 +871,25 @@ extern "C" int qed_debug_set_project_bwd_one(int blocks) {  // 0 = off, 5 / 6 = 
     return old;
 }
 
+template <bool POSE>
+static int dispatch_project_bwd(const ProjBwdParams& p, bool vec_ok, cudaStream_t stream) {
+    switch (p.sh_degree) {
+        case 0: return vec_ok ? launch_project_bwd<0, true, false, 0, POSE>(p, stream) : launch_project_bwd<0, false, false, 0, POSE>(p, stream);
+        case 1: return vec_ok ? launch_project_bwd<1, true, false, 0, POSE>(p, stream) : launch_project_bwd<1, false, false, 0, POSE>(p, stream);
+        case 2: return vec_ok ? launch_project_bwd<2, true, false, 0, POSE>(p, stream) : launch_project_bwd<2, false, false, 0, POSE>(p, stream);
+        case 3:
+            if constexpr (POSE) {  // 4 resident blocks (128 registers): at 5 or 6 the pose variant spills
+                if (vec_ok && p.C == 1 && g_projbwd_one) return launch_project_bwd<3, true, false, 4, true>(p, stream);
+            } else {
+                if (vec_ok && p.C == 1 && g_projbwd_one == 6) return launch_project_bwd<3, true, false, 6>(p, stream);
+                if (vec_ok && p.C == 1 && g_projbwd_one) return launch_project_bwd<3, true, false, 5>(p, stream);
+            }
+            return vec_ok ? launch_project_bwd<3, true, false, 0, POSE>(p, stream) : launch_project_bwd<3, false, false, 0, POSE>(p, stream);
+        default: return launch_project_bwd<-1, false, false, 0, POSE>(p, stream);
+    }
+}
+
+// v_viewmats != NULL: the POSE variant, with pose_ws = pose_workspace_bytes(C, N) of per-warp partials (not with xch)
 static int project_bwd_impl(int C, int N, const float* means, const float* quats, const float* scales,
                             const float* opacities, int activations, const float* colors_in, int K, int sh_degree,
                             int colors_per_camera, const float* viewmats, const float* Ks, int width, int height,
@@ -738,10 +898,13 @@ static int project_bwd_impl(int C, int N, const float* means, const float* quats
                             const float* v_means2d, const float* v_depths, const float* v_conics,
                             const float* v_colors, const float* v_opacities_cn, const float* packed_grads,
                             float* v_means, float* v_quats, float* v_scales, float* v_opacities,
-                            float* v_colors_in, const ProjBwdParams* xch, cudaStream_t stream) {
+                            float* v_colors_in, const ProjBwdParams* xch, float* v_viewmats, float4* pose_ws,
+                            cudaStream_t stream) {
     if (C < 0 || N < 0) return QED_ERR_BAD_ARG;
     if (!(n_color == 0 || n_color == 3) || !(append_depth == 0 || append_depth == 1)) return QED_ERR_BAD_ARG;
+    if (v_viewmats && C > 0 && N == 0) QED_CUDA_TRY(cudaMemsetAsync(v_viewmats, 0, (size_t)C * 16 * sizeof(float), stream));
     if (C == 0 || N == 0) return QED_OK;
+    if (v_viewmats && (xch || !pose_ws)) return QED_ERR_BAD_ARG;
     if (C > 1024) return QED_ERR_UNSUPPORTED;
     if (!means || !quats || !scales || !viewmats || !Ks || !radii || !conics || !v_means || !v_quats || !v_scales)
         return QED_ERR_BAD_ARG;
@@ -802,16 +965,13 @@ static int project_bwd_impl(int C, int N, const float* means, const float* quats
         size_t bytes = sh_degree < 0 ? (size_t)(colors_per_camera ? (size_t)C * N : (size_t)N) * 3 * 4 : (size_t)N * K * 3 * 4;
         QED_CUDA_TRY(cudaMemsetAsync(v_colors_in, 0, bytes, stream));
     }
-    switch (sh_degree) {
-        case 0: return vec_ok ? launch_project_bwd<0, true>(p, stream) : launch_project_bwd<0, false>(p, stream);
-        case 1: return vec_ok ? launch_project_bwd<1, true>(p, stream) : launch_project_bwd<1, false>(p, stream);
-        case 2: return vec_ok ? launch_project_bwd<2, true>(p, stream) : launch_project_bwd<2, false>(p, stream);
-        case 3:
-            if (vec_ok && p.C == 1 && g_projbwd_one == 6) return launch_project_bwd<3, true, false, 6>(p, stream);
-            if (vec_ok && p.C == 1 && g_projbwd_one) return launch_project_bwd<3, true, false, 5>(p, stream);
-            return vec_ok ? launch_project_bwd<3, true>(p, stream) : launch_project_bwd<3, false>(p, stream);
-        default: return launch_project_bwd<-1, false>(p, stream);
-    }
+    if (!v_viewmats) return dispatch_project_bwd<false>(p, vec_ok, stream);
+    p.pose_ws = pose_ws;
+    const int rc = dispatch_project_bwd<true>(p, vec_ok, stream);
+    if (rc != QED_OK) return rc;
+    const int warps = ((N + kProjBwdThreads - 1) / kProjBwdThreads) * (kProjBwdThreads / 32);
+    QED_CUDA_TRY(launch_pdl(pose_finish_kernel, dim3(C), dim3(kPoseFinishThreads), 0, stream, warps, (const float4*)pose_ws, viewmats, v_viewmats));
+    return QED_OK;
 }
 
 extern "C" int qed_project_bwd(int C, int N, const float* means, const float* quats, const float* scales,
@@ -826,7 +986,32 @@ extern "C" int qed_project_bwd(int C, int N, const float* means, const float* qu
     return project_bwd_impl(C, N, means, quats, scales, opacities, activations, colors_in, K, sh_degree, colors_per_camera, viewmats, Ks, width,
                             height, eps2d, calc_compensations, n_color, append_depth, radii, conics, compensations, v_means2d, v_depths, v_conics,
                             v_colors, v_opacities_cn, packed_grads, v_means, v_quats, v_scales, v_opacities, v_colors_in, nullptr,
-                            (cudaStream_t)stream_);
+                            nullptr, nullptr, (cudaStream_t)stream_);
+}
+
+extern "C" size_t qed_project_bwd_pose_workspace_bytes(int C, int N) { return pose_workspace_bytes(C, N); }
+
+extern "C" int qed_project_bwd_pose(int C, int N, const float* means, const float* quats, const float* scales,
+                                    const float* opacities, int activations, const float* colors_in, int K, int sh_degree,
+                                    int colors_per_camera, const float* viewmats, const float* Ks, int width, int height,
+                                    float eps2d, int calc_compensations, int n_color, int append_depth,
+                                    const int32_t* radii, const float* conics, const float* compensations,
+                                    const float* v_means2d, const float* v_depths, const float* v_conics,
+                                    const float* v_colors, const float* v_opacities_cn, const float* packed_grads,
+                                    float* v_means, float* v_quats, float* v_scales, float* v_opacities,
+                                    float* v_colors_in, float* v_viewmats, void* workspace, size_t workspace_bytes,
+                                    qed_stream_t stream_) {
+    if (C < 0 || N < 0) return QED_ERR_BAD_ARG;
+    if (C == 0) return QED_OK;
+    if (!v_viewmats) return QED_ERR_BAD_ARG;
+    if (N > 0) {
+        if (!workspace || (reinterpret_cast<uintptr_t>(workspace) & 15)) return QED_ERR_BAD_ARG;
+        if (workspace_bytes < pose_workspace_bytes(C, N)) return QED_ERR_WORKSPACE;
+    }
+    return project_bwd_impl(C, N, means, quats, scales, opacities, activations, colors_in, K, sh_degree, colors_per_camera, viewmats, Ks, width,
+                            height, eps2d, calc_compensations, n_color, append_depth, radii, conics, compensations, v_means2d, v_depths, v_conics,
+                            v_colors, v_opacities_cn, packed_grads, v_means, v_quats, v_scales, v_opacities, v_colors_in, nullptr,
+                            v_viewmats, reinterpret_cast<float4*>(workspace), (cudaStream_t)stream_);
 }
 
 extern "C" int qed_project_bwd_exchange(int C, int N, const float* means, const float* quats, const float* scales,
@@ -851,7 +1036,7 @@ extern "C" int qed_project_bwd_exchange(int C, int N, const float* means, const 
     x.xch_tag = tag;
     return project_bwd_impl(C, N, means, quats, scales, opacities, activations, sh_coeffs, K, sh_degree, 0, viewmats, Ks, width, height, eps2d,
                             calc_compensations, 3, append_depth, radii, conics, compensations, nullptr, nullptr, nullptr, nullptr, nullptr,
-                            packed_grads, v_means, v_quats, v_scales, v_opacities, nullptr, &x, (cudaStream_t)stream_);
+                            packed_grads, v_means, v_quats, v_scales, v_opacities, nullptr, &x, nullptr, nullptr, (cudaStream_t)stream_);
 }
 
 extern "C" int qed_sh_grad_from_view_colors(int total_slots, int N, int K, int sh_degree, const float* means, const float* exchange_local,

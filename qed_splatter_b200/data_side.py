@@ -24,21 +24,47 @@ from . import _lib
 from ._lib import check, current_stream, ptr
 
 
-def get_viewmat(optimized_camera_to_world: Tensor) -> Tensor:
-    """model.py:22-38: c2w [C,3|4,4] (OpenGL camera axes) -> gsplat world-to-camera [C,4,4]."""
+def _viewmat_from_c2w(c2w: Tensor) -> Tensor:
+    C = c2w.shape[0]
+    out = torch.empty(C, 4, 4, dtype=torch.float32, device=c2w.device)
+    check(_lib.load().qed_viewmat_from_c2w(C, int(c2w.shape[1]), ptr(c2w), ptr(out), current_stream()), "qed_viewmat_from_c2w")
+    return out
+
+
+class _GetViewmat(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, c2w):
+        c2w = c2w.detach().contiguous()
+        ctx.save_for_backward(c2w)
+        return _viewmat_from_c2w(c2w)
+
+    @staticmethod
+    def backward(ctx, v_viewmats):
+        (c2w,) = ctx.saved_tensors
+        v_viewmats = v_viewmats.to(torch.float32).contiguous()
+        v_c2w = torch.empty_like(c2w)
+        check(_lib.load().qed_viewmat_from_c2w_bwd(c2w.shape[0], int(c2w.shape[1]), ptr(c2w), ptr(v_viewmats), ptr(v_c2w), current_stream()),
+              "qed_viewmat_from_c2w_bwd")
+        return v_c2w
+
+
+def get_viewmat(optimized_camera_to_world: Tensor, pose_gradients: bool = False) -> Tensor:
+    """model.py:22-38: c2w [C,3|4,4] (OpenGL camera axes) -> gsplat world-to-camera [C,4,4].
+
+    `pose_gradients=True`: when c2w requires grad, the result carries the gradient back to it (the camera optimizer's
+    pose; bind `functools.partial(get_viewmat, pose_gradients=True)`, INTEGRATION.md section 2b).  The forward values are
+    the same bits either way."""
     c2w = optimized_camera_to_world
     _lib.require_cuda(c2w)
     _lib.require_dtype(c2w, (torch.float32,), "optimized_camera_to_world")
     if c2w.dim() != 3 or c2w.shape[1] not in (3, 4) or c2w.shape[2] != 4:
         raise ValueError("optimized_camera_to_world must be [C,3,4] or [C,4,4]")
     if c2w.requires_grad and torch.is_grad_enabled():
-        # camera_optimizer.mode != "off": the projection has no pose gradient (rasterization() raises for it too)
-        raise NotImplementedError("get_viewmat: no gradient with respect to the camera pose (camera_optimizer must be 'off')")
-    c2w = c2w.detach().contiguous()
-    C = c2w.shape[0]
-    out = torch.empty(C, 4, 4, dtype=torch.float32, device=c2w.device)
-    check(_lib.load().qed_viewmat_from_c2w(C, int(c2w.shape[1]), ptr(c2w), ptr(out), current_stream()), "qed_viewmat_from_c2w")
-    return out
+        if pose_gradients:
+            return _GetViewmat.apply(c2w)
+        # camera_optimizer.mode != "off" without asking for pose gradients: refuse rather than train with zero gradients
+        raise NotImplementedError("get_viewmat: c2w requires grad (camera optimisation): pass pose_gradients=True, or c2w.detach()")
+    return _viewmat_from_c2w(c2w.detach().contiguous())
 
 
 def _host_f32(x, shape, what: str) -> np.ndarray:

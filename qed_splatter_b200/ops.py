@@ -150,12 +150,19 @@ class _ProjectGaussians(torch.autograd.Function):
             separate = (None, ptr(_f32c(v_depths)), None, None, None)
         else:
             separate = (ptr(_f32c(v_means2d)), ptr(_f32c(v_depths)), ptr(_f32c(v_conics)), ptr(_f32c(v_colors)), ptr(_f32c(v_opac)))
-        check(lib.qed_project_bwd(C, N, ptr(means), ptr(quats), ptr(scales), ptr(opacities), 0, ptr(colors) if n_color else None,
-                                  K, sh_degree, per_cam, ptr(viewmats), ptr(Ks), width, height, eps2d, int(calc_comp),
-                                  n_color, append_depth, ptr(radii), ptr(conics), ptr(comps),
-                                  *separate, ctypes_ptr(packed), ptr(v_means), ptr(v_quats), ptr(v_scales), ptr(v_opacities),
-                                  ptr(v_colors_in), current_stream()), "qed_project_bwd")
-        return (v_means, v_quats, v_scales, v_opacities, v_colors_in, None, None) + (None,) * 11
+        args = (C, N, ptr(means), ptr(quats), ptr(scales), ptr(opacities), 0, ptr(colors) if n_color else None,
+                K, sh_degree, per_cam, ptr(viewmats), ptr(Ks), width, height, eps2d, int(calc_comp),
+                n_color, append_depth, ptr(radii), ptr(conics), ptr(comps),
+                *separate, ctypes_ptr(packed), ptr(v_means), ptr(v_quats), ptr(v_scales), ptr(v_opacities), ptr(v_colors_in))
+        v_viewmats = None
+        if ctx.needs_input_grad[5]:  # camera poses (gsplat's v_viewmats)
+            v_viewmats = torch.empty(C, 4, 4, device=dev)
+            ws_bytes = lib.qed_project_bwd_pose_workspace_bytes(C, N)
+            ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dev)
+            check(lib.qed_project_bwd_pose(*args, ptr(v_viewmats), ptr(ws), ws_bytes, current_stream()), "qed_project_bwd_pose")
+        else:
+            check(lib.qed_project_bwd(*args, current_stream()), "qed_project_bwd")
+        return (v_means, v_quats, v_scales, v_opacities, v_colors_in, v_viewmats, None) + (None,) * 11
 
 
 def project_gaussians(means: Tensor, quats: Tensor, scales: Tensor, opacities: Tensor, colors: Optional[Tensor],

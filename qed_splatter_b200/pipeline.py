@@ -34,6 +34,7 @@ class StepOutput:
     alphas: Tensor  # [C,H,W,1]
     n_isects: int
     n_visible: Optional[int] = None
+    v_viewmats: Optional[Tensor] = None  # [C,4,4] d loss / d viewmats, step(pose_gradients=True) only
 
 
 ACT_LOG_SCALES, ACT_LOGIT_OPACITIES = 1, 2  # `activations` bits (include/qed_splat.h)
@@ -231,7 +232,7 @@ class FusedSplatStep:
     # -- backward from explicit output gradients ------------------------------------------------
     @torch.no_grad()
     def backward(self, v_render: Tensor, v_alphas: Optional[Tensor], grad_out: Optional[Dict[str, Tensor]] = None,
-                 n_chunks: int = 1, on_chunk=None, exchange=None, _redo=None):
+                 n_chunks: int = 1, on_chunk=None, exchange=None, v_viewmats: Optional[Tensor] = None, _redo=None):
         """`grad_out`: optional preallocated {means,quats,scales,opacities,sh} (e.g. views into a flat
         all-reduce arena) that the projection backward writes straight into.
 
@@ -242,8 +243,13 @@ class FusedSplatStep:
         `exchange` (comm.ViewShardedGradients, world_size > 1): the gradients are SUMMED OVER ALL RANKS' views before this
         returns (in stream order): the projection backward stores its per-view colour gradients into every rank's exchange
         buffer, one all-reduce kernel sums the 11 non-SH floats per Gaussian and every rank rebuilds the SH coefficient
-        gradient locally.  Returns views into the exchange's arena."""
+        gradient locally.  Returns views into the exchange's arena.
+
+        `v_viewmats` ([C,4,4] float32, optional): receives the gradient with respect to the camera poses (overwritten).
+        Not with `exchange` or `n_chunks` > 1."""
         lib, stream = self.lib, current_stream()
+        if v_viewmats is not None and (exchange is not None or n_chunks > 1):
+            raise ValueError("pose gradients (v_viewmats) are not available with exchange= or n_chunks > 1")
 
         def composite_backward(v_r, v_a):
             f = self._fwd
@@ -298,15 +304,20 @@ class FusedSplatStep:
         for k, (n0, n1) in enumerate(bounds):
             # C == 1 when chunked: flat index == n, so a range is just a pointer offset on every [N,...] / [1,N,...] array
             sl = slice(n0, n1)
-            check(lib.qed_project_bwd(C, n1 - n0, ptr(means[sl]), ptr(quats[sl]), ptr(scales[sl]), ptr(opacities[sl]), f["activations"],
-                                      ptr(sh[sl]) if has_sh else None, f["K"], f["deg"], 0, ptr(viewmats), ptr(Ks), f["width"], f["height"],
-                                      f["eps2d"], int(f["comp"]), f["n_color"], f["append"],
-                                      ptr(f["radii"][:, sl] if len(bounds) > 1 else f["radii"]),
-                                      ptr(f["conics"][:, sl] if len(bounds) > 1 else f["conics"]),
-                                      ptr((f["comps"][:, sl] if len(bounds) > 1 else f["comps"]) if f["comps"] is not None else None),
-                                      None, None, None, None, None, ptr(packed[n0:n1] if len(bounds) > 1 else packed),
-                                      ptr(v_means[sl]), ptr(v_quats[sl]), ptr(v_scales[sl]), ptr(v_opac[sl]),
-                                      ptr(v_sh[sl]) if has_sh else None, stream), "qed_project_bwd")
+            args = (C, n1 - n0, ptr(means[sl]), ptr(quats[sl]), ptr(scales[sl]), ptr(opacities[sl]), f["activations"],
+                    ptr(sh[sl]) if has_sh else None, f["K"], f["deg"], 0, ptr(viewmats), ptr(Ks), f["width"], f["height"],
+                    f["eps2d"], int(f["comp"]), f["n_color"], f["append"],
+                    ptr(f["radii"][:, sl] if len(bounds) > 1 else f["radii"]),
+                    ptr(f["conics"][:, sl] if len(bounds) > 1 else f["conics"]),
+                    ptr((f["comps"][:, sl] if len(bounds) > 1 else f["comps"]) if f["comps"] is not None else None),
+                    None, None, None, None, None, ptr(packed[n0:n1] if len(bounds) > 1 else packed),
+                    ptr(v_means[sl]), ptr(v_quats[sl]), ptr(v_scales[sl]), ptr(v_opac[sl]), ptr(v_sh[sl]) if has_sh else None)
+            if v_viewmats is None:
+                check(lib.qed_project_bwd(*args, stream), "qed_project_bwd")
+            else:  # one range (n_chunks > 1 is refused above)
+                ws_bytes = lib.qed_project_bwd_pose_workspace_bytes(C, N)
+                ws = self._get("pose_ws", (max(ws_bytes, 16),), torch.uint8)
+                check(lib.qed_project_bwd_pose(*args, ptr(v_viewmats), ptr(ws), ws_bytes, stream), "qed_project_bwd_pose")
             if on_chunk is not None:
                 on_chunk(k, n0, n1)
         self._mark("project_bwd")
@@ -319,13 +330,18 @@ class FusedSplatStep:
              gt_rgb: Tensor, gt_depth: Tensor, background: Tensor, render_mode: str = "RGB+ED", rgb_weight: float = 0.8,
              depth_lambda: float = 0.2, grad_scale: float = 1.0, rasterize_mode: str = "classic",
              grad_out: Optional[Dict[str, Tensor]] = None, ssim_lambda: float = 0.0, n_chunks: int = 1, on_chunk=None,
-             activations: int = 0, mask: Optional[Tensor] = None, exchange=None, depth_unit_scale: float = 0.001) -> StepOutput:
+             activations: int = 0, mask: Optional[Tensor] = None, exchange=None, depth_unit_scale: float = 0.001,
+             pose_gradients: bool = False) -> StepOutput:
         """`render_mode` RGB+ED (north_star) or RGB+D (what qed_splatter/model.py:257 passes).
         loss = rgb_weight * L1 + ssim_lambda * (1 - SSIM) + depth_lambda * masked depth-L1 (splatfacto: 0.8 / 0.2 / 0.2).
         `mask` [C,H,W(,1)] float32 / uint8 / bool = `batch["mask"]` (model.py:93-97), see losses.depth_supervised_loss.
         The returned StepOutput aliases buffers this object reuses: the next step() overwrites loss / render / alphas /
-        packed_grads / radii in place -- clone() what must outlive the step."""
+        packed_grads / radii / v_viewmats in place -- clone() what must outlive the step.
+        `pose_gradients=True`: StepOutput.v_viewmats [C,4,4] = d loss / d viewmats (camera optimisation); not with
+        `exchange` or `n_chunks` > 1."""
         assert render_mode in ("RGB+D", "RGB+ED")
+        if pose_gradients and (exchange is not None or n_chunks > 1):
+            raise ValueError("pose_gradients=True is not available with exchange= or n_chunks > 1")
         lib, stream = self.lib, current_stream()
         # raw pointers cross the C-ABI: wrong device / dtype must raise here, not fault in the kernel
         _lib.require_cuda(means, gt_rgb, gt_depth, background, mask)
@@ -366,11 +382,13 @@ class FusedSplatStep:
             return forward_and_loss(True)[2:]
 
         render, alphas, v_render, v_alphas = forward_and_loss(False)
-        grads, packed = self.backward(v_render, v_alphas, grad_out, n_chunks=n_chunks, on_chunk=on_chunk, exchange=exchange, _redo=redo)
+        v_viewmats = self._get("v_viewmats", (C, 4, 4)) if pose_gradients else None
+        grads, packed = self.backward(v_render, v_alphas, grad_out, n_chunks=n_chunks, on_chunk=on_chunk, exchange=exchange, v_viewmats=v_viewmats,
+                                      _redo=redo)
         self._last_v = (v_render, v_alphas)
         f = self._fwd
         return StepOutput(loss=self._loss, grads=grads, packed_grads=packed, radii=f["radii"], render=f["render"], alphas=f["alphas"],
-                          n_isects=f.get("n_isects_real", f["M"]), n_visible=f.get("n_visible"))
+                          n_isects=f.get("n_isects_real", f["M"]), n_visible=f.get("n_visible"), v_viewmats=v_viewmats)
 
     # -- instrumentation (never inside a timed region) --------------------------------------------
     def n_isects_exact(self) -> int:

@@ -95,8 +95,14 @@ def rasterization(
     distributed: bool = False,
     camera_model: str = "pinhole",
     covars: Optional[Tensor] = None,
+    pose_gradients: bool = False,
 ) -> Tuple[Tensor, Tensor, Dict]:
-    """-> (render_colors[C,H,W,D], render_alphas[C,H,W,1], info)."""
+    """-> (render_colors[C,H,W,D], render_alphas[C,H,W,1], info).
+
+    `pose_gradients=True`: `viewmats` may require grad and receives d loss / d viewmats (gsplat's v_viewmats, what
+    splatfacto's camera optimizer trains the poses with; row 3 is zero).  Bind it for the reference model with
+    `functools.partial(rasterization, pose_gradients=True)` (INTEGRATION.md section 2b).  Off by default: a viewmat that
+    requires grad then raises, as before."""
     if render_mode not in RENDER_MODES:
         raise ValueError(f"render_mode must be one of {RENDER_MODES}, got {render_mode!r}")
     if rasterize_mode not in ("classic", "antialiased"):
@@ -107,13 +113,15 @@ def rasterization(
             "qed_splatter/model.py:267-288 and are out of scope for this path")
     if tile_size != 16:
         raise NotImplementedError("tile_size is 16 on this path (qed_splatter/model.py:243)")
-    if torch.is_grad_enabled() and (viewmats.requires_grad or Ks.requires_grad):
-        # gsplat returns v_viewmats; this path does not (qed_project_bwd has no pose gradient).  With splatfacto's
-        # camera_optimizer mode "off" (the default, and what qed_splatter/config.py keeps) the viewmat built at
-        # model.py:212,246 carries no gradient; any other mode would silently train with zero pose gradients.
+    if torch.is_grad_enabled() and Ks.requires_grad:
+        raise NotImplementedError("gradients with respect to Ks (intrinsics) are not implemented on this path: pass Ks.detach()")
+    if torch.is_grad_enabled() and viewmats.requires_grad and not pose_gradients:
+        # With splatfacto's camera_optimizer mode "off" (the default, and what qed_splatter/config.py keeps) the viewmat
+        # built at model.py:212,246 carries no gradient.  A viewmat that does is refused unless pose gradients were asked
+        # for, so that a camera optimizer never trains silently with zero pose gradients.
         raise NotImplementedError(
-            "gradients with respect to viewmats / Ks (camera optimisation) are not implemented on this path: "
-            "use camera_optimizer mode 'off' or pass viewmats.detach()")
+            "viewmats requires grad (camera optimisation): pass pose_gradients=True to compute v_viewmats, "
+            "or pass viewmats.detach()")
     N = means.shape[0]
     C = viewmats.shape[0]
     assert means.shape == (N, 3), means.shape

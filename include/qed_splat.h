@@ -323,6 +323,25 @@ int qed_viewmat_from_c2w(int C, int rows, const float* camera_to_worlds, float* 
 int qed_viewmat_from_c2w_bwd(int C, int rows, const float* camera_to_worlds, const float* v_viewmats, float* v_camera_to_worlds,
                              qed_stream_t stream);
 
+/* Splatfacto's camera optimizer in mode SO3xR3 (nerfstudio CameraOptimizer, applied at model.py:212/246).
+ *  pose_adjustment[num_cameras,6] float32: per training camera {translation t (3), rotation log omega (3)}.
+ *  camera_ids[C] int32 in [0, num_cameras): the table row of each view (the caller validates; an id outside the range
+ *  gives a NaN viewmat and no gradient).  camera_to_worlds [C, rows, 4] as for qed_viewmat_from_c2w.
+ *  theta^2 = max(|omega|^2, 1e-4), R = I + (sin theta / theta) [omega]x + ((1 - cos theta) / theta^2) [omega]x^2 (float64),
+ *  c2w' = c2w[:3,:4] @ [[R, t], [0, 1]]  (R' = Rc R, t' = Rc t + tc; t is not rotated), viewmat = get_viewmat(c2w').
+ * qed_camera_opt_apply: viewmats[C,4,4].  A view whose table row is zero gets exactly the bits of qed_viewmat_from_c2w.
+ * qed_camera_opt_bwd: v_pose_adjustment[num_cameras,6] (overwritten; rows of no view get zero) = d loss / d table from
+ *  v_viewmats[C,4,4], float64 inside; views sharing a camera id are summed in view order (no atomics, deterministic).
+ * qed_camera_opt_reg: the regulariser of CameraOptimizer.get_loss_dict over all rows,
+ *  reg_loss[1] (device) = trans_weight * mean_rows |t| + rot_weight * mean_rows |omega|; its gradient (zero at a zero
+ *  norm) is ADDED to v_pose_adjustment.  One block, fixed-order float64 sums. */
+int qed_camera_opt_apply(int C, int rows, int num_cameras, const int32_t* camera_ids, const float* camera_to_worlds,
+                         const float* pose_adjustment, float* viewmats, qed_stream_t stream);
+int qed_camera_opt_bwd(int C, int rows, int num_cameras, const int32_t* camera_ids, const float* camera_to_worlds,
+                       const float* pose_adjustment, const float* v_viewmats, float* v_pose_adjustment, qed_stream_t stream);
+int qed_camera_opt_reg(int num_cameras, const float* pose_adjustment, float trans_weight, float rot_weight, float* v_pose_adjustment,
+                       float* reg_loss, qed_stream_t stream);
+
 /* qed_splatter/create_init_pointcloud.py:148-196 `backproject_frame` (Open3D PointCloud.create_from_depth_image, :176-185):
  * depth [height,width] float32 or raw uint16 (depth_is_u16), metres = value * depth_unit_scale (float32 product, :165);
  * every `stride`-th pixel (u, v) with 0 < d < depth_max gives the world point inverse(extrinsic) * ((u-cx) d/fx, (v-cy) d/fy, d).
@@ -381,6 +400,17 @@ int qed_project_bwd_exchange(int C, int N, const float* means, const float* quat
                              const float* compensations, const float* packed_grads, float* v_means, float* v_quats,
                              float* v_scales, float* v_opacities, float* exchange_multicast, float* const* exchange_peers,
                              int world, int first_slot, int total_slots, float tag, qed_stream_t stream);
+/* qed_project_bwd_exchange that also returns the gradient with respect to this rank's C view poses, as qed_project_bwd_pose
+ * does: v_viewmats[C,4,4] (overwritten, the rank's own views, not summed over ranks) and pose_ws / ws_bytes >=
+ * qed_project_bwd_pose_workspace_bytes(C, N) (16-byte aligned; may be NULL when N == 0).  Deterministic. */
+int qed_project_bwd_exchange_pose(int C, int N, const float* means, const float* quats, const float* scales,
+                                  const float* opacities, int activations, const float* sh_coeffs, int K, int sh_degree,
+                                  const float* viewmats, const float* Ks, int width, int height, float eps2d,
+                                  int calc_compensations, int append_depth, const int32_t* radii, const float* conics,
+                                  const float* compensations, const float* packed_grads, float* v_means, float* v_quats,
+                                  float* v_scales, float* v_opacities, float* exchange_multicast, float* const* exchange_peers,
+                                  int world, int first_slot, int total_slots, float tag, float* v_viewmats, void* pose_ws,
+                                  size_t ws_bytes, qed_stream_t stream);
 int qed_sh_grad_from_view_colors(int total_slots, int N, int K, int sh_degree, const float* means, const float* exchange_local,
                                  float tag, float* v_sh, qed_stream_t stream);
 int qed_comm_flag_words(void);

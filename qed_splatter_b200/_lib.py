@@ -54,6 +54,8 @@ SIGNATURES = {
     "qed_strategy_update": (c_int, [c_int, c_int, P, c_int, P, c_int, c_int, c_int, P, P, P, P]),
     "qed_project_bwd_exchange": (c_int, [c_int, c_int, P, P, P, P, c_int, P, c_int, c_int, P, P, c_int, c_int, c_float, c_int, c_int, P, P, P, P,
                                          P, P, P, P, P, P, c_int, c_int, c_int, c_float, P]),
+    "qed_project_bwd_exchange_pose": (c_int, [c_int, c_int, P, P, P, P, c_int, P, c_int, c_int, P, P, c_int, c_int, c_float, c_int, c_int, P, P,
+                                              P, P, P, P, P, P, P, P, c_int, c_int, c_int, c_float, P, P, c_size_t, P]),
     "qed_sh_grad_from_view_colors": (c_int, [c_int, c_int, c_int, c_int, P, P, c_float, P, P]),
     "qed_comm_flag_words": (c_int, []),
     "qed_comm_barrier": (c_int, [P, c_int, c_int, ctypes.c_uint32, P]),
@@ -61,6 +63,9 @@ SIGNATURES = {
     "qed_arena_gather": (c_int, [c_int64, P, P, P, P, P, P, P, P, P, P, P, P, P, P]),
     "qed_viewmat_from_c2w": (c_int, [c_int, c_int, P, P, P]),
     "qed_viewmat_from_c2w_bwd": (c_int, [c_int, c_int, P, P, P, P]),
+    "qed_camera_opt_apply": (c_int, [c_int, c_int, c_int, P, P, P, P, P]),
+    "qed_camera_opt_bwd": (c_int, [c_int, c_int, c_int, P, P, P, P, P, P]),
+    "qed_camera_opt_reg": (c_int, [c_int, P, c_float, c_float, P, P, P]),
     "qed_backproject_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "qed_backproject_depth": (c_int, [c_int, c_int, P, c_int, c_double, c_float, c_int, P, P, P, P, P, c_size_t, P]),
     "qed_voxel_downsample_workspace_bytes": (c_size_t, [c_int64]),

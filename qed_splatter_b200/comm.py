@@ -84,12 +84,17 @@ class ViewShardedGradients:
       * `finish(...)`      : one all-reduce kernel over the 11 non-SH floats per Gaussian + the local rebuild of the SH
         coefficient gradient from all views.  After it the arena holds the sum over all ranks' views, bit-identical on
         every rank.
+      * with `num_cameras` > 0 (camera_opt.CameraPoseOptimizer): `project_bwd` also returns the pose gradient of the rank's
+        views, and `pose_grad` is a small symmetric buffer for the [num_cameras, 6] table gradient that
+        `reduce_pose_grad()` sums over the ranks with one more all-reduce kernel.
 
     No NCCL call, no host synchronisation; collective: every rank makes the same calls in the same order."""
 
-    def __init__(self, N: int, views_per_rank: int, device, group=None, force_peer_path: bool = False, headroom: float = 0.0):
+    def __init__(self, N: int, views_per_rank: int, device, group=None, force_peer_path: bool = False, headroom: float = 0.0,
+                 num_cameras: int = 0):
         """`headroom`: allocate for N * (1 + headroom) Gaussians so that `resize()` after a densification step usually
-        needs no new symmetric allocation (a collective)."""
+        needs no new symmetric allocation (a collective).  `num_cameras` > 0: pose-gradient capacity for a camera table of
+        that many rows."""
         from .trainer import GaussianArena
 
         self.views_per_rank = int(views_per_rank)
@@ -100,6 +105,8 @@ class ViewShardedGradients:
         self.slots = self.world * self.views_per_rank
         n_xch = (self.slots * self.capacity + self.slots) * 4
         self.xch = [SymmetricArena(n_xch, device, group, force_peer_path=force_peer_path) for _ in range(2)]
+        self.num_cameras = int(num_cameras)
+        self._pose = SymmetricArena(self.num_cameras * 6, device, group, force_peer_path=force_peer_path) if self.num_cameras > 0 else None
         self.step = 0
         self._side = torch.cuda.Stream(device=self.arena.device)
         self._fork, self._join = torch.cuda.Event(), torch.cuda.Event()
@@ -126,20 +133,35 @@ class ViewShardedGradients:
         shape = {"means": (N, 3), "quats": (N, 4), "scales": (N, 3), "opacities": (N,), "sh": (N, 16, 3)}
         return {g: self.arena.buf[a:b].view(*shape[g]) for g, (a, b) in self.offsets.items()}
 
+    @property
+    def pose_grad(self) -> Optional[torch.Tensor]:
+        """[num_cameras * 6 rounded up to 4] float32 in symmetric memory (None without pose capacity)."""
+        return None if self._pose is None else self._pose.buf
+
+    def reduce_pose_grad(self) -> None:
+        """pose_grad <- its sum over the ranks, bit-identical everywhere.  Collective; no NCCL."""
+        self._pose.all_reduce_()
+
     def _tag(self) -> float:
         return float(self.step % 8_000_000 + 1)  # exactly representable, never 0 (the buffers start zeroed)
 
     def project_bwd(self, lib, C, means, quats, scales, opacities, activations, sh, K, deg, viewmats, Ks, width, height, eps2d, comp, append,
-                    radii, conics, comps, packed, stream) -> None:
+                    radii, conics, comps, packed, stream, v_viewmats=None, pose_ws=None) -> None:
+        """`v_viewmats` [C,4,4] (pose capacity only): also the pose gradient of this rank's views, with `pose_ws` of
+        qed_project_bwd_pose_workspace_bytes(C, N) bytes."""
         assert C == self.views_per_rank and means.shape[0] == self.N
         x = self.xch[self.step & 1]
         g = self.views()
         ptr = _lib.ptr
-        _lib.check(lib.qed_project_bwd_exchange(C, self.N, ptr(means), ptr(quats), ptr(scales), ptr(opacities), int(activations), ptr(sh), K, deg,
-                                                ptr(viewmats), ptr(Ks), width, height, eps2d, int(comp), int(append), ptr(radii), ptr(conics),
-                                                ptr(comps), ptr(packed), ptr(g["means"]), ptr(g["quats"]), ptr(g["scales"]), ptr(g["opacities"]),
-                                                ctypes.c_void_p(x.multicast_ptr) if x.multicast_ptr else None, x._bases, self.world,
-                                                self.rank * C, self.slots, self._tag(), stream), "qed_project_bwd_exchange")
+        args = (C, self.N, ptr(means), ptr(quats), ptr(scales), ptr(opacities), int(activations), ptr(sh), K, deg, ptr(viewmats), ptr(Ks), width, height,
+                eps2d, int(comp), int(append), ptr(radii), ptr(conics), ptr(comps), ptr(packed), ptr(g["means"]), ptr(g["quats"]), ptr(g["scales"]),
+                ptr(g["opacities"]), ctypes.c_void_p(x.multicast_ptr) if x.multicast_ptr else None, x._bases, self.world, self.rank * C, self.slots,
+                self._tag())
+        if v_viewmats is None:
+            _lib.check(lib.qed_project_bwd_exchange(*args, stream), "qed_project_bwd_exchange")
+        else:
+            assert self.num_cameras > 0
+            _lib.check(lib.qed_project_bwd_exchange_pose(*args, ptr(v_viewmats), ptr(pose_ws), pose_ws.numel(), stream), "qed_project_bwd_exchange_pose")
 
     def finish(self, lib, means, K: int, deg: int, stream) -> None:
         x = self.xch[self.step & 1]

@@ -42,7 +42,7 @@ struct ProjBwdParams {
     float4* xch_peer[16];          // else: its unicast address on every rank
     int xch_world, xch_slot0, xch_total_slots;
     float xch_tag;
-    // camera pose gradient (POSE, see qed_project_bwd_pose): per-warp partial sums of the 15 per-view values
+    // camera pose gradient (POSE, see qed_project_bwd_pose / qed_project_bwd_exchange_pose): per-warp partial sums of the 15 per-view values
     // {v_W (9, row-major), v_t (3), sum of the SH direction gradient (3), 0}, 4 float4 at (c * warps + warp) * 4
     float4* pose_ws;
 };
@@ -186,11 +186,12 @@ __device__ __forceinline__ void quat_to_rotmat(float qw, float qx, float qy, flo
 // views, so it overwrites the staged coefficient row in place: half the shared memory, and with it 5 resident blocks per SM
 // instead of 4 (the kernel is latency-bound: 35 % issue-active at 16 warps per SM).  ONE = resident blocks asked of ptxas (5: 96
 // registers, 6: 80 registers).
-// POSE (not with XCH): also the gradient with respect to each view's world-to-camera matrix [W | t].  For every visible
+// POSE: also the gradient with respect to each view's world-to-camera matrix [W | t].  For every visible
 // (view, Gaussian) the values below are already in registers: the camera-space mean gradient v_p, the camera-space
 // covariance gradient vSc with A = W Sigma, and the SH direction gradient v_d.  v_W += v_p mu^T + 2 vSc A, v_t += v_p,
 // and sum v_d is kept for the camera-position term, which pose_finish_kernel applies once per view.  Per-warp partials
-// (pose_flush) at the end for ONE, after every view otherwise: the view loop then runs in every lane of the warp.
+// (pose_flush) at the end for ONE, after every view otherwise: the view loop then runs in every lane of the warp.  With XCH
+// the direction gradient comes from the same vb the exchange branch builds, so the pose values are the same.
 template <int DEG, bool VEC, bool XCH = false, int ONE = 0, bool POSE = false>
 __global__ void __launch_bounds__(kProjBwdThreads, ONE ? ONE : 4) project_bwd_kernel(const ProjBwdParams p) {
     extern __shared__ float4 smem4[];
@@ -889,7 +890,7 @@ static int dispatch_project_bwd(const ProjBwdParams& p, bool vec_ok, cudaStream_
     }
 }
 
-// v_viewmats != NULL: the POSE variant, with pose_ws = pose_workspace_bytes(C, N) of per-warp partials (not with xch)
+// v_viewmats != NULL: the POSE variant, with pose_ws = pose_workspace_bytes(C, N) of per-warp partials
 static int project_bwd_impl(int C, int N, const float* means, const float* quats, const float* scales,
                             const float* opacities, int activations, const float* colors_in, int K, int sh_degree,
                             int colors_per_camera, const float* viewmats, const float* Ks, int width, int height,
@@ -904,7 +905,7 @@ static int project_bwd_impl(int C, int N, const float* means, const float* quats
     if (!(n_color == 0 || n_color == 3) || !(append_depth == 0 || append_depth == 1)) return QED_ERR_BAD_ARG;
     if (v_viewmats && C > 0 && N == 0) QED_CUDA_TRY(cudaMemsetAsync(v_viewmats, 0, (size_t)C * 16 * sizeof(float), stream));
     if (C == 0 || N == 0) return QED_OK;
-    if (v_viewmats && (xch || !pose_ws)) return QED_ERR_BAD_ARG;
+    if (v_viewmats && !pose_ws) return QED_ERR_BAD_ARG;
     if (C > 1024) return QED_ERR_UNSUPPORTED;
     if (!means || !quats || !scales || !viewmats || !Ks || !radii || !conics || !v_means || !v_quats || !v_scales)
         return QED_ERR_BAD_ARG;
@@ -951,14 +952,30 @@ static int project_bwd_impl(int C, int N, const float* means, const float* quats
 
     const bool vec_ok = sh_degree >= 0 && ((K * 3) % 4 == 0) && ((reinterpret_cast<uintptr_t>(colors_in) & 15) == 0) &&
                         (xch || (reinterpret_cast<uintptr_t>(v_colors_in) & 15) == 0);
+    const auto pose_finish = [&]() -> int {
+        const int warps = ((N + kProjBwdThreads - 1) / kProjBwdThreads) * (kProjBwdThreads / 32);
+        QED_CUDA_TRY(launch_pdl(pose_finish_kernel, dim3(C), dim3(kPoseFinishThreads), 0, stream, warps, (const float4*)pose_ws, viewmats, v_viewmats));
+        return QED_OK;
+    };
     if (xch) {
         if (!vec_ok || n_color != 3) return QED_ERR_UNSUPPORTED;  // the exchange carries SH colour gradients
-        switch (sh_degree) {
-            case 0: return launch_project_bwd<0, true, true>(p, stream);
-            case 1: return launch_project_bwd<1, true, true>(p, stream);
-            case 2: return launch_project_bwd<2, true, true>(p, stream);
-            default: return launch_project_bwd<3, true, true>(p, stream);
+        if (!v_viewmats) {
+            switch (sh_degree) {
+                case 0: return launch_project_bwd<0, true, true>(p, stream);
+                case 1: return launch_project_bwd<1, true, true>(p, stream);
+                case 2: return launch_project_bwd<2, true, true>(p, stream);
+                default: return launch_project_bwd<3, true, true>(p, stream);
+            }
         }
+        p.pose_ws = pose_ws;
+        int rc;
+        switch (sh_degree) {
+            case 0: rc = launch_project_bwd<0, true, true, 0, true>(p, stream); break;
+            case 1: rc = launch_project_bwd<1, true, true, 0, true>(p, stream); break;
+            case 2: rc = launch_project_bwd<2, true, true, 0, true>(p, stream); break;
+            default: rc = launch_project_bwd<3, true, true, 0, true>(p, stream); break;
+        }
+        return rc != QED_OK ? rc : pose_finish();
     }
     if (n_color > 0 && (sh_degree < 0 || !vec_ok)) {
         // fallback paths accumulate straight into v_colors_in: clear it first
@@ -968,10 +985,7 @@ static int project_bwd_impl(int C, int N, const float* means, const float* quats
     if (!v_viewmats) return dispatch_project_bwd<false>(p, vec_ok, stream);
     p.pose_ws = pose_ws;
     const int rc = dispatch_project_bwd<true>(p, vec_ok, stream);
-    if (rc != QED_OK) return rc;
-    const int warps = ((N + kProjBwdThreads - 1) / kProjBwdThreads) * (kProjBwdThreads / 32);
-    QED_CUDA_TRY(launch_pdl(pose_finish_kernel, dim3(C), dim3(kPoseFinishThreads), 0, stream, warps, (const float4*)pose_ws, viewmats, v_viewmats));
-    return QED_OK;
+    return rc != QED_OK ? rc : pose_finish();
 }
 
 extern "C" int qed_project_bwd(int C, int N, const float* means, const float* quats, const float* scales,
@@ -1014,13 +1028,12 @@ extern "C" int qed_project_bwd_pose(int C, int N, const float* means, const floa
                             v_viewmats, reinterpret_cast<float4*>(workspace), (cudaStream_t)stream_);
 }
 
-extern "C" int qed_project_bwd_exchange(int C, int N, const float* means, const float* quats, const float* scales,
-                                        const float* opacities, int activations, const float* sh_coeffs, int K, int sh_degree,
-                                        const float* viewmats, const float* Ks, int width, int height, float eps2d,
-                                        int calc_compensations, int append_depth, const int32_t* radii, const float* conics,
-                                        const float* compensations, const float* packed_grads, float* v_means, float* v_quats,
-                                        float* v_scales, float* v_opacities, float* exchange_multicast, float* const* exchange_peers,
-                                        int world, int first_slot, int total_slots, float tag, qed_stream_t stream_) {
+static int project_bwd_exchange(int C, int N, const float* means, const float* quats, const float* scales, const float* opacities,
+                                int activations, const float* sh_coeffs, int K, int sh_degree, const float* viewmats, const float* Ks, int width,
+                                int height, float eps2d, int calc_compensations, int append_depth, const int32_t* radii, const float* conics,
+                                const float* compensations, const float* packed_grads, float* v_means, float* v_quats, float* v_scales,
+                                float* v_opacities, float* exchange_multicast, float* const* exchange_peers, int world, int first_slot,
+                                int total_slots, float tag, float* v_viewmats, float4* pose_ws, cudaStream_t stream) {
     if (world < 1 || world > 16 || first_slot < 0 || C < 0 || first_slot + C > total_slots) return QED_ERR_BAD_ARG;
     if (!exchange_multicast && !exchange_peers) return QED_ERR_BAD_ARG;
     if (!packed_grads || sh_degree < 0) return QED_ERR_BAD_ARG;
@@ -1036,7 +1049,41 @@ extern "C" int qed_project_bwd_exchange(int C, int N, const float* means, const 
     x.xch_tag = tag;
     return project_bwd_impl(C, N, means, quats, scales, opacities, activations, sh_coeffs, K, sh_degree, 0, viewmats, Ks, width, height, eps2d,
                             calc_compensations, 3, append_depth, radii, conics, compensations, nullptr, nullptr, nullptr, nullptr, nullptr,
-                            packed_grads, v_means, v_quats, v_scales, v_opacities, nullptr, &x, nullptr, nullptr, (cudaStream_t)stream_);
+                            packed_grads, v_means, v_quats, v_scales, v_opacities, nullptr, &x, v_viewmats, pose_ws, stream);
+}
+
+extern "C" int qed_project_bwd_exchange(int C, int N, const float* means, const float* quats, const float* scales,
+                                        const float* opacities, int activations, const float* sh_coeffs, int K, int sh_degree,
+                                        const float* viewmats, const float* Ks, int width, int height, float eps2d,
+                                        int calc_compensations, int append_depth, const int32_t* radii, const float* conics,
+                                        const float* compensations, const float* packed_grads, float* v_means, float* v_quats,
+                                        float* v_scales, float* v_opacities, float* exchange_multicast, float* const* exchange_peers,
+                                        int world, int first_slot, int total_slots, float tag, qed_stream_t stream_) {
+    return project_bwd_exchange(C, N, means, quats, scales, opacities, activations, sh_coeffs, K, sh_degree, viewmats, Ks, width, height, eps2d,
+                                calc_compensations, append_depth, radii, conics, compensations, packed_grads, v_means, v_quats, v_scales,
+                                v_opacities, exchange_multicast, exchange_peers, world, first_slot, total_slots, tag, nullptr, nullptr,
+                                (cudaStream_t)stream_);
+}
+
+extern "C" int qed_project_bwd_exchange_pose(int C, int N, const float* means, const float* quats, const float* scales,
+                                             const float* opacities, int activations, const float* sh_coeffs, int K, int sh_degree,
+                                             const float* viewmats, const float* Ks, int width, int height, float eps2d,
+                                             int calc_compensations, int append_depth, const int32_t* radii, const float* conics,
+                                             const float* compensations, const float* packed_grads, float* v_means, float* v_quats,
+                                             float* v_scales, float* v_opacities, float* exchange_multicast, float* const* exchange_peers,
+                                             int world, int first_slot, int total_slots, float tag, float* v_viewmats, void* pose_ws,
+                                             size_t ws_bytes, qed_stream_t stream_) {
+    if (C < 0 || N < 0) return QED_ERR_BAD_ARG;
+    if (C == 0) return QED_OK;
+    if (!v_viewmats) return QED_ERR_BAD_ARG;
+    if (N > 0) {
+        if (!pose_ws || (reinterpret_cast<uintptr_t>(pose_ws) & 15)) return QED_ERR_BAD_ARG;
+        if (ws_bytes < pose_workspace_bytes(C, N)) return QED_ERR_WORKSPACE;
+    }
+    return project_bwd_exchange(C, N, means, quats, scales, opacities, activations, sh_coeffs, K, sh_degree, viewmats, Ks, width, height, eps2d,
+                                calc_compensations, append_depth, radii, conics, compensations, packed_grads, v_means, v_quats, v_scales,
+                                v_opacities, exchange_multicast, exchange_peers, world, first_slot, total_slots, tag, v_viewmats,
+                                reinterpret_cast<float4*>(pose_ws), (cudaStream_t)stream_);
 }
 
 extern "C" int qed_sh_grad_from_view_colors(int total_slots, int N, int K, int sh_degree, const float* means, const float* exchange_local,

@@ -40,6 +40,11 @@ class StepOutput:
 ACT_LOG_SCALES, ACT_LOGIT_OPACITIES = 1, 2  # `activations` bits (include/qed_splat.h)
 
 
+def _pose_capable(exchange) -> bool:
+    """No exchange, or one with a pose-gradient buffer (comm.ViewShardedGradients(num_cameras > 0))."""
+    return exchange is None or getattr(exchange, "num_cameras", 0) > 0
+
+
 class FusedSplatStep:
     """Holds reusable device buffers; `forward()` renders, `step()` renders + loss + full backward."""
 
@@ -245,11 +250,12 @@ class FusedSplatStep:
         buffer, one all-reduce kernel sums the 11 non-SH floats per Gaussian and every rank rebuilds the SH coefficient
         gradient locally.  Returns views into the exchange's arena.
 
-        `v_viewmats` ([C,4,4] float32, optional): receives the gradient with respect to the camera poses (overwritten).
-        Not with `exchange` or `n_chunks` > 1."""
+        `v_viewmats` ([C,4,4] float32, optional): receives the gradient with respect to the camera poses (overwritten; with
+        `exchange`, this rank's views only).  Not with `n_chunks` > 1, nor with an exchange built without pose capacity
+        (comm.ViewShardedGradients(num_cameras=...))."""
         lib, stream = self.lib, current_stream()
-        if v_viewmats is not None and (exchange is not None or n_chunks > 1):
-            raise ValueError("pose gradients (v_viewmats) are not available with exchange= or n_chunks > 1")
+        if v_viewmats is not None and (n_chunks > 1 or not _pose_capable(exchange)):
+            raise ValueError("pose gradients (v_viewmats) are not available with n_chunks > 1 or an exchange without pose capacity")
 
         def composite_backward(v_r, v_a):
             f = self._fwd
@@ -280,8 +286,12 @@ class FusedSplatStep:
         if exchange is not None:
             if not f["n_color"] or f["deg"] < 0:
                 raise ValueError("the view-colour exchange needs SH colours (render_mode RGB / RGB+D / RGB+ED with sh_degree)")
+            ws = None
+            if v_viewmats is not None:
+                ws_bytes = lib.qed_project_bwd_pose_workspace_bytes(C, N)
+                ws = self._get("pose_ws", (max(ws_bytes, 16),), torch.uint8)
             exchange.project_bwd(lib, C, means, quats, scales, opacities, f["activations"], sh, f["K"], f["deg"], viewmats, Ks, f["width"], f["height"],
-                                 f["eps2d"], f["comp"], f["append"], f["radii"], f["conics"], f["comps"], packed, stream)
+                                 f["eps2d"], f["comp"], f["append"], f["radii"], f["conics"], f["comps"], packed, stream, v_viewmats=v_viewmats, pose_ws=ws)
             self._mark("project_bwd")
             exchange.finish(lib, means, f["K"], f["deg"], stream)
             self._mark("grad_exchange")
@@ -338,10 +348,10 @@ class FusedSplatStep:
         The returned StepOutput aliases buffers this object reuses: the next step() overwrites loss / render / alphas /
         packed_grads / radii / v_viewmats in place -- clone() what must outlive the step.
         `pose_gradients=True`: StepOutput.v_viewmats [C,4,4] = d loss / d viewmats (camera optimisation); not with
-        `exchange` or `n_chunks` > 1."""
+        `n_chunks` > 1, and with `exchange` only when it was built with pose capacity (num_cameras > 0)."""
         assert render_mode in ("RGB+D", "RGB+ED")
-        if pose_gradients and (exchange is not None or n_chunks > 1):
-            raise ValueError("pose_gradients=True is not available with exchange= or n_chunks > 1")
+        if pose_gradients and (n_chunks > 1 or not _pose_capable(exchange)):
+            raise ValueError("pose_gradients=True is not available with n_chunks > 1 or an exchange without pose capacity")
         lib, stream = self.lib, current_stream()
         # raw pointers cross the C-ABI: wrong device / dtype must raise here, not fault in the kernel
         _lib.require_cuda(means, gt_rgb, gt_depth, background, mask)

@@ -47,6 +47,15 @@ class Scene:
         return self.viewmats.shape[0]
 
 
+def camera_to_worlds(viewmats: Tensor) -> Tensor:
+    """Inverse of `get_viewmat` (model.py:22-38) for rigid world->camera viewmats [C,4,4] -> nerfstudio camera-to-world
+    [C,3,4] (OpenGL camera axes): R = W^T with the y / z columns flipped back, T = -W^T t."""
+    W, t = viewmats[:, :3, :3], viewmats[:, :3, 3:]
+    R = W.transpose(1, 2)
+    flip = torch.tensor([[[1.0, -1.0, -1.0]]], dtype=R.dtype, device=R.device)
+    return torch.cat([R * flip, -(R @ t)], dim=-1).contiguous()
+
+
 def look_at(eye: Tensor, target: Tensor, up=(0.0, -1.0, 0.0)) -> Tensor:
     """World->camera [4,4] in gsplat/OpenCV convention (+z forward, +y down)."""
     eye = eye.to(torch.float64)

@@ -83,6 +83,25 @@ class TrainConfig:
     comm: str = "auto"
     comm_chunks: int = 4  # "nccl": Gaussian ranges whose SH gradients are all-reduced / Adam-stepped in a pipeline
     chunk_project_bwd: bool = True  # "nccl": also split the projection backward so the first reductions start earlier
+    # splatfacto's camera optimizer (camera_opt.py): "off" or "SO3xR3" (a [num_cameras, 6] pose table trained with the
+    # Gaussians; SplatTrainer(num_cameras=...), step(None, ..., camera_to_worlds=, camera_ids=)).  [UP] = nerfstudio 1.1.5
+    # defaults restated from memory of the upstream code (CameraOptimizerConfig, splatfacto's "camera_opt" param group).
+    camera_optimizer: str = "off"
+    camera_opt_lr: float = 1e-4  # [UP] Adam lr (eps = adam_eps 1e-15 [UP])
+    camera_opt_lr_final: float = 5e-7  # [UP] ExponentialDecayScheduler lr_final, reached at max_steps
+    camera_opt_warmup: int = 1000  # [UP] warm-up steps from lr 0 (cosine ramp)
+    camera_opt_trans_l2_penalty: float = 1e-2  # [UP] weight of mean_rows |t| in the loss
+    camera_opt_rot_l2_penalty: float = 1e-3  # [UP] weight of mean_rows |omega| in the loss
+
+    def __post_init__(self):
+        self.validate()
+
+    def validate(self) -> None:
+        """Raises ValueError for settings no code path accepts (checked at construction and by SplatTrainer)."""
+        from .camera_opt import CAMERA_OPTIMIZER_MODES
+
+        if self.camera_optimizer not in CAMERA_OPTIMIZER_MODES:
+            raise ValueError(f"camera_optimizer must be one of {CAMERA_OPTIMIZER_MODES}, got {self.camera_optimizer!r}")
 
     def lr_means_at(self, step: int) -> float:
         """nerfstudio ExponentialDecayScheduler (no warmup): log-linear from lr to lr_final over max_steps."""
@@ -388,8 +407,10 @@ class SplatTrainer:
 
     def __init__(self, means: Tensor, quats: Tensor, log_scales: Tensor, logit_opacities: Tensor, sh: Tensor,
                  cfg: Optional[TrainConfig] = None, rank: int = 0, world_size: int = 1, process_group=None,
-                 backend: str = "cuda"):
+                 backend: str = "cuda", num_cameras: int = 0):
+        """`num_cameras`: rows of the camera optimizer's pose table (the training cameras; cfg.camera_optimizer != "off")."""
         self.cfg = cfg or TrainConfig()
+        self.cfg.validate()  # fields may have been changed after construction
         self.rank, self.world = rank, world_size
         self.pg = process_group
         self.backend = backend
@@ -405,6 +426,25 @@ class SplatTrainer:
         self._lr_dev = None
         self._xg = None  # comm.ViewShardedGradients for the current (N, views per rank), built lazily
         self.comm = self._pick_comm()
+        self.camera_opt = None
+        if self.cfg.camera_optimizer != "off":
+            from .camera_opt import CameraPoseOptimizer
+
+            c = self.cfg
+            self.camera_opt = CameraPoseOptimizer(num_cameras, self.device, lr=c.camera_opt_lr, lr_final=c.camera_opt_lr_final,
+                                                  warmup_steps=c.camera_opt_warmup, max_steps=c.max_steps,
+                                                  trans_weight=c.camera_opt_trans_l2_penalty, rot_weight=c.camera_opt_rot_l2_penalty,
+                                                  betas=c.adam_betas, eps=c.adam_eps, backend=backend)
+
+    @property
+    def pose_adjustment(self) -> Optional[Tensor]:
+        """The camera optimizer's [num_cameras, 6] table (translation, rotation log); None when it is off."""
+        return None if self.camera_opt is None else self.camera_opt.pose_adjustment
+
+    @property
+    def camera_opt_loss(self) -> Optional[Tensor]:
+        """The camera optimizer's regulariser of the last step (device scalar [1]); None when it is off."""
+        return None if self.camera_opt is None else self.camera_opt.reg_loss
 
     def _pick_comm(self) -> str:
         c = self.cfg.comm
@@ -432,7 +472,8 @@ class SplatTrainer:
             err = None
             try:
                 x = ViewShardedGradients(self.arena.N, views_per_rank, self.device, self.pg,
-                                         headroom=0.25 if self.step_count < self.cfg.stop_split_at else 0.0)
+                                         headroom=0.25 if self.step_count < self.cfg.stop_split_at else 0.0,
+                                         num_cameras=0 if self.camera_opt is None else self.camera_opt.num_cameras)
             except Exception as e:  # noqa: BLE001  (no peer mappings / symmetric memory on this box)
                 x, err = None, e
             ok = torch.tensor([0.0 if x is None else 1.0], device=self.device)
@@ -446,6 +487,8 @@ class SplatTrainer:
         if self.arena.grad.data_ptr() != x.grad.data_ptr():
             assert x.grad.numel() == self.arena.grad.numel()
             self.arena.grad = x.grad  # Adam reads the summed gradients straight from the symmetric arena
+        if self.camera_opt is not None and self.camera_opt.grad.data_ptr() != x.pose_grad.data_ptr():
+            self.camera_opt.use_grad_buffer(x.pose_grad)
         return x
 
     # -- collectives --------------------------------------------------------------------------
@@ -528,6 +571,24 @@ class SplatTrainer:
             assert lo == 0 and hi == a.param.numel()
             adam_step_torch(a, lrs, c.lr_features_rest, c, t)
 
+    def camera_opt_update(self, v_viewmats: Tensor, camera_ids: Tensor, camera_to_worlds: Tensor, exchange=None) -> None:
+        """The camera optimizer's part of a step, after the backward: table gradient of the local views, its sum over the
+        ranks (this library's all-reduce kernel with `exchange`, else torch.distributed), the regulariser (once, identically
+        on every rank) and Adam on the table.  Replicas keep bit-identical tables."""
+        camera_to_worlds, camera_ids = self.camera_opt.prepare(camera_to_worlds, camera_ids)
+        self._camera_opt_update(v_viewmats, camera_ids, camera_to_worlds, exchange)
+
+    def _camera_opt_update(self, v_viewmats: Tensor, camera_ids: Tensor, camera_to_worlds: Tensor, exchange) -> None:
+        """camera_opt_update on inputs already passed through CameraPoseOptimizer.prepare."""
+        cam = self.camera_opt
+        cam._backward(v_viewmats, camera_ids, camera_to_worlds)
+        if exchange is not None:
+            exchange.reduce_pose_grad()
+        else:
+            self._all_reduce(cam.grad)
+        cam.regularize()
+        cam.step(self.step_count)
+
     def maybe_refine(self, step: int) -> Optional[Dict[str, int]]:
         """DefaultStrategy.step_post_backward schedule, called after the optimizer step of 0-based iteration
         `step` (nerfstudio passes its 0-based step; note gsplat resets opacities at step 0 too)."""
@@ -549,13 +610,24 @@ class SplatTrainer:
 
     # -- the full step --------------------------------------------------------------------------
     @torch.no_grad()
-    def step(self, viewmats: Tensor, Ks: Tensor, width: int, height: int, gt_rgb: Tensor, gt_depth: Tensor,
-             background: Tensor, total_views: Optional[int] = None, mask: Optional[Tensor] = None):
+    def step(self, viewmats: Optional[Tensor], Ks: Tensor, width: int, height: int, gt_rgb: Tensor, gt_depth: Tensor,
+             background: Tensor, total_views: Optional[int] = None, mask: Optional[Tensor] = None, *,
+             camera_to_worlds: Optional[Tensor] = None, camera_ids: Optional[Tensor] = None):
         """Local views [C_local,...]; `mask` = the batch's optional loss mask (model.py:93-97).
-        Returns (loss[3] device tensor of the local views -- a fresh copy, safe to keep for logging --, refine info|None)."""
+        With the camera optimizer on, `viewmats` is None and the views come as `camera_to_worlds` [C,3|4,4] (nerfstudio
+        camera-to-world) and `camera_ids` [C] (rows of the pose table); the viewmats are those of the adjusted poses.
+        Returns (loss[3] device tensor of the local views -- a fresh copy, safe to keep for logging --, refine info|None);
+        the camera optimizer's regulariser is `camera_opt_loss`."""
         if self._fused is None:
             raise RuntimeError("rendering needs the CUDA library (backend='cuda'); there is no CPU fallback")
-        c, a = self.cfg, self.arena
+        c, a, cam = self.cfg, self.arena, self.camera_opt
+        if cam is not None:
+            if viewmats is not None or camera_to_worlds is None or camera_ids is None:
+                raise ValueError("camera optimizer on: pass viewmats=None with camera_to_worlds= and camera_ids=")
+            camera_to_worlds, camera_ids = cam.prepare(camera_to_worlds, camera_ids)  # validated once per step
+            viewmats = cam._viewmats(camera_to_worlds, camera_ids)
+        elif camera_to_worlds is not None or camera_ids is not None:
+            raise ValueError("camera_to_worlds= / camera_ids= need cfg.camera_optimizer != 'off'")
         C = viewmats.shape[0]
         total = total_views or C * self.world
         pv = a.views(a.param)
@@ -567,14 +639,19 @@ class SplatTrainer:
             out = self._fused.step(pv["means"], pv["quats"], pv["scales"], pv["opacities"], pv["sh"], viewmats, Ks, width, height,
                                    self.sh_degree_to_use(), gt_rgb, gt_depth, background, render_mode=c.render_mode, rgb_weight=1.0 - c.ssim_lambda,
                                    depth_lambda=c.depth_lambda, grad_scale=C / float(total), rasterize_mode=c.rasterize_mode, activations=3,
-                                   mask=mask, ssim_lambda=c.ssim_lambda, exchange=xg, depth_unit_scale=c.depth_unit_scale)
+                                   mask=mask, ssim_lambda=c.ssim_lambda, exchange=xg, depth_unit_scale=c.depth_unit_scale,
+                                   pose_gradients=cam is not None)
             self.accumulate_stats(out.packed_grads, out.radii, width, height, packed=True, n_cameras=total)
             self.optimizer_step()
+            if cam is not None:
+                self._camera_opt_update(out.v_viewmats, camera_ids, camera_to_worlds, xg)
             loss = out.loss.clone()
             info = self.maybe_refine(self.step_count)
             self.step_count += 1
             return loss, info
         pipelined = self.world > 1 and C == 1 and c.comm_chunks > 1
+        # pose gradients need the projection backward in one launch: the pipelined path then chunks only the reductions
+        chunked_bwd = pipelined and c.chunk_project_bwd and cam is None
         sh0 = a.offsets["sh"][0]
         works = []
 
@@ -590,13 +667,13 @@ class SplatTrainer:
                                depth_lambda=c.depth_lambda, grad_scale=C / float(total), rasterize_mode=c.rasterize_mode, grad_out=gv,
                                activations=3,  # ACT_LOG_SCALES | ACT_LOGIT_OPACITIES (pipeline.py / include/qed_splat.h)
                                mask=mask, depth_unit_scale=c.depth_unit_scale, ssim_lambda=c.ssim_lambda,
-                               n_chunks=c.comm_chunks if (pipelined and c.chunk_project_bwd) else 1,
-                               on_chunk=on_chunk if (pipelined and c.chunk_project_bwd) else None)
+                               n_chunks=c.comm_chunks if chunked_bwd else 1, on_chunk=on_chunk if chunked_bwd else None,
+                               pose_gradients=cam is not None)
         self.accumulate_stats(out.packed_grads, out.radii, width, height, packed=True, n_cameras=total)
         if pipelined:
             import torch.distributed as dist
 
-            if not c.chunk_project_bwd:  # one projection-backward launch, then chunked reductions
+            if not chunked_bwd:  # one projection-backward launch, then chunked reductions
                 step_n = ((a.N + c.comm_chunks - 1) // c.comm_chunks + 3) // 4 * 4
                 for k, n0 in enumerate(range(0, a.N, step_n)):
                     on_chunk(k, n0, min(n0 + step_n, a.N))
@@ -609,6 +686,8 @@ class SplatTrainer:
         else:
             self._all_reduce(a.grad)
             self.optimizer_step()
+        if cam is not None:
+            self._camera_opt_update(out.v_viewmats, camera_ids, camera_to_worlds, None)
         loss = out.loss.clone()  # out.loss is a buffer the next step overwrites in place
         info = self.maybe_refine(self.step_count)
         self.step_count += 1

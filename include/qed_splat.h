@@ -272,6 +272,40 @@ int qed_loss_fwd_bwd(int C, int width, int height, const float* render, const fl
                      float depth_lambda, float ssim_lambda, float grad_scale, double* stats_dev, float* loss_dev,
                      float* v_render, float* v_alphas, void* workspace, size_t workspace_bytes, qed_stream_t stream);
 
+/* The same loss with splatfacto's bilateral grid (nerfstudio lib_bilagrid, per-image colour correction) applied to the
+ * clamped composite of every view before the mask, L1 and SSIM.  The depth term is unchanged.
+ *  grids[num_grids,12,L,Y,X] float32: per training image a 3x4 affine colour matrix A[i][j] = grid channel 4i+j.
+ *  grid_ids[C] int32 in [0, num_grids): the grid of each view (the caller validates; an id outside the range gives NaN).
+ *  Slice of pixel (row h, column w) with clamped colour c: x = w/(W-1), y = h/(H-1) (0 for an extent of 1),
+ *  gray = 0.299 c0 + 0.587 c1 + 0.114 c2; lattice coordinates gx = x (X-1), gy = y (Y-1), gz = gray (L-1), each clamped
+ *  to its axis, as grid_sample(mode="bilinear", align_corners=True, padding_mode="border") on [12, L, Y, X]; A = trilinear
+ *  interpolation of the 8 neighbouring cells; out_i = sum_j A[i][j] c_j + A[i][3], not clamped.
+ *  The gradient to render / alphas runs through out -> c, including the guidance term through gz (zero where gz is clamped).
+ *  v_grid_rows[C,12,L,Y,X] (overwritten): d loss / d grid of each VIEW, i.e. before views sharing a grid are summed
+ *  (qed_bilagrid_accumulate does that).  Deterministic: no atomics, the same inputs give the same bits.
+ *  Supported: 2 <= X, Y <= 1024, 2 <= L <= 16 (QED_ERR_UNSUPPORTED otherwise).  workspace_bytes >=
+ *  qed_loss_bilagrid_workspace_bytes (32 B/pixel of per-pixel records, plus the SSIM buffers when ssim_lambda > 0). */
+size_t qed_loss_bilagrid_workspace_bytes(int C, int width, int height, float ssim_lambda);
+int qed_loss_fwd_bwd_bilagrid(int C, int width, int height, const float* render, const float* alphas,
+                              const void* gt_rgb, int gt_rgb_is_u8, const void* gt_depth, int gt_depth_is_u16, double depth_unit_scale,
+                              const void* mask, int mask_is_u8, const float* bg, float rgb_weight,
+                              float depth_lambda, float ssim_lambda, float grad_scale, double* stats_dev, float* loss_dev,
+                              float* v_render, float* v_alphas, const float* grids, const int32_t* grid_ids, int num_grids,
+                              int grid_X, int grid_Y, int grid_L, float* v_grid_rows, void* workspace, size_t workspace_bytes,
+                              qed_stream_t stream);
+
+/* Total-variation regulariser of the bilateral grids (splatfacto get_loss_dict while training):
+ *  loss_out[1] = weight / G * sum_{axes d in L, Y, X} sum (x[.., i+1, ..] - x[.., i, ..])^2 / (elements of one grid's
+ *  difference along d, i.e. 12 L Y X (n_d - 1) / n_d).  v_grids[G,12,L,Y,X] is OVERWRITTEN with its gradient;
+ *  tv_per_grid[G] (double, overwritten) = each grid's unweighted sum of the per-axis means.  Fixed-order sums, no atomics.
+ *  Shapes as for qed_loss_fwd_bwd_bilagrid. */
+int qed_bilagrid_tv(int num_grids, int grid_X, int grid_Y, int grid_L, const float* grids, float weight, float* v_grids,
+                    double* tv_per_grid, float* loss_out, qed_stream_t stream);
+/* v_grids[grid_ids[r]] += v_grid_rows[r] for r = 0 .. n_rows-1 in row order, so rows sharing an id are summed
+ * deterministically.  Rows whose id is outside [0, num_grids) are skipped. */
+int qed_bilagrid_accumulate(int n_rows, const int32_t* grid_ids, const float* v_grid_rows, int num_grids, int grid_X, int grid_Y,
+                            int grid_L, float* v_grids, qed_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * trainer-side kernels (SURVEY.md §8 rows a14, a16)
  */

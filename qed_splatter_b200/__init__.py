@@ -6,7 +6,7 @@ loss-gradient / trainer step built on the same kernels.  Hand-written CUDA behin
 (`include/qed_splat.h`, `libqedsplat.so`); no CPU fallback.
 """
 from .rendering import rasterization  # noqa: F401
-from .losses import depth_supervised_loss  # noqa: F401
+from .losses import bilateral_grid_tv_loss, depth_supervised_loss  # noqa: F401
 from .data_side import get_viewmat  # noqa: F401
 from . import data_side, ops, scenes  # noqa: F401
 

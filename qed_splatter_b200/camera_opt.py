@@ -192,18 +192,22 @@ class CameraPoseOptimizer:
 
     def step(self, step: int) -> None:
         """Adam on the whole table with the scheduled lr of 0-based iteration `step` (bias corrections use step + 1)."""
-        lr = self.lr_at(step)
-        b1, b2 = self.betas
-        t = step + 1
-        if self.backend != "cuda":
-            self.exp_avg.mul_(b1).add_(self.grad, alpha=1 - b1)
-            self.exp_avg_sq.mul_(b2).addcmul_(self.grad, self.grad, value=1 - b2)
-            denom = self.exp_avg_sq.sqrt() / math.sqrt(1.0 - b2 ** t) + self.eps
-            self.param.sub_(lr / (1.0 - b1 ** t) * (self.exp_avg / denom))
-            return
-        from . import _lib
+        adam_table_step(self, self.lr_at(step), step + 1)
 
-        self._lr.fill_(lr)
-        _lib.check(self.lib.qed_adam_arena(self.padded, _lib.ptr(self.param), _lib.ptr(self.grad), _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq),
-                                           1, _lib.ptr(self._ends), _lib.ptr(self._lr), None, None, None, b1, b2, self.eps, t,
-                                           _lib.current_stream()), "qed_adam_arena")
+
+def adam_table_step(tab, lr: float, t: int) -> None:
+    """Adam (torch semantics) over a whole flat table `tab` (param / grad / exp_avg / exp_avg_sq, betas, eps, backend, and
+    for the CUDA backend lib, _lr [1] and _ends [1] on the device): `qed_adam_arena` as a one-group call."""
+    b1, b2 = tab.betas
+    if tab.backend != "cuda":
+        tab.exp_avg.mul_(b1).add_(tab.grad, alpha=1 - b1)
+        tab.exp_avg_sq.mul_(b2).addcmul_(tab.grad, tab.grad, value=1 - b2)
+        denom = tab.exp_avg_sq.sqrt() / math.sqrt(1.0 - b2 ** t) + tab.eps
+        tab.param.sub_(lr / (1.0 - b1 ** t) * (tab.exp_avg / denom))
+        return
+    from . import _lib
+
+    tab._lr.fill_(lr)
+    _lib.check(tab.lib.qed_adam_arena(tab.param.numel(), _lib.ptr(tab.param), _lib.ptr(tab.grad), _lib.ptr(tab.exp_avg), _lib.ptr(tab.exp_avg_sq),
+                                      1, _lib.ptr(tab._ends), _lib.ptr(tab._lr), None, None, None, b1, b2, tab.eps, t,
+                                      _lib.current_stream()), "qed_adam_arena")

@@ -75,15 +75,82 @@ __global__ void __launch_bounds__(kLossThreads) loss_stats_kernel(int64_t HW, co
 
 __device__ __forceinline__ double n_valid_of(const double* s, float maxd) { return s[2] + (finitef(maxd) ? s[6] : 0.0); }
 
+// ---- splatfacto's bilateral grid (nerfstudio lib_bilagrid `slice`), applied to the clamped rgb of training views ----
+// grids[G,12,L,Y,X]: per training image a 3x4 affine colour matrix A[i][j] = ch[4i+j] on an X x Y x L lattice.  A pixel
+// (row h, column w) looks up x = w/(W-1), y = h/(H-1), z = BT.601 gray of its colour, as grid_sample(align_corners=True,
+// padding_mode="border") does: g = coordinate * (n-1), clamped to [0, n-1]; trilinear over the 8 neighbouring cells.
+constexpr int kBilagridMaxL = 16;
+constexpr int kBilagridMaxXY = 1024;
+
+struct BilagridArgs {
+    const float* grids;     // [G,12,L,Y,X]
+    const int32_t* ids;     // [C] grid of each view
+    int num_grids, W, H, X, Y, L;
+    float4* rec_c;          // [C*HW] per pixel {c0, c1, c2, gz} (workspace; written by the gradient pass)
+    float4* rec_v;          // [C*HW] per pixel {d loss / d out (3), 0}
+};
+
+// lattice coordinate of pixel index p of an axis of n_px pixels on an axis of n cells: cell i0 in [0, n-2] and weight f
+// of cell i0 + 1 (f = 1 on the last cell, which grid_sample reaches with weight 1 as well)
+__device__ __forceinline__ void bilagrid_axis(int p, int n_px, int n, int& i0, float& f) {
+    const float x = n_px > 1 ? (float)p / (float)(n_px - 1) : 0.0f;
+    const float g = fminf(fmaxf(x * (float)(n - 1), 0.0f), (float)(n - 1));
+    i0 = min((int)floorf(g), n - 2);
+    f = g - (float)i0;
+}
+
+__device__ __forceinline__ float bilagrid_gz(float c0, float c1, float c2, int L, bool& inside) {
+    const float gz = (0.299f * c0 + 0.587f * c1 + 0.114f * c2) * (float)(L - 1);
+    inside = gz >= 0.0f && gz <= (float)(L - 1);  // grid_sample's border padding: no gradient through a clamped coordinate
+    return fminf(fmaxf(gz, 0.0f), (float)(L - 1));
+}
+
+// A[12] (trilinear) at pixel (h, w) with guidance gz of the view's grid g (NULL: NaN, an invalid id), and
+// dout[3] = d out_i / d gz for the colour c
+__device__ __forceinline__ void bilagrid_sample(const float* __restrict__ g, int X, int Y, int L, int h, int w, int H, int W, float gz,
+                                                float c0, float c1, float c2, float A[12], float dout[3]) {
+    int x0, y0;
+    float fx, fy;
+    bilagrid_axis(w, W, X, x0, fx);
+    bilagrid_axis(h, H, Y, y0, fy);
+    const int z0 = min((int)floorf(gz), L - 2);
+    const float fz = gz - (float)z0;
+    const int64_t sz = (int64_t)X * Y, sc = sz * L;
+    const float wxy[4] = {(1.0f - fx) * (1.0f - fy), fx * (1.0f - fy), (1.0f - fx) * fy, fx * fy};
+    const int64_t oxy[4] = {(int64_t)y0 * X + x0, (int64_t)y0 * X + x0 + 1, (int64_t)(y0 + 1) * X + x0, (int64_t)(y0 + 1) * X + x0 + 1};
+#pragma unroll
+    for (int ch = 0; ch < 12; ++ch) {
+        float a = 0.0f, d = 0.0f;
+        if (g) {
+            const float* gc = g + ch * sc + (int64_t)z0 * sz;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const float lo = __ldg(gc + oxy[k]), hi = __ldg(gc + sz + oxy[k]);
+                a += wxy[k] * ((1.0f - fz) * lo + fz * hi);
+                d += wxy[k] * (hi - lo);
+            }
+        } else {
+            a = d = __int_as_float(0x7fffffff);
+        }
+        A[ch] = a;
+        const float cj = (ch & 3) == 0 ? c0 : ((ch & 3) == 1 ? c1 : ((ch & 3) == 2 ? c2 : 1.0f));
+        if ((ch & 3) == 0) dout[ch >> 2] = d * cj;
+        else dout[ch >> 2] += d * cj;
+    }
+}
+
 // pass 2 (68 B/pixel): per-pixel loss terms and their gradient w.r.t. the compositor outputs.
 //   WRITE_PRED : only write the clamped rgb image (input of the SSIM kernels), no sums, no gradients
 //   otherwise  : loss sums + gradients (v_rgb_extra = gradient of the SSIM term w.r.t. the clamped rgb, or NULL)
-template <bool WRITE_PRED>
+//   BILAGRID   : the loss sees the clamped rgb after the view's bilateral grid; the gradient pass chains through the slice
+//                and leaves per-pixel records for bilagrid_grad_kernel
+template <bool WRITE_PRED, bool BILAGRID = false>
 __global__ void __launch_bounds__(kLossThreads) loss_grad_kernel(int64_t HW, int C, const float4* __restrict__ render, const float* __restrict__ alphas,
                                                                 const GtImage gt_rgb, const GtDepth gt_depth, const PixelMask mask,
                                                                 const float* __restrict__ bg, float rgb_weight, float depth_lambda, float grad_scale,
                                                                 double* __restrict__ stats, float4* __restrict__ v_render, float* __restrict__ v_alphas,
-                                                                float* __restrict__ pred_rgb, const float* __restrict__ v_rgb_extra) {
+                                                                float* __restrict__ pred_rgb, const float* __restrict__ v_rgb_extra,
+                                                                const BilagridArgs bla = BilagridArgs{}) {
     pdl_enter();
     const int cam = blockIdx.y;
     const float maxd = __int_as_float(*reinterpret_cast<const int*>(stats + cam * 8 + 3));
@@ -104,14 +171,26 @@ __global__ void __launch_bounds__(kLossThreads) loss_grad_kernel(int64_t HW, int
         const float pre0 = r.x + om * b0, pre1 = r.y + om * b1, pre2 = r.z + om * b2;
         const float c0 = fminf(fmaxf(pre0, 0.0f), 1.0f), c1 = fminf(fmaxf(pre1, 0.0f), 1.0f), c2 = fminf(fmaxf(pre2, 0.0f), 1.0f);
         const float mk = mask.at(pix);  // 1 without a mask: every product below is then exact
+        float o0 = c0, o1 = c1, o2 = c2;  // the colour the loss sees
+        float A[BILAGRID ? 12 : 1], dout[3], gz = 0.0f;
+        bool z_in = false;
+        if constexpr (BILAGRID) {
+            const int gid = bla.ids[cam];
+            const float* g = (gid >= 0 && gid < bla.num_grids) ? bla.grids + (int64_t)gid * 12 * bla.L * bla.Y * bla.X : nullptr;
+            gz = bilagrid_gz(c0, c1, c2, bla.L, z_in);
+            bilagrid_sample(g, bla.X, bla.Y, bla.L, (int)(i / bla.W), (int)(i % bla.W), bla.H, bla.W, gz, c0, c1, c2, A, dout);
+            o0 = A[0] * c0 + A[1] * c1 + A[2] * c2 + A[3];
+            o1 = A[4] * c0 + A[5] * c1 + A[6] * c2 + A[7];
+            o2 = A[8] * c0 + A[9] * c1 + A[10] * c2 + A[11];
+        }
         if (WRITE_PRED) {  // splatfacto multiplies prediction and ground truth by the mask before L1 and SSIM
-            pred_rgb[pix * 3 + 0] = c0 * mk;
-            pred_rgb[pix * 3 + 1] = c1 * mk;
-            pred_rgb[pix * 3 + 2] = c2 * mk;
+            pred_rgb[pix * 3 + 0] = o0 * mk;
+            pred_rgb[pix * 3 + 1] = o1 * mk;
+            pred_rgb[pix * 3 + 2] = o2 * mk;
             continue;
         }
-        const float e0 = __fmul_rn(c0, mk) - __fmul_rn(gt_rgb.at(pix * 3 + 0), mk), e1 = __fmul_rn(c1, mk) - __fmul_rn(gt_rgb.at(pix * 3 + 1), mk),
-                    e2 = __fmul_rn(c2, mk) - __fmul_rn(gt_rgb.at(pix * 3 + 2), mk);
+        const float e0 = __fmul_rn(o0, mk) - __fmul_rn(gt_rgb.at(pix * 3 + 0), mk), e1 = __fmul_rn(o1, mk) - __fmul_rn(gt_rgb.at(pix * 3 + 1), mk),
+                    e2 = __fmul_rn(o2, mk) - __fmul_rn(gt_rgb.at(pix * 3 + 2), mk);
         const float gd = __fmul_rn(gt_depth.at(pix), mk);              // model.py:96-97
         const float d = __fmul_rn((a > 0.0f) ? r.w : maxd, mk);
         const bool valid = finitef(d) && finitef(gd) && (gd > 0.0f);
@@ -125,9 +204,23 @@ __global__ void __launch_bounds__(kLossThreads) loss_grad_kernel(int64_t HW, int
         }
         const float gm_rgb = g_rgb * mk, gm_d = g_d * mk;
         float4 v;
-        v.x = (pre0 >= 0.0f && pre0 <= 1.0f) ? gm_rgb * signf(e0) + x0 : 0.0f;
-        v.y = (pre1 >= 0.0f && pre1 <= 1.0f) ? gm_rgb * signf(e1) + x1 : 0.0f;
-        v.z = (pre2 >= 0.0f && pre2 <= 1.0f) ? gm_rgb * signf(e2) + x2 : 0.0f;
+        if constexpr (BILAGRID) {
+            // d loss / d out, then through out_i = sum_j A[i][j] c_j + A[i][3] (A depends on c through gz) to c
+            const float u0 = gm_rgb * signf(e0) + x0, u1 = gm_rgb * signf(e1) + x1, u2 = gm_rgb * signf(e2) + x2;
+            bla.rec_c[pix] = make_float4(c0, c1, c2, gz);
+            bla.rec_v[pix] = make_float4(u0, u1, u2, 0.0f);
+            float vz = 0.0f;
+            if (z_in) vz = (u0 * dout[0] + u1 * dout[1] + u2 * dout[2]) * (float)(bla.L - 1);
+            const float w0 = u0 * A[0] + u1 * A[4] + u2 * A[8] + 0.299f * vz, w1 = u0 * A[1] + u1 * A[5] + u2 * A[9] + 0.587f * vz,
+                        w2 = u0 * A[2] + u1 * A[6] + u2 * A[10] + 0.114f * vz;
+            v.x = (pre0 >= 0.0f && pre0 <= 1.0f) ? w0 : 0.0f;
+            v.y = (pre1 >= 0.0f && pre1 <= 1.0f) ? w1 : 0.0f;
+            v.z = (pre2 >= 0.0f && pre2 <= 1.0f) ? w2 : 0.0f;
+        } else {
+            v.x = (pre0 >= 0.0f && pre0 <= 1.0f) ? gm_rgb * signf(e0) + x0 : 0.0f;
+            v.y = (pre1 >= 0.0f && pre1 <= 1.0f) ? gm_rgb * signf(e1) + x1 : 0.0f;
+            v.z = (pre2 >= 0.0f && pre2 <= 1.0f) ? gm_rgb * signf(e2) + x2 : 0.0f;
+        }
         v.w = (valid && a > 0.0f) ? gm_d * signf(d - gd) : 0.0f;
         v_render[pix] = v;
         v_alphas[pix] = -(v.x * b0 + v.y * b1 + v.z * b2);
@@ -175,6 +268,89 @@ __global__ void loss_finalize_kernel(int C, int64_t HW, float rgb_weight, float 
     loss[0] = (float)(lr + ld);
     loss[1] = (float)lr;
     loss[2] = (float)ld;
+}
+
+// Bilateral-grid gradient, gathered: one block per (lattice column (ix, iy), ROWS output rows of A starting at blockIdx.y *
+// ROWS, view).  It visits the pixels whose x / y cell touches the column, in a fixed order (warps over consecutive columns of
+// an image row), and keeps sum_pixels w * d loss / d out_i * [c, 1] for every level of the column in registers; then a
+// fixed-order block reduction (xor shuffles, warps in order) writes the ROWS x 4 x L values.  No atomics: the same inputs
+// give the same bits.  v_grid_rows[C,12,L,Y,X] is overwritten.
+constexpr int kBilagridThreads = 256;
+
+template <int LM, int ROWS>
+__global__ void __launch_bounds__(kBilagridThreads) bilagrid_grad_kernel(int64_t HW, const BilagridArgs bla, float* __restrict__ v_rows) {
+    __shared__ float s_part[kBilagridThreads / 32][ROWS * 4 * LM];
+    pdl_enter();
+    const int X = bla.X, Y = bla.Y, L = bla.L, W = bla.W, H = bla.H;
+    const int ix = blockIdx.x % X, iy = blockIdx.x / X, row0 = blockIdx.y * ROWS, cam = blockIdx.z;
+    // pixels whose cell is ix-1 or ix (resp. iy-1 or iy), with one pixel of slack each side; the weights decide exactly
+    auto span = [](int i, int n, int n_px, int& lo, int& hi) {
+        const double s = n_px > 1 ? (double)(n_px - 1) / (double)(n - 1) : 0.0;
+        lo = max(0, (int)floor((i - 1) * s) - 1);
+        hi = min(n_px - 1, (int)ceil((i + 1) * s) + 1);
+    };
+    int w_lo, w_hi, h_lo, h_hi;
+    span(ix, X, W, w_lo, w_hi);
+    span(iy, Y, H, h_lo, h_hi);
+    float acc[ROWS][LM][4];
+#pragma unroll
+    for (int r = 0; r < ROWS; ++r)
+#pragma unroll
+        for (int l = 0; l < LM; ++l)
+#pragma unroll
+            for (int j = 0; j < 4; ++j) acc[r][l][j] = 0.0f;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int w = w_lo + lane; w <= w_hi; w += 32) {
+        int x0;
+        float fx;
+        bilagrid_axis(w, W, X, x0, fx);
+        const float wx = x0 == ix ? 1.0f - fx : (x0 + 1 == ix ? fx : 0.0f);
+        if (wx == 0.0f) continue;
+        for (int h = h_lo + warp; h <= h_hi; h += kBilagridThreads / 32) {
+            int y0;
+            float fy;
+            bilagrid_axis(h, H, Y, y0, fy);
+            const float wy = y0 == iy ? 1.0f - fy : (y0 + 1 == iy ? fy : 0.0f);
+            if (wy == 0.0f) continue;
+            const int64_t pix = (int64_t)cam * HW + (int64_t)h * W + w;
+            const float4 c = bla.rec_c[pix];
+            const float4 u = bla.rec_v[pix];
+            const int z0 = min((int)floorf(c.w), L - 2);
+            const float fz = c.w - (float)z0, wxy = wx * wy;
+#pragma unroll
+            for (int r = 0; r < ROWS; ++r) {
+                const int row = row0 + r;
+                const float val = wxy * (row == 0 ? u.x : (row == 1 ? u.y : u.z));
+                const float a0 = (1.0f - fz) * val, a1 = fz * val;
+#pragma unroll
+                for (int l = 0; l < LM; ++l) {
+                    const float wl = l == z0 ? a0 : (l == z0 + 1 ? a1 : 0.0f);
+                    acc[r][l][0] += wl * c.x;
+                    acc[r][l][1] += wl * c.y;
+                    acc[r][l][2] += wl * c.z;
+                    acc[r][l][3] += wl;
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int r = 0; r < ROWS; ++r)
+#pragma unroll
+        for (int l = 0; l < LM; ++l)
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                float a = acc[r][l][j];
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
+                if (lane == 0) s_part[warp][(r * LM + l) * 4 + j] = a;
+            }
+    __syncthreads();
+    for (int t = threadIdx.x; t < ROWS * 4 * L; t += kBilagridThreads) {
+        const int r = t / (4 * L), l = (t >> 2) % L, j = t & 3, k = (r * LM + l) * 4 + j;
+        float a = s_part[0][k];
+        for (int wp = 1; wp < kBilagridThreads / 32; ++wp) a += s_part[wp][k];
+        v_rows[(((int64_t)cam * 12 + (row0 + r) * 4 + j) * L + l) * Y * X + (int64_t)iy * X + ix] = a;
+    }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -297,12 +473,14 @@ extern "C" size_t qed_loss_workspace_bytes(int C, int width, int height, float s
     return px * 3 * 4 /* clamped rgb */ + px * 9 * 4 /* derivative maps (upper bound) */ + px * 3 * 4 /* v_ssim */;
 }
 
-extern "C" int qed_loss_fwd_bwd(int C, int width, int height, const float* render, const float* alphas,
-                                const void* gt_rgb_, int gt_rgb_is_u8, const void* gt_depth_, int gt_depth_is_u16, double depth_unit_scale,
-                                const void* mask_, int mask_is_u8, const float* bg, float rgb_weight,
-                                float depth_lambda, float ssim_lambda, float grad_scale, double* stats_dev, float* loss_dev,
-                                float* v_render, float* v_alphas, void* workspace, size_t workspace_bytes, qed_stream_t stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
+// qed_loss_fwd_bwd, and with `bla` the same loss on the bilateral-grid-corrected colour.  The workspace of the grid variant
+// starts with its 32 B/pixel records; the SSIM buffers follow.
+template <bool BILAGRID>
+static int loss_fwd_bwd(int C, int width, int height, const float* render, const float* alphas, const void* gt_rgb_, int gt_rgb_is_u8,
+                        const void* gt_depth_, int gt_depth_is_u16, double depth_unit_scale, const void* mask_, int mask_is_u8, const float* bg,
+                        float rgb_weight, float depth_lambda, float ssim_lambda, float grad_scale, double* stats_dev, float* loss_dev,
+                        float* v_render, float* v_alphas, BilagridArgs bla, float* v_grid_rows, void* workspace, size_t workspace_bytes,
+                        cudaStream_t stream) {
     if (C <= 0 || width <= 0 || height <= 0) return QED_ERR_BAD_ARG;
     if (!render || !alphas || !gt_rgb_ || !gt_depth_ || !bg || !stats_dev || !loss_dev || !v_render || !v_alphas) return QED_ERR_BAD_ARG;
     const GtImage gt_rgb{gt_rgb_, gt_rgb_is_u8 ? 1 : 0};
@@ -310,13 +488,19 @@ extern "C" int qed_loss_fwd_bwd(int C, int width, int height, const float* rende
     const GtDepth gt_depth{gt_depth_, gt_depth_is_u16 ? 1 : 0, depth_unit_scale};
     if (C > 21845) return QED_ERR_UNSUPPORTED;
     const bool use_ssim = ssim_lambda > 0.0f;
-    if (use_ssim) {
-        if (!workspace) return QED_ERR_BAD_ARG;
-        if (workspace_bytes < qed_loss_workspace_bytes(C, width, height, ssim_lambda)) return QED_ERR_WORKSPACE;
-        if (width <= 10 || height <= 10) return QED_ERR_UNSUPPORTED;
-    }
     const int64_t HW = (int64_t)width * height;
     const size_t px = (size_t)C * HW;
+    const size_t rec_bytes = BILAGRID ? px * 2 * sizeof(float4) : 0;
+    if (use_ssim || BILAGRID) {
+        if (!workspace) return QED_ERR_BAD_ARG;
+        if (workspace_bytes < rec_bytes + qed_loss_workspace_bytes(C, width, height, ssim_lambda)) return QED_ERR_WORKSPACE;
+    }
+    if (use_ssim && (width <= 10 || height <= 10)) return QED_ERR_UNSUPPORTED;
+    if (BILAGRID) {
+        bla.rec_c = reinterpret_cast<float4*>(workspace);
+        bla.rec_v = bla.rec_c + px;
+        workspace = reinterpret_cast<char*>(workspace) + rec_bytes;
+    }
     float* pred_rgb = use_ssim ? reinterpret_cast<float*>(workspace) : nullptr;
     float* dmaps = use_ssim ? pred_rgb + px * 3 : nullptr;
     float* v_ssim = use_ssim ? dmaps + px * 9 : nullptr;
@@ -327,20 +511,61 @@ extern "C" int qed_loss_fwd_bwd(int C, int width, int height, const float* rende
                             stats_dev));
     const double ssim_count = (double)(width - 10) * (double)(height - 10) * 3.0;
     if (use_ssim) {
-        QED_CUDA_TRY(launch_pdl(loss_grad_kernel<true>, grid, dim3(kLossThreads), 0, stream, HW, C, reinterpret_cast<const float4*>(render), alphas, gt_rgb,
-                                gt_depth, mask, bg, rgb_weight, depth_lambda, grad_scale, stats_dev, (float4*)nullptr, (float*)nullptr, pred_rgb,
-                                (const float*)nullptr));
+        QED_CUDA_TRY(launch_pdl(loss_grad_kernel<true, BILAGRID>, grid, dim3(kLossThreads), 0, stream, HW, C, reinterpret_cast<const float4*>(render), alphas,
+                                gt_rgb, gt_depth, mask, bg, rgb_weight, depth_lambda, grad_scale, stats_dev, (float4*)nullptr, (float*)nullptr, pred_rgb,
+                                (const float*)nullptr, bla));
         // loss term = ssim_lambda * (1 - mean(map)) per camera, mean over cameras
         const float scale = -ssim_lambda * grad_scale / ((float)C * (float)ssim_count);
         int rc = qed_ssim_launch(C, width, height, pred_rgb, gt_rgb, mask, dmaps, stats_dev, scale, v_ssim, stream);
         if (rc != QED_OK) return rc;
     }
-    QED_CUDA_TRY(launch_pdl(loss_grad_kernel<false>, grid, dim3(kLossThreads), 0, stream, HW, C, reinterpret_cast<const float4*>(render), alphas, gt_rgb,
-                            gt_depth, mask, bg, rgb_weight, depth_lambda, grad_scale, stats_dev, reinterpret_cast<float4*>(v_render), v_alphas,
-                            (float*)nullptr, (const float*)v_ssim));
+    QED_CUDA_TRY(launch_pdl(loss_grad_kernel<false, BILAGRID>, grid, dim3(kLossThreads), 0, stream, HW, C, reinterpret_cast<const float4*>(render), alphas,
+                            gt_rgb, gt_depth, mask, bg, rgb_weight, depth_lambda, grad_scale, stats_dev, reinterpret_cast<float4*>(v_render), v_alphas,
+                            (float*)nullptr, (const float*)v_ssim, bla));
+    if (BILAGRID) {
+        // all three output rows per block while their L x 12 sums fit in registers, one row per block above 8 levels
+        if (bla.L <= 8)
+            QED_CUDA_TRY(launch_pdl(bilagrid_grad_kernel<8, 3>, dim3((unsigned)(bla.X * bla.Y), 1, (unsigned)C), dim3(kBilagridThreads), 0, stream, HW,
+                                    (const BilagridArgs)bla, v_grid_rows));
+        else
+            QED_CUDA_TRY(launch_pdl(bilagrid_grad_kernel<kBilagridMaxL, 1>, dim3((unsigned)(bla.X * bla.Y), 3, (unsigned)C), dim3(kBilagridThreads), 0,
+                                    stream, HW, (const BilagridArgs)bla, v_grid_rows));
+    }
     QED_CUDA_TRY(launch_pdl(loss_finalize_kernel, dim3(1), dim3(32), 0, stream, C, HW, rgb_weight, depth_lambda, use_ssim ? ssim_lambda : 0.0f, ssim_count,
                             stats_dev, loss_dev));
     return QED_OK;
+}
+
+extern "C" int qed_loss_fwd_bwd(int C, int width, int height, const float* render, const float* alphas,
+                                const void* gt_rgb_, int gt_rgb_is_u8, const void* gt_depth_, int gt_depth_is_u16, double depth_unit_scale,
+                                const void* mask_, int mask_is_u8, const float* bg, float rgb_weight,
+                                float depth_lambda, float ssim_lambda, float grad_scale, double* stats_dev, float* loss_dev,
+                                float* v_render, float* v_alphas, void* workspace, size_t workspace_bytes, qed_stream_t stream_) {
+    return loss_fwd_bwd<false>(C, width, height, render, alphas, gt_rgb_, gt_rgb_is_u8, gt_depth_, gt_depth_is_u16, depth_unit_scale, mask_, mask_is_u8, bg,
+                               rgb_weight, depth_lambda, ssim_lambda, grad_scale, stats_dev, loss_dev, v_render, v_alphas, BilagridArgs{}, nullptr,
+                               workspace, workspace_bytes, (cudaStream_t)stream_);
+}
+
+extern "C" size_t qed_loss_bilagrid_workspace_bytes(int C, int width, int height, float ssim_lambda) {
+    if (C <= 0 || width <= 0 || height <= 0) return 0;
+    return (size_t)C * width * height * 2 * sizeof(float4) + qed_loss_workspace_bytes(C, width, height, ssim_lambda);
+}
+
+extern "C" int qed_loss_fwd_bwd_bilagrid(int C, int width, int height, const float* render, const float* alphas,
+                                         const void* gt_rgb, int gt_rgb_is_u8, const void* gt_depth, int gt_depth_is_u16, double depth_unit_scale,
+                                         const void* mask, int mask_is_u8, const float* bg, float rgb_weight,
+                                         float depth_lambda, float ssim_lambda, float grad_scale, double* stats_dev, float* loss_dev,
+                                         float* v_render, float* v_alphas, const float* grids, const int32_t* grid_ids, int num_grids,
+                                         int grid_X, int grid_Y, int grid_L, float* v_grid_rows, void* workspace, size_t workspace_bytes,
+                                         qed_stream_t stream_) {
+    if (!grids || !grid_ids || !v_grid_rows || num_grids <= 0) return QED_ERR_BAD_ARG;
+    if (grid_X < 2 || grid_Y < 2 || grid_L < 2 || grid_X > kBilagridMaxXY || grid_Y > kBilagridMaxXY || grid_L > kBilagridMaxL) return QED_ERR_UNSUPPORTED;
+    if ((int64_t)grid_X * grid_Y * grid_L * 12 * num_grids > 0x7fffffffLL) return QED_ERR_UNSUPPORTED;
+    if (C > 65535) return QED_ERR_UNSUPPORTED;
+    BilagridArgs bla{grids, grid_ids, num_grids, width, height, grid_X, grid_Y, grid_L, nullptr, nullptr};
+    return loss_fwd_bwd<true>(C, width, height, render, alphas, gt_rgb, gt_rgb_is_u8, gt_depth, gt_depth_is_u16, depth_unit_scale, mask, mask_is_u8, bg,
+                              rgb_weight, depth_lambda, ssim_lambda, grad_scale, stats_dev, loss_dev, v_render, v_alphas, bla, v_grid_rows, workspace,
+                              workspace_bytes, (cudaStream_t)stream_);
 }
 
 extern "C" int qed_adam_arena(int64_t n, float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int G,

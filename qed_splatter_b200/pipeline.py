@@ -341,14 +341,18 @@ class FusedSplatStep:
              depth_lambda: float = 0.2, grad_scale: float = 1.0, rasterize_mode: str = "classic",
              grad_out: Optional[Dict[str, Tensor]] = None, ssim_lambda: float = 0.0, n_chunks: int = 1, on_chunk=None,
              activations: int = 0, mask: Optional[Tensor] = None, exchange=None, depth_unit_scale: float = 0.001,
-             pose_gradients: bool = False) -> StepOutput:
+             pose_gradients: bool = False, bilateral_grid=None) -> StepOutput:
         """`render_mode` RGB+ED (north_star) or RGB+D (what qed_splatter/model.py:257 passes).
         loss = rgb_weight * L1 + ssim_lambda * (1 - SSIM) + depth_lambda * masked depth-L1 (splatfacto: 0.8 / 0.2 / 0.2).
         `mask` [C,H,W(,1)] float32 / uint8 / bool = `batch["mask"]` (model.py:93-97), see losses.depth_supervised_loss.
         The returned StepOutput aliases buffers this object reuses: the next step() overwrites loss / render / alphas /
         packed_grads / radii / v_viewmats in place -- clone() what must outlive the step.
         `pose_gradients=True`: StepOutput.v_viewmats [C,4,4] = d loss / d viewmats (camera optimisation); not with
-        `n_chunks` > 1, and with `exchange` only when it was built with pose capacity (num_cameras > 0)."""
+        `n_chunks` > 1, and with `exchange` only when it was built with pose capacity (num_cameras > 0).
+        `bilateral_grid=(grids, grid_ids, v_grid_rows)`: splatfacto's bilateral grid on every view before the RGB loss
+        (qed_loss_fwd_bwd_bilagrid): grids [G,12,L,Y,X] float32, grid_ids [C] int32 on the device (validated by the caller),
+        v_grid_rows [C,12,L,Y,X] overwritten with each view's grid gradient.  Only the loss stage changes, so it combines
+        with `n_chunks` and `exchange`."""
         assert render_mode in ("RGB+D", "RGB+ED")
         if pose_gradients and (n_chunks > 1 or not _pose_capable(exchange)):
             raise ValueError("pose_gradients=True is not available with n_chunks > 1 or an exchange without pose capacity")
@@ -378,12 +382,23 @@ class FusedSplatStep:
             self._prezeroed, self._prezero = self._prezero, False
             v_render = self._get("v_render", (C, height, width, 4))
             v_alphas = self._get("v_alphas", (C, height, width, 1))
-            lws_bytes = lib.qed_loss_workspace_bytes(C, width, height, ssim_lambda)
-            lws = self._get("loss_ws", (lws_bytes,), torch.uint8) if lws_bytes else None
-            check(lib.qed_loss_fwd_bwd(C, width, height, ptr(render), ptr(alphas), ptr(gt_rgb), int(gt_rgb.dtype == torch.uint8), ptr(gt_depth), int(gt_depth.dtype != torch.float32),
-                                       float(depth_unit_scale), ptr(mask), int(mask is not None and mask.dtype == torch.uint8), ptr(background), rgb_weight,
-                                       depth_lambda, ssim_lambda, grad_scale, ptr(self._stats), ptr(self._loss), ptr(v_render), ptr(v_alphas),
-                                       ptr(lws), lws_bytes, stream), "qed_loss_fwd_bwd")
+            if bilateral_grid is None:
+                lws_bytes = lib.qed_loss_workspace_bytes(C, width, height, ssim_lambda)
+                lws = self._get("loss_ws", (lws_bytes,), torch.uint8) if lws_bytes else None
+                check(lib.qed_loss_fwd_bwd(C, width, height, ptr(render), ptr(alphas), ptr(gt_rgb), int(gt_rgb.dtype == torch.uint8), ptr(gt_depth), int(gt_depth.dtype != torch.float32),
+                                           float(depth_unit_scale), ptr(mask), int(mask is not None and mask.dtype == torch.uint8), ptr(background), rgb_weight,
+                                           depth_lambda, ssim_lambda, grad_scale, ptr(self._stats), ptr(self._loss), ptr(v_render), ptr(v_alphas),
+                                           ptr(lws), lws_bytes, stream), "qed_loss_fwd_bwd")
+            else:
+                grids, ids, rows = bilateral_grid
+                G, _, L, Y, X = grids.shape
+                lws_bytes = lib.qed_loss_bilagrid_workspace_bytes(C, width, height, ssim_lambda)
+                lws = self._get("loss_ws", (lws_bytes,), torch.uint8)
+                check(lib.qed_loss_fwd_bwd_bilagrid(C, width, height, ptr(render), ptr(alphas), ptr(gt_rgb), int(gt_rgb.dtype == torch.uint8), ptr(gt_depth),
+                                                    int(gt_depth.dtype != torch.float32), float(depth_unit_scale), ptr(mask),
+                                                    int(mask is not None and mask.dtype == torch.uint8), ptr(background), rgb_weight, depth_lambda, ssim_lambda,
+                                                    grad_scale, ptr(self._stats), ptr(self._loss), ptr(v_render), ptr(v_alphas), ptr(grids), ptr(ids), G, X,
+                                                    Y, L, ptr(rows), ptr(lws), lws_bytes, stream), "qed_loss_fwd_bwd_bilagrid")
             self._mark("loss")
             return render, alphas, v_render, v_alphas
 

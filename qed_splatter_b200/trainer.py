@@ -92,6 +92,15 @@ class TrainConfig:
     camera_opt_warmup: int = 1000  # [UP] warm-up steps from lr 0 (cosine ramp)
     camera_opt_trans_l2_penalty: float = 1e-2  # [UP] weight of mean_rows |t| in the loss
     camera_opt_rot_l2_penalty: float = 1e-3  # [UP] weight of mean_rows |omega| in the loss
+    # splatfacto's bilateral grid (bilateral_grid.py): one affine colour grid per training camera, applied to the training
+    # views before the RGB loss; SplatTrainer(num_cameras=...), step(..., camera_ids=).  [UP] = nerfstudio >= 1.1.4 defaults
+    # restated from memory of the upstream code (splatfacto's "bilateral_grid" param group and tv loss).
+    use_bilateral_grid: bool = False
+    bilateral_grid_shape: Tuple[int, int, int] = (16, 16, 8)  # [UP] (X, Y, L) = grid_X, grid_Y, grid_W
+    bilateral_grid_lr: float = 2e-3  # [UP] Adam lr (eps = adam_eps 1e-15 [UP])
+    bilateral_grid_lr_final: float = 1e-4  # [UP] ExponentialDecayScheduler lr_final, reached at max_steps
+    bilateral_grid_warmup: int = 1000  # [UP] warm-up steps from lr 0
+    bilateral_grid_tv_weight: float = 10.0  # [UP] weight of the total-variation loss
 
     def __post_init__(self):
         self.validate()
@@ -102,6 +111,15 @@ class TrainConfig:
 
         if self.camera_optimizer not in CAMERA_OPTIMIZER_MODES:
             raise ValueError(f"camera_optimizer must be one of {CAMERA_OPTIMIZER_MODES}, got {self.camera_optimizer!r}")
+        if self.use_bilateral_grid:
+            from .bilateral_grid import check_grid_shape
+
+            shape = tuple(self.bilateral_grid_shape)
+            if len(shape) != 3 or not all(isinstance(v, int) for v in shape):
+                raise ValueError(f"bilateral_grid_shape must be three ints (X, Y, L), got {self.bilateral_grid_shape!r}")
+            check_grid_shape(*shape)
+            if self.bilateral_grid_lr < 0 or self.bilateral_grid_lr_final <= 0 or self.bilateral_grid_warmup < 0 or self.bilateral_grid_tv_weight < 0:
+                raise ValueError("bilateral grid: lr >= 0, lr_final > 0, warmup >= 0 and tv_weight >= 0 expected")
 
     def lr_means_at(self, step: int) -> float:
         """nerfstudio ExponentialDecayScheduler (no warmup): log-linear from lr to lr_final over max_steps."""
@@ -408,7 +426,8 @@ class SplatTrainer:
     def __init__(self, means: Tensor, quats: Tensor, log_scales: Tensor, logit_opacities: Tensor, sh: Tensor,
                  cfg: Optional[TrainConfig] = None, rank: int = 0, world_size: int = 1, process_group=None,
                  backend: str = "cuda", num_cameras: int = 0):
-        """`num_cameras`: rows of the camera optimizer's pose table (the training cameras; cfg.camera_optimizer != "off")."""
+        """`num_cameras`: the training cameras: rows of the camera optimizer's pose table (cfg.camera_optimizer != "off") and
+        the number of bilateral grids (cfg.use_bilateral_grid)."""
         self.cfg = cfg or TrainConfig()
         self.cfg.validate()  # fields may have been changed after construction
         self.rank, self.world = rank, world_size
@@ -435,6 +454,17 @@ class SplatTrainer:
                                                   warmup_steps=c.camera_opt_warmup, max_steps=c.max_steps,
                                                   trans_weight=c.camera_opt_trans_l2_penalty, rot_weight=c.camera_opt_rot_l2_penalty,
                                                   betas=c.adam_betas, eps=c.adam_eps, backend=backend)
+        self.bilagrid = None
+        self._bg_buf = None  # rows + ids of the whole view batch ("nccl" / one rank; the exchange keeps its own, symmetric)
+        if self.cfg.use_bilateral_grid:
+            from .bilateral_grid import BilateralGridOptimizer
+
+            c = self.cfg
+            if num_cameras < 1:
+                raise ValueError("the bilateral grid needs num_cameras >= 1")
+            self.bilagrid = BilateralGridOptimizer(num_cameras, self.device, shape=c.bilateral_grid_shape, lr=c.bilateral_grid_lr,
+                                                   lr_final=c.bilateral_grid_lr_final, warmup_steps=c.bilateral_grid_warmup, max_steps=c.max_steps,
+                                                   tv_weight=c.bilateral_grid_tv_weight, betas=c.adam_betas, eps=c.adam_eps, backend=backend)
 
     @property
     def pose_adjustment(self) -> Optional[Tensor]:
@@ -445,6 +475,16 @@ class SplatTrainer:
     def camera_opt_loss(self) -> Optional[Tensor]:
         """The camera optimizer's regulariser of the last step (device scalar [1]); None when it is off."""
         return None if self.camera_opt is None else self.camera_opt.reg_loss
+
+    @property
+    def bilateral_grids(self) -> Optional[Tensor]:
+        """The bilateral grids [num_cameras, 12, L, Y, X]; None when the grid is off."""
+        return None if self.bilagrid is None else self.bilagrid.grids
+
+    @property
+    def bilagrid_tv_loss(self) -> Optional[Tensor]:
+        """The grids' total-variation loss of the last step (device scalar [1]); None when the grid is off."""
+        return None if self.bilagrid is None else self.bilagrid.tv_loss
 
     def _pick_comm(self) -> str:
         c = self.cfg.comm
@@ -473,7 +513,8 @@ class SplatTrainer:
             try:
                 x = ViewShardedGradients(self.arena.N, views_per_rank, self.device, self.pg,
                                          headroom=0.25 if self.step_count < self.cfg.stop_split_at else 0.0,
-                                         num_cameras=0 if self.camera_opt is None else self.camera_opt.num_cameras)
+                                         num_cameras=0 if self.camera_opt is None else self.camera_opt.num_cameras,
+                                         bilagrid_row=0 if self.bilagrid is None else self.bilagrid.row)
             except Exception as e:  # noqa: BLE001  (no peer mappings / symmetric memory on this box)
                 x, err = None, e
             ok = torch.tensor([0.0 if x is None else 1.0], device=self.device)
@@ -589,6 +630,49 @@ class SplatTrainer:
         cam.regularize()
         cam.step(self.step_count)
 
+    def _bilagrid_slots(self, C: int, exchange=None):
+        """-> (buffer, rows [world*C, 12, L, Y, X], ids as floats [world*C], this rank's rows [C, ...]): views of the buffer the
+        ranks sum, the exchange's symmetric one or else an ordinary tensor.  Slots of other ranks are zero."""
+        bg, slots = self.bilagrid, self.world * C
+        n = slots * (bg.row + 1)
+        if exchange is not None:
+            buf = exchange.bilagrid
+        else:
+            if self._bg_buf is None or self._bg_buf.numel() < n:
+                self._bg_buf = torch.zeros(n, device=self.device)
+            buf = self._bg_buf
+        if exchange is not None or self.world > 1:
+            buf.zero_()
+        buf = buf[:n]
+        rows = buf[:slots * bg.row].view(slots, 12, bg.L, bg.Y, bg.X)
+        return buf, rows, buf[slots * bg.row:], rows[self.rank * C:(self.rank + 1) * C]
+
+    def _bilagrid_finish(self, C: int, ids: Tensor, buf: Tensor, rows: Tensor, ids_f: Tensor, exchange) -> None:
+        """After the local rows are written: the ids into their slots, the sum over the ranks, TV (overwrites the dense
+        gradient), every view's row added in global view order, Adam.  Replicas keep bit-identical grids."""
+        bg = self.bilagrid
+        if exchange is not None or self.world > 1:
+            ids_f[self.rank * C:(self.rank + 1) * C].copy_(ids)
+            if exchange is not None:
+                exchange.reduce_bilagrid()  # the whole symmetric buffer; floats past this batch's slots are zero
+            else:
+                self._all_reduce(buf)
+            ids = ids_f.to(torch.int32)
+        bg.regularize()
+        bg.accumulate(ids, rows)
+        bg.step(self.step_count)
+
+    def bilagrid_update(self, v_grid_rows: Tensor, camera_ids: Tensor) -> None:
+        """The bilateral grid's part of a step from this rank's per-view grid gradients v_grid_rows [C,12,L,Y,X] (what the
+        fused step writes; they already carry 1 / total_views): sum over the ranks, TV, accumulate, Adam."""
+        from .camera_opt import check_camera_ids
+
+        C = v_grid_rows.shape[0]
+        ids = check_camera_ids(camera_ids, C, self.bilagrid.num_grids, self.device)
+        buf, rows, ids_f, mine = self._bilagrid_slots(C)
+        mine.copy_(v_grid_rows)
+        self._bilagrid_finish(C, ids, buf, rows, ids_f, None)
+
     def maybe_refine(self, step: int) -> Optional[Dict[str, int]]:
         """DefaultStrategy.step_post_backward schedule, called after the optimizer step of 0-based iteration
         `step` (nerfstudio passes its 0-based step; note gsplat resets opacities at step 0 too)."""
@@ -617,17 +701,27 @@ class SplatTrainer:
         With the camera optimizer on, `viewmats` is None and the views come as `camera_to_worlds` [C,3|4,4] (nerfstudio
         camera-to-world) and `camera_ids` [C] (rows of the pose table); the viewmats are those of the adjusted poses.
         Returns (loss[3] device tensor of the local views -- a fresh copy, safe to keep for logging --, refine info|None);
-        the camera optimizer's regulariser is `camera_opt_loss`."""
+        the camera optimizer's regulariser is `camera_opt_loss`.
+        With the bilateral grid on, `camera_ids` [C] (the training camera of each view, the same ids the camera optimizer
+        uses) selects each view's grid; the grids' TV loss is `bilagrid_tv_loss`."""
         if self._fused is None:
             raise RuntimeError("rendering needs the CUDA library (backend='cuda'); there is no CPU fallback")
-        c, a, cam = self.cfg, self.arena, self.camera_opt
+        c, a, cam, bg = self.cfg, self.arena, self.camera_opt, self.bilagrid
         if cam is not None:
             if viewmats is not None or camera_to_worlds is None or camera_ids is None:
                 raise ValueError("camera optimizer on: pass viewmats=None with camera_to_worlds= and camera_ids=")
             camera_to_worlds, camera_ids = cam.prepare(camera_to_worlds, camera_ids)  # validated once per step
             viewmats = cam._viewmats(camera_to_worlds, camera_ids)
-        elif camera_to_worlds is not None or camera_ids is not None:
-            raise ValueError("camera_to_worlds= / camera_ids= need cfg.camera_optimizer != 'off'")
+        elif camera_to_worlds is not None:
+            raise ValueError("camera_to_worlds= needs cfg.camera_optimizer != 'off'")
+        elif camera_ids is not None and bg is None:
+            raise ValueError("camera_ids= needs cfg.camera_optimizer != 'off' or cfg.use_bilateral_grid")
+        elif bg is not None:
+            from .camera_opt import check_camera_ids
+
+            if camera_ids is None:
+                raise ValueError("bilateral grid on: pass camera_ids= (the training camera of each view)")
+            camera_ids = check_camera_ids(camera_ids, viewmats.shape[0], bg.num_grids, self.device)
         C = viewmats.shape[0]
         total = total_views or C * self.world
         pv = a.views(a.param)
@@ -635,16 +729,22 @@ class SplatTrainer:
         # the stored parameters go straight in: exp / sigmoid (model.py:269-271) and their chain rule run inside the
         # projection kernels, the gradients land in the arena
         xg = self._exchange_for(C) if self.comm == "exchange" else None  # may fall back to "nccl" (comm="auto", no symmetric memory)
+        bl = None
+        if bg is not None:
+            bl = self._bilagrid_slots(C, xg)  # this rank's rows are written by the loss kernels of the fused step
+        bl_arg = None if bl is None else (bg.grids, camera_ids, bl[3])
         if xg is not None:
             out = self._fused.step(pv["means"], pv["quats"], pv["scales"], pv["opacities"], pv["sh"], viewmats, Ks, width, height,
                                    self.sh_degree_to_use(), gt_rgb, gt_depth, background, render_mode=c.render_mode, rgb_weight=1.0 - c.ssim_lambda,
                                    depth_lambda=c.depth_lambda, grad_scale=C / float(total), rasterize_mode=c.rasterize_mode, activations=3,
                                    mask=mask, ssim_lambda=c.ssim_lambda, exchange=xg, depth_unit_scale=c.depth_unit_scale,
-                                   pose_gradients=cam is not None)
+                                   pose_gradients=cam is not None, bilateral_grid=bl_arg)
             self.accumulate_stats(out.packed_grads, out.radii, width, height, packed=True, n_cameras=total)
             self.optimizer_step()
             if cam is not None:
                 self._camera_opt_update(out.v_viewmats, camera_ids, camera_to_worlds, xg)
+            if bg is not None:
+                self._bilagrid_finish(C, camera_ids, *bl[:3], xg)
             loss = out.loss.clone()
             info = self.maybe_refine(self.step_count)
             self.step_count += 1
@@ -668,7 +768,7 @@ class SplatTrainer:
                                activations=3,  # ACT_LOG_SCALES | ACT_LOGIT_OPACITIES (pipeline.py / include/qed_splat.h)
                                mask=mask, depth_unit_scale=c.depth_unit_scale, ssim_lambda=c.ssim_lambda,
                                n_chunks=c.comm_chunks if chunked_bwd else 1, on_chunk=on_chunk if chunked_bwd else None,
-                               pose_gradients=cam is not None)
+                               pose_gradients=cam is not None, bilateral_grid=bl_arg)
         self.accumulate_stats(out.packed_grads, out.radii, width, height, packed=True, n_cameras=total)
         if pipelined:
             import torch.distributed as dist
@@ -688,6 +788,8 @@ class SplatTrainer:
             self.optimizer_step()
         if cam is not None:
             self._camera_opt_update(out.v_viewmats, camera_ids, camera_to_worlds, None)
+        if bg is not None:
+            self._bilagrid_finish(C, camera_ids, *bl[:3], None)
         loss = out.loss.clone()  # out.loss is a buffer the next step overwrites in place
         info = self.maybe_refine(self.step_count)
         self.step_count += 1

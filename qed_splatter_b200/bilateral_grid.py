@@ -16,7 +16,7 @@ from __future__ import annotations
 import torch
 from torch import Tensor
 
-from .camera_opt import adam_table_step, lr_at
+from .camera_opt import AdamTable
 
 # (X, Y, L) bounds of the kernels (include/qed_splat.h, qed_loss_fwd_bwd_bilagrid)
 MAX_XY, MAX_L = 1024, 16
@@ -39,33 +39,20 @@ def total_variation_torch(grids: Tensor, weight: float) -> Tensor:
     return weight * tv / grids.shape[0]
 
 
-class BilateralGridOptimizer:
-    """The grids, their gradient and Adam moments as flat [num_grids * 12 L Y X] buffers."""
+class BilateralGridOptimizer(AdamTable):
+    """The grids (identity at init), their gradient and Adam moments as flat [num_grids * 12 L Y X] buffers."""
 
     def __init__(self, num_grids: int, device, shape=(16, 16, 8), lr: float = 2e-3, lr_final: float = 1e-4, warmup_steps: int = 1000,
                  max_steps: int = 30000, tv_weight: float = 10.0, betas=(0.9, 0.999), eps: float = 1e-15, backend: str = "cuda"):
         X, Y, L = (int(v) for v in shape)
         check_grid_shape(X, Y, L, num_grids)
-        if lr < 0 or lr_final <= 0 or warmup_steps < 0:
-            raise ValueError("bilateral grid: lr >= 0, lr_final > 0 and warmup_steps >= 0 expected")
         self.num_grids, self.X, self.Y, self.L = int(num_grids), X, Y, L
-        self.row = 12 * L * Y * X
-        self.backend = backend
-        self.lr, self.lr_final, self.warmup_steps, self.max_steps = lr, lr_final, warmup_steps, max_steps
-        self.tv_weight, self.betas, self.eps = tv_weight, betas, eps
-        n = self.num_grids * self.row  # a multiple of 4: 12 | row
-        self.param = torch.eye(3, 4).reshape(1, 12, 1, 1, 1).repeat(self.num_grids, 1, L, Y, X).reshape(-1).to(device)
-        self.device = self.param.device
-        self.grad, self.exp_avg, self.exp_avg_sq = (torch.zeros(n, device=self.device) for _ in range(3))
+        self.row = 12 * L * Y * X  # a multiple of 4: the table needs no padding
+        super().__init__(self.num_grids * self.row, device, "bilateral grid", lr, lr_final, warmup_steps, max_steps, betas, eps, backend)
+        self.grids.copy_(torch.eye(3, 4, device=self.device).reshape(1, 12, 1, 1, 1))
+        self.tv_weight = tv_weight
         self.tv_loss = torch.zeros(1, device=self.device)
         self._partials = torch.empty(self.num_grids, dtype=torch.float64, device=self.device)
-        self._lr = torch.zeros(1, device=self.device)
-        self._ends = torch.tensor([n], dtype=torch.int64, device=self.device)
-        self.lib = None
-        if backend == "cuda":
-            from . import _lib
-
-            self.lib = _lib.load()
 
     @property
     def grids(self) -> Tensor:
@@ -103,10 +90,3 @@ class BilateralGridOptimizer:
 
         _lib.check(self.lib.qed_bilagrid_accumulate(n, _lib.ptr(ids), _lib.ptr(rows), self.num_grids, self.X, self.Y, self.L, _lib.ptr(self.grad),
                                                     _lib.current_stream()), "qed_bilagrid_accumulate")
-
-    def lr_at(self, step: int) -> float:
-        return lr_at(step, self.lr, self.lr_final, self.warmup_steps, self.max_steps)
-
-    def step(self, step: int) -> None:
-        """Adam on every grid with the scheduled lr of 0-based iteration `step` (bias corrections use step + 1)."""
-        adam_table_step(self, self.lr_at(step), step + 1)

@@ -83,30 +83,21 @@ def check_camera_ids(camera_ids: Tensor, n_views: int, num_cameras: int, device)
     return ids
 
 
-class CameraPoseOptimizer:
-    """The pose table, its gradient and its Adam moments (flat [num_cameras * 6] buffers, padded to 4 floats).
+class AdamTable:
+    """A flat table trained by Adam (torch semantics, dense) with the `lr_at` schedule: `param`, `grad`, `exp_avg` and
+    `exp_avg_sq` of `n` floats, padded to 4, zero at init.  `backend="cuda"`: `qed_adam_arena` as a one-group call;
+    `backend="torch"`: the same arithmetic in torch."""
 
-    Per training step: `viewmats(c2w, ids)` -> render / backward with pose gradients -> `backward(v_viewmats, ids, c2w)`
-    (data term, overwrites `grad`) -> sum `grad` over the ranks -> `regularize()` -> `step(t)`."""
-
-    def __init__(self, num_cameras: int, device, lr: float = 1e-4, lr_final: float = 5e-7, warmup_steps: int = 1000,
-                 max_steps: int = 30000, trans_weight: float = 1e-2, rot_weight: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-15,
-                 backend: str = "cuda"):
-        if num_cameras < 1:
-            raise ValueError("the camera optimizer needs num_cameras >= 1")
+    def __init__(self, n: int, device, what: str, lr: float, lr_final: float, warmup_steps: int, max_steps: int, betas, eps: float,
+                 backend: str):
         if lr < 0 or lr_final <= 0 or warmup_steps < 0:
-            raise ValueError("camera optimizer: lr >= 0, lr_final > 0 and warmup_steps >= 0 expected")
-        self.num_cameras = int(num_cameras)
-        self.device = torch.device(device)
+            raise ValueError(f"{what}: lr >= 0, lr_final > 0 and warmup_steps >= 0 expected")
         self.backend = backend
         self.lr, self.lr_final, self.warmup_steps, self.max_steps = lr, lr_final, warmup_steps, max_steps
-        self.trans_weight, self.rot_weight = trans_weight, rot_weight
         self.betas, self.eps = betas, eps
-        n = self.num_cameras * 6
         self.padded = (n + 3) // 4 * 4
-        self.param, self.grad, self.exp_avg, self.exp_avg_sq = (torch.zeros(self.padded, device=self.device) for _ in range(4))
+        self.param, self.grad, self.exp_avg, self.exp_avg_sq = (torch.zeros(self.padded, device=device) for _ in range(4))
         self.device = self.param.device  # with its index
-        self.reg_loss = torch.zeros(1, device=self.device)
         self._lr = torch.zeros(1, device=self.device)
         self._ends = torch.tensor([self.padded], dtype=torch.int64, device=self.device)
         self.lib = None
@@ -119,6 +110,43 @@ class CameraPoseOptimizer:
         """Let the gradient live in `buf` (e.g. the symmetric buffer the ranks all-reduce)."""
         assert buf.numel() == self.padded and buf.dtype == torch.float32
         self.grad = buf
+
+    def lr_at(self, step: int) -> float:
+        return lr_at(step, self.lr, self.lr_final, self.warmup_steps, self.max_steps)
+
+    def step(self, step: int) -> None:
+        """Adam on the whole table with the scheduled lr of 0-based iteration `step` (bias corrections use step + 1)."""
+        lr, t = self.lr_at(step), step + 1
+        b1, b2 = self.betas
+        if self.backend != "cuda":
+            self.exp_avg.mul_(b1).add_(self.grad, alpha=1 - b1)
+            self.exp_avg_sq.mul_(b2).addcmul_(self.grad, self.grad, value=1 - b2)
+            denom = self.exp_avg_sq.sqrt() / math.sqrt(1.0 - b2 ** t) + self.eps
+            self.param.sub_(lr / (1.0 - b1 ** t) * (self.exp_avg / denom))
+            return
+        from . import _lib
+
+        self._lr.fill_(lr)
+        _lib.check(self.lib.qed_adam_arena(self.padded, _lib.ptr(self.param), _lib.ptr(self.grad), _lib.ptr(self.exp_avg), _lib.ptr(self.exp_avg_sq),
+                                           1, _lib.ptr(self._ends), _lib.ptr(self._lr), None, None, None, b1, b2, self.eps, t,
+                                           _lib.current_stream()), "qed_adam_arena")
+
+
+class CameraPoseOptimizer(AdamTable):
+    """The pose table [num_cameras * 6] (zero at init), its gradient and its Adam moments.
+
+    Per training step: `viewmats(c2w, ids)` -> render / backward with pose gradients -> `backward(v_viewmats, ids, c2w)`
+    (data term, overwrites `grad`) -> sum `grad` over the ranks -> `regularize()` -> `step(t)`."""
+
+    def __init__(self, num_cameras: int, device, lr: float = 1e-4, lr_final: float = 5e-7, warmup_steps: int = 1000,
+                 max_steps: int = 30000, trans_weight: float = 1e-2, rot_weight: float = 1e-3, betas=(0.9, 0.999), eps: float = 1e-15,
+                 backend: str = "cuda"):
+        if num_cameras < 1:
+            raise ValueError("the camera optimizer needs num_cameras >= 1")
+        self.num_cameras = int(num_cameras)
+        super().__init__(self.num_cameras * 6, device, "camera optimizer", lr, lr_final, warmup_steps, max_steps, betas, eps, backend)
+        self.trans_weight, self.rot_weight = trans_weight, rot_weight
+        self.reg_loss = torch.zeros(1, device=self.device)
 
     @property
     def pose_adjustment(self) -> Tensor:
@@ -186,28 +214,3 @@ class CameraPoseOptimizer:
         _lib.check(self.lib.qed_camera_opt_reg(self.num_cameras, _lib.ptr(self.param), self.trans_weight, self.rot_weight, _lib.ptr(self.grad),
                                                _lib.ptr(self.reg_loss), _lib.current_stream()), "qed_camera_opt_reg")
         return self.reg_loss
-
-    def lr_at(self, step: int) -> float:
-        return lr_at(step, self.lr, self.lr_final, self.warmup_steps, self.max_steps)
-
-    def step(self, step: int) -> None:
-        """Adam on the whole table with the scheduled lr of 0-based iteration `step` (bias corrections use step + 1)."""
-        adam_table_step(self, self.lr_at(step), step + 1)
-
-
-def adam_table_step(tab, lr: float, t: int) -> None:
-    """Adam (torch semantics) over a whole flat table `tab` (param / grad / exp_avg / exp_avg_sq, betas, eps, backend, and
-    for the CUDA backend lib, _lr [1] and _ends [1] on the device): `qed_adam_arena` as a one-group call."""
-    b1, b2 = tab.betas
-    if tab.backend != "cuda":
-        tab.exp_avg.mul_(b1).add_(tab.grad, alpha=1 - b1)
-        tab.exp_avg_sq.mul_(b2).addcmul_(tab.grad, tab.grad, value=1 - b2)
-        denom = tab.exp_avg_sq.sqrt() / math.sqrt(1.0 - b2 ** t) + tab.eps
-        tab.param.sub_(lr / (1.0 - b1 ** t) * (tab.exp_avg / denom))
-        return
-    from . import _lib
-
-    tab._lr.fill_(lr)
-    _lib.check(tab.lib.qed_adam_arena(tab.param.numel(), _lib.ptr(tab.param), _lib.ptr(tab.grad), _lib.ptr(tab.exp_avg), _lib.ptr(tab.exp_avg_sq),
-                                      1, _lib.ptr(tab._ends), _lib.ptr(tab._lr), None, None, None, b1, b2, tab.eps, t,
-                                      _lib.current_stream()), "qed_adam_arena")

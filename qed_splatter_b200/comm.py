@@ -85,12 +85,12 @@ class ViewShardedGradients:
         coefficient gradient from all views.  After it the arena holds the sum over all ranks' views, bit-identical on
         every rank.
       * with `num_cameras` > 0 (camera_opt.CameraPoseOptimizer): `project_bwd` also returns the pose gradient of the rank's
-        views, and `pose_grad` is a small symmetric buffer for the [num_cameras, 6] table gradient that
-        `reduce_pose_grad()` sums over the ranks with one more all-reduce kernel.
+        views, and `pose` is a small SymmetricArena for the [num_cameras, 6] table gradient, summed over the ranks by its
+        `all_reduce_()`.
       * with `bilagrid_row` > 0 (bilateral_grid.BilateralGridOptimizer, one grid = `bilagrid_row` floats): `bilagrid`, a
-        symmetric buffer of one grid-gradient row per view of the whole batch followed by the views' grid ids (as exact
-        floats).  Each rank writes its own slots, leaves the others zero, and `reduce_bilagrid()` makes every rank hold all
-        rows and ids, bit-identical, without all-reducing the dense [num_grids, row] gradient.
+        SymmetricArena of one grid-gradient row per view of the whole batch followed by the views' grid ids (as exact
+        floats).  Each rank writes its own slots, leaves the others zero, and `bilagrid.all_reduce_()` makes every rank hold
+        all rows and ids, bit-identical, without all-reducing the dense [num_grids, row] gradient.
 
     No NCCL call, no host synchronisation; collective: every rank makes the same calls in the same order."""
 
@@ -110,10 +110,9 @@ class ViewShardedGradients:
         n_xch = (self.slots * self.capacity + self.slots) * 4
         self.xch = [SymmetricArena(n_xch, device, group, force_peer_path=force_peer_path) for _ in range(2)]
         self.num_cameras = int(num_cameras)
-        self._pose = SymmetricArena(self.num_cameras * 6, device, group, force_peer_path=force_peer_path) if self.num_cameras > 0 else None
-        self.bilagrid_row = int(bilagrid_row)
-        n_bg = (self.slots * (self.bilagrid_row + 1) + 3) // 4 * 4
-        self._bilagrid = SymmetricArena(n_bg, device, group, force_peer_path=force_peer_path) if self.bilagrid_row > 0 else None
+        self.pose = SymmetricArena(self.num_cameras * 6, device, group, force_peer_path=force_peer_path) if self.num_cameras > 0 else None
+        n_bg = self.slots * (int(bilagrid_row) + 1)
+        self.bilagrid = SymmetricArena(n_bg, device, group, force_peer_path=force_peer_path) if bilagrid_row > 0 else None
         self.step = 0
         self._side = torch.cuda.Stream(device=self.arena.device)
         self._fork, self._join = torch.cuda.Event(), torch.cuda.Event()
@@ -136,27 +135,9 @@ class ViewShardedGradients:
         return self.arena.buf[:self.total]
 
     def views(self):
-        N = self.N
-        shape = {"means": (N, 3), "quats": (N, 4), "scales": (N, 3), "opacities": (N,), "sh": (N, 16, 3)}
-        return {g: self.arena.buf[a:b].view(*shape[g]) for g, (a, b) in self.offsets.items()}
+        from .trainer import GROUP_SHAPES
 
-    @property
-    def pose_grad(self) -> Optional[torch.Tensor]:
-        """[num_cameras * 6 rounded up to 4] float32 in symmetric memory (None without pose capacity)."""
-        return None if self._pose is None else self._pose.buf
-
-    def reduce_pose_grad(self) -> None:
-        """pose_grad <- its sum over the ranks, bit-identical everywhere.  Collective; no NCCL."""
-        self._pose.all_reduce_()
-
-    @property
-    def bilagrid(self) -> Optional[torch.Tensor]:
-        """[slots * (bilagrid_row + 1) rounded up to 4] float32 in symmetric memory: the rows, then the ids (None without)."""
-        return None if self._bilagrid is None else self._bilagrid.buf
-
-    def reduce_bilagrid(self) -> None:
-        """bilagrid <- its sum over the ranks, bit-identical everywhere (each slot has one non-zero writer).  Collective."""
-        self._bilagrid.all_reduce_()
+        return {g: self.arena.buf[a:b].view(self.N, *GROUP_SHAPES[g]) for g, (a, b) in self.offsets.items()}
 
     def _tag(self) -> float:
         return float(self.step % 8_000_000 + 1)  # exactly representable, never 0 (the buffers start zeroed)

@@ -33,7 +33,8 @@ import torch
 from torch import Tensor
 
 GROUPS = ("means", "quats", "scales", "opacities", "sh")
-GROUP_DIMS = {"means": 3, "quats": 4, "scales": 3, "opacities": 1, "sh": 48}
+GROUP_SHAPES = {"means": (3,), "quats": (4,), "scales": (3,), "opacities": (), "sh": (16, 3)}  # per Gaussian
+GROUP_DIMS = {g: math.prod(GROUP_SHAPES[g]) for g in GROUPS}
 FLOATS_PER_GAUSSIAN = sum(GROUP_DIMS.values())  # 59
 
 
@@ -138,62 +139,50 @@ class GaussianArena:
         self.device = means.device
         self._build(dict(means=means, quats=quats, scales=log_scales, opacities=logit_opacities, sh=sh), None, None)
 
-    def _build(self, params: Dict[str, Tensor], m: Optional[Dict[str, Tensor]], v: Optional[Dict[str, Tensor]]):
-        N = params["means"].shape[0]
-        self.N = N
-        # every group starts on a 16-byte boundary (vectorised loads in the kernels); the <= 3 padding floats
-        # per group carry zero gradients, so Adam and the all-reduce leave them at zero
-        pad4 = lambda k: (k + 3) // 4 * 4
-        n = sum(pad4(GROUP_DIMS[g] * N) for g in GROUPS)
-        self.param = torch.zeros(n, device=self.device)
-        self.grad = torch.zeros(n, device=self.device)
-        self.exp_avg = torch.zeros(n, device=self.device)
-        self.exp_avg_sq = torch.zeros(n, device=self.device)
-        self.offsets = {}
-        o = 0
+    def _build(self, params: Dict[str, Tensor], m: Optional[Dict[str, Tensor]], v: Optional[Dict[str, Tensor]]) -> None:
+        """New arenas for the Gaussians of `params` (tensors shaped as `view` returns them); Adam moments from m / v, or zero."""
+        n = self._set_layout(params["means"].shape[0])
+        self.param, self.grad, self.exp_avg, self.exp_avg_sq = (torch.zeros(n, device=self.device) for _ in range(4))
         for g in GROUPS:
-            d = GROUP_DIMS[g]
-            self.offsets[g] = (o, o + d * N)
-            self.param[o:o + d * N] = params[g].reshape(-1).to(torch.float32)
+            a, b = self.offsets[g]
+            self.param[a:b] = params[g].reshape(-1).to(torch.float32)
             if m is not None:
-                self.exp_avg[o:o + d * N] = m[g].reshape(-1)
-                self.exp_avg_sq[o:o + d * N] = v[g].reshape(-1)
-            o += pad4(d * N)
-        ends = [pad4(self.offsets[g][1]) for g in GROUPS]
-        self.group_ends = torch.tensor(ends, dtype=torch.int64, device=self.device)
+                self.exp_avg[a:b] = m[g].reshape(-1)
+                self.exp_avg_sq[a:b] = v[g].reshape(-1)
 
     @staticmethod
     def layout(N: int):
-        """-> (offsets {group: (start, end)}, total floats) of an arena for N Gaussians (16-byte aligned groups)."""
-        pad4 = lambda k: (k + 3) // 4 * 4
+        """-> (offsets {group: (start, end)}, total floats) of an arena for N Gaussians.  Every group starts on a 16-byte
+        boundary (vectorised loads in the kernels); the <= 3 padding floats per group carry zero gradients, so Adam and the
+        all-reduce leave them at zero."""
         offsets, o = {}, 0
         for g in GROUPS:
             d = GROUP_DIMS[g]
             offsets[g] = (o, o + d * N)
-            o += pad4(d * N)
+            o += (d * N + 3) // 4 * 4
         return offsets, o
+
+    def _set_layout(self, N: int) -> int:
+        """N, offsets and group_ends (each group's padded end: where the next one starts) for N Gaussians; -> total floats."""
+        self.N = N
+        self.offsets, n = self.layout(N)
+        starts = [self.offsets[g][0] for g in GROUPS]
+        self.group_ends = torch.tensor(starts[1:] + [n], dtype=torch.int64, device=self.device)
+        return n
 
     def adopt(self, N: int, param: Tensor, exp_avg: Tensor, exp_avg_sq: Tensor) -> None:
         """Take over freshly built arenas (qed_arena_gather) for N Gaussians; gradients start at zero."""
-        pad4 = lambda k: (k + 3) // 4 * 4
-        self.N = N
-        self.offsets, n = self.layout(N)
+        n = self._set_layout(N)
         assert param.numel() == n and exp_avg.numel() == n and exp_avg_sq.numel() == n
         self.param, self.exp_avg, self.exp_avg_sq = param, exp_avg, exp_avg_sq
         self.grad = torch.zeros(n, device=self.device)
-        self.group_ends = torch.tensor([pad4(self.offsets[g][1]) for g in GROUPS], dtype=torch.int64, device=self.device)
 
     def view(self, buf: Tensor, g: str) -> Tensor:
         a, b = self.offsets[g]
-        N = self.N
-        shape = {"means": (N, 3), "quats": (N, 4), "scales": (N, 3), "opacities": (N,), "sh": (N, 16, 3)}[g]
-        return buf[a:b].view(*shape)
+        return buf[a:b].view(self.N, *GROUP_SHAPES[g])
 
     def views(self, buf: Tensor) -> Dict[str, Tensor]:
         return {g: self.view(buf, g) for g in GROUPS}
-
-    def rebuild(self, params, m, v):
-        self._build(params, m, v)
 
 
 @dataclass
@@ -384,7 +373,7 @@ def _refine_gaussians_torch(arena: GaussianArena, state: StrategyState, cfg: Tra
         for g in GROUPS:
             p[g], m[g], v[g] = p[g][keep], m[g][keep], v[g][keep]
     if p["means"].shape[0] != N0 or n_prune or info["n_split"] or info["n_dupli"]:
-        arena.rebuild(p, m, v)
+        arena._build(p, m, v)
     # reset running stats (gsplat zeroes them after every refine)
     state.grad2d = torch.zeros(arena.N, device=dev)
     state.count = torch.zeros(arena.N, device=dev)
@@ -528,16 +517,55 @@ class SplatTrainer:
         if self.arena.grad.data_ptr() != x.grad.data_ptr():
             assert x.grad.numel() == self.arena.grad.numel()
             self.arena.grad = x.grad  # Adam reads the summed gradients straight from the symmetric arena
-        if self.camera_opt is not None and self.camera_opt.grad.data_ptr() != x.pose_grad.data_ptr():
-            self.camera_opt.use_grad_buffer(x.pose_grad)
+        if self.camera_opt is not None and self.camera_opt.grad.data_ptr() != x.pose.buf.data_ptr():
+            self.camera_opt.use_grad_buffer(x.pose.buf)
         return x
 
     # -- collectives --------------------------------------------------------------------------
-    def _all_reduce(self, t: Tensor, op: str = "sum") -> None:
-        if self.world > 1:
+    def _all_reduce(self, t: Tensor, sym=None, op: str = "sum") -> None:
+        """`t` <- its sum (op "max": maximum) over the ranks, in place.  `sym`: the comm.SymmetricArena whose buffer holds
+        `t`; then that whole buffer is summed by this library's all-reduce kernel.  Otherwise torch.distributed, and with one
+        rank nothing."""
+        if sym is not None:
+            assert op == "sum"
+            sym.all_reduce_()
+        elif self.world > 1:
             import torch.distributed as dist
 
             dist.all_reduce(t, op=dist.ReduceOp.SUM if op == "sum" else dist.ReduceOp.MAX, group=self.pg)
+
+    def _all_reduce_sh_async(self, works: list, n0: int, n1: int) -> None:
+        """Starts the all-reduce of the SH gradient rows of Gaussians [n0, n1) on the NCCL stream; appends (work, lo, hi)."""
+        import torch.distributed as dist
+
+        sh0 = self.arena.offsets["sh"][0]
+        lo, hi = sh0 + 48 * n0, sh0 + 48 * n1
+        works.append((dist.all_reduce(self.arena.grad[lo:hi], group=self.pg, async_op=True), lo, hi))
+
+    def _gaussian_update(self, pipelined: bool, chunked_bwd: bool, works: list) -> None:
+        """The Gaussian gradients summed over the ranks, then Adam.  The exchange has summed them inside the fused step, and
+        one rank has nothing to sum.  `pipelined` ("nccl", one view per rank): the SH rows are reduced in `comm_chunks`
+        async ranges (started by the chunked projection backward, else here) and each range is Adam-stepped as soon as its
+        sum has landed, while the head (means | quats | scales | opacities) is reduced."""
+        c, a = self.cfg, self.arena
+        if not pipelined:
+            if self.comm == "nccl":
+                self._all_reduce(a.grad)
+            self.optimizer_step()
+            return
+        import torch.distributed as dist
+
+        if not chunked_bwd:  # one projection-backward launch, then chunked reductions
+            step_n = ((a.N + c.comm_chunks - 1) // c.comm_chunks + 3) // 4 * 4
+            for n0 in range(0, a.N, step_n):
+                self._all_reduce_sh_async(works, n0, min(n0 + step_n, a.N))
+        sh0 = a.offsets["sh"][0]
+        head = dist.all_reduce(a.grad[:sh0], group=self.pg, async_op=True)
+        for w, lo, hi in works:  # Adam on each SH range as soon as its reduction has landed
+            w.wait()
+            self.optimizer_step(lo, hi)
+        head.wait()
+        self.optimizer_step(0, sh0)
 
     # -- pieces that the tests drive directly ---------------------------------------------------
     def sh_degree_to_use(self) -> int:
@@ -623,10 +651,7 @@ class SplatTrainer:
         """camera_opt_update on inputs already passed through CameraPoseOptimizer.prepare."""
         cam = self.camera_opt
         cam._backward(v_viewmats, camera_ids, camera_to_worlds)
-        if exchange is not None:
-            exchange.reduce_pose_grad()
-        else:
-            self._all_reduce(cam.grad)
+        self._all_reduce(cam.grad, None if exchange is None else exchange.pose)
         cam.regularize()
         cam.step(self.step_count)
 
@@ -636,7 +661,7 @@ class SplatTrainer:
         bg, slots = self.bilagrid, self.world * C
         n = slots * (bg.row + 1)
         if exchange is not None:
-            buf = exchange.bilagrid
+            buf = exchange.bilagrid.buf
         else:
             if self._bg_buf is None or self._bg_buf.numel() < n:
                 self._bg_buf = torch.zeros(n, device=self.device)
@@ -653,10 +678,8 @@ class SplatTrainer:
         bg = self.bilagrid
         if exchange is not None or self.world > 1:
             ids_f[self.rank * C:(self.rank + 1) * C].copy_(ids)
-            if exchange is not None:
-                exchange.reduce_bilagrid()  # the whole symmetric buffer; floats past this batch's slots are zero
-            else:
-                self._all_reduce(buf)
+            # with the exchange: its whole symmetric buffer; floats past this batch's slots are zero
+            self._all_reduce(buf, None if exchange is None else exchange.bilagrid)
             ids = ids_f.to(torch.int32)
         bg.regularize()
         bg.accumulate(ids, rows)
@@ -685,7 +708,7 @@ class SplatTrainer:
             # the accumulators of every rank are combined only now (SUM / MAX are associative)
             self._all_reduce(self.state.grad2d)
             self._all_reduce(self.state.count)
-            self._all_reduce(self.state.radii, "max")
+            self._all_reduce(self.state.radii, op="max")
             gen = torch.Generator().manual_seed(c.seed * 1_000_003 + step)
             info = refine_gaussians(self.arena, self.state, c, step, gen)
         if step % reset_every == 0:
@@ -724,72 +747,36 @@ class SplatTrainer:
             camera_ids = check_camera_ids(camera_ids, viewmats.shape[0], bg.num_grids, self.device)
         C = viewmats.shape[0]
         total = total_views or C * self.world
-        pv = a.views(a.param)
-        gv = a.views(a.grad)
-        # the stored parameters go straight in: exp / sigmoid (model.py:269-271) and their chain rule run inside the
-        # projection kernels, the gradients land in the arena
         xg = self._exchange_for(C) if self.comm == "exchange" else None  # may fall back to "nccl" (comm="auto", no symmetric memory)
-        bl = None
-        if bg is not None:
-            bl = self._bilagrid_slots(C, xg)  # this rank's rows are written by the loss kernels of the fused step
-        bl_arg = None if bl is None else (bg.grids, camera_ids, bl[3])
-        if xg is not None:
-            out = self._fused.step(pv["means"], pv["quats"], pv["scales"], pv["opacities"], pv["sh"], viewmats, Ks, width, height,
-                                   self.sh_degree_to_use(), gt_rgb, gt_depth, background, render_mode=c.render_mode, rgb_weight=1.0 - c.ssim_lambda,
-                                   depth_lambda=c.depth_lambda, grad_scale=C / float(total), rasterize_mode=c.rasterize_mode, activations=3,
-                                   mask=mask, ssim_lambda=c.ssim_lambda, exchange=xg, depth_unit_scale=c.depth_unit_scale,
-                                   pose_gradients=cam is not None, bilateral_grid=bl_arg)
-            self.accumulate_stats(out.packed_grads, out.radii, width, height, packed=True, n_cameras=total)
-            self.optimizer_step()
-            if cam is not None:
-                self._camera_opt_update(out.v_viewmats, camera_ids, camera_to_worlds, xg)
-            if bg is not None:
-                self._bilagrid_finish(C, camera_ids, *bl[:3], xg)
-            loss = out.loss.clone()
-            info = self.maybe_refine(self.step_count)
-            self.step_count += 1
-            return loss, info
-        pipelined = self.world > 1 and C == 1 and c.comm_chunks > 1
+        # "nccl" with one view per rank: the SH gradients are all-reduced and Adam-stepped in `comm_chunks` Gaussian ranges
+        pipelined = self.comm == "nccl" and C == 1 and c.comm_chunks > 1
         # pose gradients need the projection backward in one launch: the pipelined path then chunks only the reductions
         chunked_bwd = pipelined and c.chunk_project_bwd and cam is None
-        sh0 = a.offsets["sh"][0]
-        works = []
-
-        def on_chunk(k, n0, n1):
-            # SH rows of a finished Gaussian range: all-reduce them now (NCCL stream) while the next range computes
-            import torch.distributed as dist
-
-            lo, hi = sh0 + 48 * n0, sh0 + 48 * n1
-            works.append((dist.all_reduce(a.grad[lo:hi], group=self.pg, async_op=True), lo, hi))
-
+        works = []  # (async all-reduce, lo, hi) of the SH ranges in flight
+        if xg is not None:  # the projection backward writes into the symmetric arena; the fused step ends with the sum
+            comm_args = dict(exchange=xg)
+        elif chunked_bwd:  # SH rows of a finished Gaussian range: all-reduce them now while the next range computes
+            comm_args = dict(grad_out=a.views(a.grad), n_chunks=c.comm_chunks,
+                             on_chunk=lambda k, n0, n1: self._all_reduce_sh_async(works, n0, n1))
+        else:
+            comm_args = dict(grad_out=a.views(a.grad))
+        # this rank's grid rows are written by the loss kernels of the fused step
+        bl = None if bg is None else self._bilagrid_slots(C, xg)
+        # the stored parameters go straight in: exp / sigmoid (model.py:269-271) and their chain rule run inside the
+        # projection kernels, the gradients land in the arena
+        pv = a.views(a.param)
         out = self._fused.step(pv["means"], pv["quats"], pv["scales"], pv["opacities"], pv["sh"], viewmats, Ks, width, height, self.sh_degree_to_use(),
                                gt_rgb, gt_depth, background, render_mode=c.render_mode, rgb_weight=1.0 - c.ssim_lambda,
-                               depth_lambda=c.depth_lambda, grad_scale=C / float(total), rasterize_mode=c.rasterize_mode, grad_out=gv,
+                               depth_lambda=c.depth_lambda, grad_scale=C / float(total), rasterize_mode=c.rasterize_mode,
                                activations=3,  # ACT_LOG_SCALES | ACT_LOGIT_OPACITIES (pipeline.py / include/qed_splat.h)
-                               mask=mask, depth_unit_scale=c.depth_unit_scale, ssim_lambda=c.ssim_lambda,
-                               n_chunks=c.comm_chunks if chunked_bwd else 1, on_chunk=on_chunk if chunked_bwd else None,
-                               pose_gradients=cam is not None, bilateral_grid=bl_arg)
+                               mask=mask, depth_unit_scale=c.depth_unit_scale, ssim_lambda=c.ssim_lambda, pose_gradients=cam is not None,
+                               bilateral_grid=None if bl is None else (bg.grids, camera_ids, bl[3]), **comm_args)
         self.accumulate_stats(out.packed_grads, out.radii, width, height, packed=True, n_cameras=total)
-        if pipelined:
-            import torch.distributed as dist
-
-            if not chunked_bwd:  # one projection-backward launch, then chunked reductions
-                step_n = ((a.N + c.comm_chunks - 1) // c.comm_chunks + 3) // 4 * 4
-                for k, n0 in enumerate(range(0, a.N, step_n)):
-                    on_chunk(k, n0, min(n0 + step_n, a.N))
-            head = dist.all_reduce(a.grad[:sh0], group=self.pg, async_op=True)
-            for w, lo, hi in works:  # Adam on each SH range as soon as its reduction has landed
-                w.wait()
-                self.optimizer_step(lo, hi)
-            head.wait()
-            self.optimizer_step(0, sh0)
-        else:
-            self._all_reduce(a.grad)
-            self.optimizer_step()
+        self._gaussian_update(pipelined, chunked_bwd, works)
         if cam is not None:
-            self._camera_opt_update(out.v_viewmats, camera_ids, camera_to_worlds, None)
+            self._camera_opt_update(out.v_viewmats, camera_ids, camera_to_worlds, xg)
         if bg is not None:
-            self._bilagrid_finish(C, camera_ids, *bl[:3], None)
+            self._bilagrid_finish(C, camera_ids, *bl[:3], xg)
         loss = out.loss.clone()  # out.loss is a buffer the next step overwrites in place
         info = self.maybe_refine(self.step_count)
         self.step_count += 1

@@ -235,7 +235,7 @@ def _exchange_worker(rank, port, out):
                         camera_ids=ids[v])
             res["grad_err"].append(float((xt.camera_opt.pose_grad - ref.camera_opt.pose_grad).abs().max()))
             res["grad_scale"].append(float(ref.camera_opt.pose_grad.abs().max()))
-            res["grad_in_symmetric"].append(xt.camera_opt.grad.data_ptr() == xt._xg.pose_grad.data_ptr())
+            res["grad_in_symmetric"].append(xt.camera_opt.grad.data_ptr() == xt._xg.pose.buf.data_ptr())
             res["exchanges"].append(id(xt._xg))
         res["comm"] = xt.comm
         res["table_err"] = float((xt.pose_adjustment - ref.pose_adjustment).abs().max())
@@ -249,7 +249,7 @@ def _exchange_worker(rank, port, out):
 
 def test_trainer_exchange_path_on_one_gpu(cuda, tmp_path):
     """The trainer's exchange integration -- pose gradient from qed_project_bwd_exchange_pose, the table gradient living in
-    the symmetric pose buffer and summed by reduce_pose_grad, the buffers rebuilt when the views per rank change -- gives
+    the symmetric pose buffer and summed by its all-reduce kernel, the buffers rebuilt when the views per rank change -- gives
     the table gradients and tables of the plain single-GPU trainer."""
     out = str(tmp_path / "xchg.pt")
     mp.spawn(_exchange_worker, args=(29500 + (os.getpid() + 11) % 2000, out), nprocs=1, join=True)

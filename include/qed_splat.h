@@ -294,6 +294,20 @@ int qed_loss_fwd_bwd_bilagrid(int C, int width, int height, const float* render,
                               int grid_X, int grid_Y, int grid_L, float* v_grid_rows, void* workspace, size_t workspace_bytes,
                               qed_stream_t stream);
 
+/* Ground truth of a step rendered at 1/factor resolution (splatfacto's resolution schedule: `_downscale_if_required`, a
+ * factor x factor box filter = conv2d with weights 1/factor^2 and stride factor, on the image, the depth and the mask).
+ *  In: gt_rgb[C,height,width,3] float32 or (rgb_is_u8) uint8; gt_depth[C,height,width] float32 or (depth_is_u16) raw uint16;
+ *  mask[C,height,width] float32 or (mask_is_u8) uint8 / bool, or NULL.  Values are converted as qed_loss_fwd_bwd converts
+ *  them (u8 * (1.0f / 255.0f); float(double(u16) * depth_unit_scale); bool -> 0 / 1) BEFORE the filter.
+ *  Out (float32, overwritten): out_rgb[C,h,w,3], out_depth[C,h,w] (metres), out_mask[C,h,w] (fractional; only when mask is
+ *  not NULL), h = height / factor, w = width / factor rounded down (trailing rows / columns that fill no block are dropped).
+ *  Each output = sum over its block, in row-major order starting from 0, of (1/factor^2) * x, individually rounded (no
+ *  FMA).  NaN / inf propagate; zero (invalid) depth is averaged in, as the reference does.
+ *  QED_ERR_BAD_ARG: C, width or height < 1, factor < 1, h or w == 0, a NULL input / output (out_mask when mask != NULL). */
+int qed_downscale_ground_truth(int C, int width, int height, int factor, const void* gt_rgb, int rgb_is_u8, const void* gt_depth,
+                               int depth_is_u16, double depth_unit_scale, const void* mask, int mask_is_u8, float* out_rgb,
+                               float* out_depth, float* out_mask, qed_stream_t stream);
+
 /* Total-variation regulariser of the bilateral grids (splatfacto get_loss_dict while training):
  *  loss_out[1] = weight / G * sum_{axes d in L, Y, X} sum (x[.., i+1, ..] - x[.., i, ..])^2 / (elements of one grid's
  *  difference along d, i.e. 12 L Y X (n_d - 1) / n_d).  v_grids[G,12,L,Y,X] is OVERWRITTEN with its gradient;

@@ -53,6 +53,7 @@ SIGNATURES = {
     "qed_loss_bilagrid_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_float]),
     "qed_loss_fwd_bwd_bilagrid": (c_int, [c_int, c_int, c_int, P, P, P, c_int, P, c_int, c_double, P, c_int, P, c_float, c_float, c_float, c_float,
                                           P, P, P, P, P, P, c_int, c_int, c_int, c_int, P, P, c_size_t, P]),
+    "qed_downscale_ground_truth": (c_int, [c_int, c_int, c_int, c_int, P, c_int, P, c_int, c_double, P, c_int, P, P, P, P]),
     "qed_bilagrid_tv": (c_int, [c_int, c_int, c_int, c_int, P, c_float, P, P, P, P]),
     "qed_bilagrid_accumulate": (c_int, [c_int, P, P, c_int, c_int, c_int, c_int, P, P]),
     "qed_adam_arena": (c_int, [c_int64, P, P, P, P, c_int, P, P, P, P, P, c_double, c_double, c_double, c_int, P]),

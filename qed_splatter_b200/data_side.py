@@ -9,12 +9,14 @@
   Here the frames' depth images go through `qed_backproject_depth` / `qed_voxel_downsample` and the pairwise tree merge
   stays on the device.  File handling (transforms.json, PLY, the on-disk cache, colourising from RGB) stays the
   reference's: these functions take arrays, not dataset paths.
+* `downscale_ground_truth(...)` — splatfacto's `_downscale_if_required` (resolution schedule): the full-resolution image,
+  depth and mask of a step box-downscaled in one launch of `qed_downscale_ground_truth`, read in their cached types.
 
 No CPU fallback: CPU tensors raise.
 """
 from __future__ import annotations
 
-from typing import List, Optional, Sequence
+from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -65,6 +67,59 @@ def get_viewmat(optimized_camera_to_world: Tensor, pose_gradients: bool = False)
         # camera_optimizer.mode != "off" without asking for pose gradients: refuse rather than train with zero gradients
         raise NotImplementedError("get_viewmat: c2w requires grad (camera optimisation): pass pose_gradients=True, or c2w.detach()")
     return _viewmat_from_c2w(c2w.detach().contiguous())
+
+
+def downscaled_size(width: int, height: int, factor: int) -> Tuple[int, int]:
+    """(w, h) of ground truth of size width x height box-downscaled by `factor`: rounded down, as conv2d(stride=factor)
+    drops trailing rows and columns that fill no block.  ValueError when the factor is below 1 or nothing is left."""
+    if int(factor) != factor or factor < 1:
+        raise ValueError(f"downscale factor must be an integer >= 1, got {factor!r}")
+    w, h = int(width) // int(factor), int(height) // int(factor)
+    if w < 1 or h < 1:
+        raise ValueError(f"{width}x{height} ground truth has no full {factor}x{factor} block")
+    return w, h
+
+
+def downscale_ground_truth(gt_rgb: Tensor, gt_depth: Tensor, mask: Optional[Tensor], factor: int, depth_unit_scale: float = 0.001,
+                           out: Optional[Tuple[Tensor, Tensor, Optional[Tensor]]] = None) -> Tuple[Tensor, Tensor, Optional[Tensor]]:
+    """Splatfacto's `_downscale_if_required` (nerfstudio `resize_image`: a factor x factor box filter) on the ground truth of
+    a step, one launch of `qed_downscale_ground_truth`.
+
+    gt_rgb [C,H,W,3] float32 or the uint8 image cache (u8 / 255 before the filter, as `get_gt_img` does), gt_depth
+    [C,H,W(,1)] float32 metres or the raw uint16 sensor image (torch.uint16, or its bits as torch.int16; converted with
+    `depth_unit_scale` before the filter), mask [C,H,W(,1)] float32 / uint8 / bool or None (bool -> 0 / 1 floats, so the
+    result is fractional).  -> float32 (rgb [C,h,w,3], depth [C,h,w,1] metres, mask [C,h,w,1] or None) with
+    (w, h) = downscaled_size(W, H, factor); each value is the row-major sum of (1/factor^2) * x over its block.
+    `out`: tensors of those shapes to write into (the mask slot may be None when mask is None)."""
+    _lib.require_cuda(gt_rgb, gt_depth, mask)
+    _lib.require_dtype(gt_rgb, (torch.float32, torch.uint8), "gt_rgb")
+    _lib.require_dtype(gt_depth, (torch.float32, torch.uint16, torch.int16), "gt_depth")
+    _lib.require_dtype(mask, (torch.float32, torch.uint8, torch.bool), "mask")
+    if gt_rgb.dim() != 4 or gt_rgb.shape[3] != 3:
+        raise ValueError("gt_rgb must be [C,H,W,3]")
+    C, H, W, _ = gt_rgb.shape
+    w, h = downscaled_size(W, H, factor)
+    if gt_depth.numel() != C * H * W or (mask is not None and mask.numel() != C * H * W):
+        raise ValueError("shapes: gt_rgb [C,H,W,3], gt_depth [C,H,W(,1)], mask [C,H,W(,1)]")
+    shapes = ((C, h, w, 3), (C, h, w, 1), (C, h, w, 1))
+    if out is None:
+        out = tuple(torch.empty(s, dtype=torch.float32, device=gt_rgb.device) for s in shapes)
+    out_rgb, out_depth, out_mask = out
+    out_mask = out_mask if mask is not None else None
+    for t, s in zip((out_rgb, out_depth, out_mask), shapes):
+        if t is not None and (tuple(t.shape) != s or t.dtype != torch.float32 or not t.is_contiguous() or t.device != gt_rgb.device):
+            raise ValueError(f"out: contiguous float32 tensors of shapes {shapes} on {gt_rgb.device} expected")
+    if mask is not None and out_mask is None:
+        raise ValueError("out: a mask tensor is needed when mask is given")
+    rgb, dep = gt_rgb.contiguous(), gt_depth.contiguous()
+    mk = None if mask is None else mask.contiguous()
+    if mk is not None and mk.dtype == torch.bool:
+        mk = mk.view(torch.uint8)
+    check(_lib.load().qed_downscale_ground_truth(C, W, H, int(factor), ptr(rgb), int(rgb.dtype == torch.uint8), ptr(dep),
+                                                 int(dep.dtype != torch.float32), float(depth_unit_scale), ptr(mk),
+                                                 int(mk is not None and mk.dtype == torch.uint8), ptr(out_rgb), ptr(out_depth),
+                                                 ptr(out_mask), current_stream()), "qed_downscale_ground_truth")
+    return out_rgb, out_depth, out_mask
 
 
 def _host_f32(x, shape, what: str) -> np.ndarray:

@@ -181,7 +181,7 @@ def bilateral_grid_tv_loss(grids: Tensor, weight: float = 10.0) -> Tensor:
 def depth_supervised_loss(render: Tensor, alphas: Tensor, gt_rgb: Tensor, gt_depth: Tensor, background: Tensor, rgb_weight: float = 0.8,
                           depth_lambda: float = 0.2, ssim_lambda: float = 0.0, mask: Optional[Tensor] = None,
                           depth_unit_scale: float = 0.001, bilateral_grids: Optional[Tensor] = None,
-                          grid_ids: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor]:
+                          grid_ids: Optional[Tensor] = None, gt_downscale: int = 1) -> Tuple[Tensor, Tensor, Tensor]:
     """-> (total, rgb_term, depth_term), 0-dim tensors; `total` carries the gradient to `render` and `alphas`.
 
     render [C,H,W,4] (RGB + depth; expected depth for 'RGB+ED'), alphas [C,H,W,1], gt_rgb [C,H,W,3] float in [0,1] or uint8
@@ -199,9 +199,23 @@ def depth_supervised_loss(render: Tensor, alphas: Tensor, gt_rgb: Tensor, gt_dep
     the training image of each view): the clamped composite of every view goes through its grid's affine colour transform
     (nerfstudio lib_bilagrid `slice`) before the mask, L1 and SSIM, as splatfacto does for training views; the depth term is
     unchanged.  `total` then carries the gradient to the grids too.  Supported grid shapes: 2 <= X, Y <= 1024, 2 <= L <= 16.
+
+    gt_downscale d > 1 (splatfacto's resolution schedule, `_get_downscale_factor()`): render / alphas are [C,h,w,...] at the
+    rescaled camera and gt_rgb / gt_depth / mask are at full resolution [C,H,W,...] with H // d == h and W // d == w; they
+    are box-downscaled first as splatfacto's `_downscale_if_required` does (data_side.downscale_ground_truth, one launch).
     """
     if (bilateral_grids is None) != (grid_ids is None):
         raise ValueError("bilateral_grids and grid_ids go together")
+    if gt_downscale != 1:
+        from .data_side import downscale_ground_truth, downscaled_size
+
+        if render.dim() != 4 or gt_rgb.dim() != 4:
+            raise ValueError("gt_downscale: render [C,h,w,4] and full-resolution gt_rgb [C,H,W,3] expected")
+        size = downscaled_size(gt_rgb.shape[2], gt_rgb.shape[1], gt_downscale)
+        if size != (render.shape[2], render.shape[1]) or gt_rgb.shape[0] != render.shape[0]:
+            raise ValueError(f"gt_downscale={gt_downscale}: {gt_rgb.shape[2]}x{gt_rgb.shape[1]} ground truth downscales to {size[0]}x{size[1]}, "
+                             f"the render is {render.shape[2]}x{render.shape[1]}")
+        gt_rgb, gt_depth, mask = downscale_ground_truth(gt_rgb, gt_depth, mask, gt_downscale, depth_unit_scale)
     if bilateral_grids is not None:
         return _DepthSupervisedLossBilagrid.apply(render, alphas, bilateral_grids, grid_ids, gt_rgb, gt_depth, background, rgb_weight, depth_lambda,
                                                   ssim_lambda, mask, depth_unit_scale)

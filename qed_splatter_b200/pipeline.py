@@ -341,7 +341,7 @@ class FusedSplatStep:
              depth_lambda: float = 0.2, grad_scale: float = 1.0, rasterize_mode: str = "classic",
              grad_out: Optional[Dict[str, Tensor]] = None, ssim_lambda: float = 0.0, n_chunks: int = 1, on_chunk=None,
              activations: int = 0, mask: Optional[Tensor] = None, exchange=None, depth_unit_scale: float = 0.001,
-             pose_gradients: bool = False, bilateral_grid=None) -> StepOutput:
+             pose_gradients: bool = False, bilateral_grid=None, gt_downscale: int = 1) -> StepOutput:
         """`render_mode` RGB+ED (north_star) or RGB+D (what qed_splatter/model.py:257 passes).
         loss = rgb_weight * L1 + ssim_lambda * (1 - SSIM) + depth_lambda * masked depth-L1 (splatfacto: 0.8 / 0.2 / 0.2).
         `mask` [C,H,W(,1)] float32 / uint8 / bool = `batch["mask"]` (model.py:93-97), see losses.depth_supervised_loss.
@@ -352,7 +352,10 @@ class FusedSplatStep:
         `bilateral_grid=(grids, grid_ids, v_grid_rows)`: splatfacto's bilateral grid on every view before the RGB loss
         (qed_loss_fwd_bwd_bilagrid): grids [G,12,L,Y,X] float32, grid_ids [C] int32 on the device (validated by the caller),
         v_grid_rows [C,12,L,Y,X] overwritten with each view's grid gradient.  Only the loss stage changes, so it combines
-        with `n_chunks` and `exchange`."""
+        with `n_chunks` and `exchange`.
+        `gt_downscale` d > 1 (splatfacto's resolution schedule): the camera (Ks, width, height) is the rescaled one and
+        gt_rgb [C,H,W,3] / gt_depth / mask are at full resolution with H // d == height and W // d == width; they are
+        box-downscaled into buffers of this object (data_side.downscale_ground_truth) before the projection is queued."""
         assert render_mode in ("RGB+D", "RGB+ED")
         if pose_gradients and (n_chunks > 1 or not _pose_capable(exchange)):
             raise ValueError("pose_gradients=True is not available with n_chunks > 1 or an exchange without pose capacity")
@@ -364,6 +367,18 @@ class FusedSplatStep:
         _lib.require_dtype(background, (torch.float32,), "background")
         _lib.require_dtype(mask, (torch.float32, torch.uint8, torch.bool), "mask")
         C_, HW_ = viewmats.shape[0], width * height
+        if gt_downscale != 1:
+            from .data_side import downscale_ground_truth, downscaled_size
+
+            if gt_rgb.dim() != 4 or gt_rgb.shape[0] != C_:
+                raise ValueError("gt_downscale: full-resolution gt_rgb [C,H,W,3] expected")
+            C_, H_, W_, _ = gt_rgb.shape
+            if downscaled_size(W_, H_, gt_downscale) != (width, height):
+                raise ValueError(f"gt_downscale={gt_downscale}: {W_}x{H_} ground truth does not downscale to the {width}x{height} render")
+            # queued ahead of the projection: the loss then reads float32 ground truth at render size
+            gt_rgb, gt_depth, mask = downscale_ground_truth(gt_rgb, gt_depth, mask, gt_downscale, depth_unit_scale,
+                                                            out=(self._get("gt_rgb_ds", (C_, height, width, 3)), self._get("gt_depth_ds", (C_, height, width, 1)),
+                                                                 self._get("mask_ds", (C_, height, width, 1)) if mask is not None else None))
         if gt_rgb.numel() != C_ * HW_ * 3 or gt_depth.numel() != C_ * HW_ or background.numel() != 3 or (mask is not None and mask.numel() != C_ * HW_):
             raise ValueError("shapes: gt_rgb [C,H,W,3], gt_depth [C,H,W(,1)], background [3], mask [C,H,W(,1)]")
         gt_rgb, gt_depth, background = gt_rgb.contiguous(), gt_depth.contiguous(), background.contiguous()

@@ -102,6 +102,11 @@ class TrainConfig:
     bilateral_grid_lr_final: float = 1e-4  # [UP] ExponentialDecayScheduler lr_final, reached at max_steps
     bilateral_grid_warmup: int = 1000  # [UP] warm-up steps from lr 0
     bilateral_grid_tv_weight: float = 10.0  # [UP] weight of the total-variation loss
+    # splatfacto's resolution schedule: steps [k * resolution_schedule, (k + 1) * resolution_schedule) render at 1 / 2^(n - k)
+    # of the full resolution for k < n = num_downscales, with the ground truth box-downscaled to match.  Splatfacto's default
+    # (and qed-splatter's) is num_downscales = 2; it stays 0 (always full resolution) here so existing runs are unchanged.
+    num_downscales: int = 0
+    resolution_schedule: int = 3000
 
     def __post_init__(self):
         self.validate()
@@ -112,6 +117,8 @@ class TrainConfig:
 
         if self.camera_optimizer not in CAMERA_OPTIMIZER_MODES:
             raise ValueError(f"camera_optimizer must be one of {CAMERA_OPTIMIZER_MODES}, got {self.camera_optimizer!r}")
+        if self.num_downscales < 0 or self.resolution_schedule < 1:
+            raise ValueError(f"num_downscales >= 0 and resolution_schedule >= 1 expected, got {self.num_downscales} and {self.resolution_schedule}")
         if self.use_bilateral_grid:
             from .bilateral_grid import check_grid_shape
 
@@ -408,6 +415,24 @@ def adam_step_torch(arena: GaussianArena, lrs: Dict[str, float], lr_sh_rest: flo
     arena.param.sub_(lr / bias1 * (arena.exp_avg / denom))
 
 
+def rescaled_camera(Ks: Tensor, width: int, height: int, factor: int) -> Tuple[Tensor, int, int]:
+    """The render camera of a step at 1/factor resolution, as nerfstudio's `Cameras.rescale_output_resolution(1 / factor)`
+    builds it: rows 0-1 of the intrinsics [C,3,3] times 1/factor (float32), size floor(W / factor + 0.5) x
+    floor(H / factor + 0.5).  ValueError when that size is not the size of the box-downscaled ground truth
+    (data_side.downscaled_size: W // factor x H // factor), where splatfacto's L1 would fail to broadcast."""
+    from .data_side import downscaled_size
+
+    if factor == 1:
+        return Ks, width, height
+    w, h = math.floor(width / factor + 0.5), math.floor(height / factor + 0.5)
+    gw, gh = downscaled_size(width, height, factor)
+    if (w, h) != (gw, gh):
+        raise ValueError(f"{width}x{height} at 1/{factor}: the rescaled camera is {w}x{h} but the downscaled ground truth is {gw}x{gh}")
+    Ks = Ks.clone()
+    Ks[..., :2, :] *= 1.0 / factor
+    return Ks, w, h
+
+
 class SplatTrainer:
     """One process per GPU.  `step()` = render local views + loss + backward + gradient all-reduce + Adam
     (+ densify / opacity reset on schedule)."""
@@ -572,6 +597,11 @@ class SplatTrainer:
         c = self.cfg
         return min(self.step_count // c.sh_degree_interval, c.sh_degree)
 
+    def downscale_factor(self) -> int:
+        """splatfacto `_get_downscale_factor` while training: the resolution divisor of the current step."""
+        c = self.cfg
+        return 2 ** max(c.num_downscales - self.step_count // c.resolution_schedule, 0)
+
     def accumulate_stats(self, absgrad_or_packed: Tensor, radii: Tensor, width: int, height: int, packed: bool,
                          n_cameras: Optional[int] = None) -> None:
         """DefaultStrategy._update_state for the local views.  gsplat scales the image-plane gradient by
@@ -726,7 +756,10 @@ class SplatTrainer:
         Returns (loss[3] device tensor of the local views -- a fresh copy, safe to keep for logging --, refine info|None);
         the camera optimizer's regulariser is `camera_opt_loss`.
         With the bilateral grid on, `camera_ids` [C] (the training camera of each view, the same ids the camera optimizer
-        uses) selects each view's grid; the grids' TV loss is `bilagrid_tv_loss`."""
+        uses) selects each view's grid; the grids' TV loss is `bilagrid_tv_loss`.
+        With cfg.num_downscales > 0 the camera (Ks, width, height) and gt_rgb / gt_depth / mask are at full resolution, as
+        nerfstudio's datamanager supplies them; a step whose `downscale_factor()` d is above 1 renders at the camera
+        `rescaled_camera` builds and trains against the ground truth box-downscaled by d."""
         if self._fused is None:
             raise RuntimeError("rendering needs the CUDA library (backend='cuda'); there is no CPU fallback")
         c, a, cam, bg = self.cfg, self.arena, self.camera_opt, self.bilagrid
@@ -746,6 +779,9 @@ class SplatTrainer:
                 raise ValueError("bilateral grid on: pass camera_ids= (the training camera of each view)")
             camera_ids = check_camera_ids(camera_ids, viewmats.shape[0], bg.num_grids, self.device)
         C = viewmats.shape[0]
+        # the resolution schedule: every rank derives the same factor from step_count
+        d = self.downscale_factor()
+        Ks, width, height = rescaled_camera(Ks, width, height, d)
         total = total_views or C * self.world
         xg = self._exchange_for(C) if self.comm == "exchange" else None  # may fall back to "nccl" (comm="auto", no symmetric memory)
         # "nccl" with one view per rank: the SH gradients are all-reduced and Adam-stepped in `comm_chunks` Gaussian ranges
@@ -770,7 +806,7 @@ class SplatTrainer:
                                depth_lambda=c.depth_lambda, grad_scale=C / float(total), rasterize_mode=c.rasterize_mode,
                                activations=3,  # ACT_LOG_SCALES | ACT_LOGIT_OPACITIES (pipeline.py / include/qed_splat.h)
                                mask=mask, depth_unit_scale=c.depth_unit_scale, ssim_lambda=c.ssim_lambda, pose_gradients=cam is not None,
-                               bilateral_grid=None if bl is None else (bg.grids, camera_ids, bl[3]), **comm_args)
+                               bilateral_grid=None if bl is None else (bg.grids, camera_ids, bl[3]), gt_downscale=d, **comm_args)
         self.accumulate_stats(out.packed_grads, out.radii, width, height, packed=True, n_cameras=total)
         self._gaussian_update(pipelined, chunked_bwd, works)
         if cam is not None:

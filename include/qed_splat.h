@@ -358,6 +358,40 @@ int qed_arena_gather(int64_t n_new, const int32_t* src, const uint8_t* fresh, co
                      float* new_param, float* new_exp_avg, float* new_exp_avg_sq, const int64_t* new_group_starts,
                      qed_stream_t stream);
 
+/* Splatfacto's MCMC strategy (nerfstudio strategy="mcmc" -> gsplat MCMCStrategy) on the flat arenas above (group_starts:
+ * HOST int64[5], the quats and SH starts multiples of 4 floats, param 16-byte aligned).  o = sigmoid(logit-opacity).
+ * Random numbers: Philox4x32-10 (curand_Philox4x32_10) with key = seed and counter = (index, step, stream_id, 0).
+ *
+ * qed_mcmc_census: dead rows (o <= min_opacity, float32) -> dead_idx[0 .. n_dead) ascending, *n_dead_dev (device int64).
+ * qed_mcmc_sample: weights w_i = floor(o_i * 2^24) (o in float64; 0 for dead rows when zero_dead), their exact int64
+ *   inclusive scan, *total_dev = sum w.  Draw j (< n_draws, with replacement) = first row i with scan[i] > u_j, u_j =
+ *   (64-bit Philox word (x << 32 | y) of counter (j, step, stream_id, 0) * total) >> 64; counts[N] = bincount(draws)
+ *   (overwritten).  total == 0: draws untouched, counts zero.
+ *   Both take workspace_bytes >= qed_mcmc_workspace_bytes(N) (16-byte aligned).
+ * qed_mcmc_relocate: every row i with counts[i] > 0 gets gsplat compute_relocation at ratio min(counts[i] + 1, 51):
+ *   o' = 1 - (1 - o)^(1/ratio) (then clamped to [min_opacity, 1 - FLT_EPSILON]), scale' = o / D(o', ratio) * scale with
+ *   D(x, n) = sum_{j=1..n} C(n, j) (-1)^(j-1) x^j / sqrt(j) in float64; with zero_moments its exp_avg / exp_avg_sq rows
+ *   are zeroed.  Then, after that, parameter row src[j] is copied to row dst[j] for j < n_copies (src and dst disjoint;
+ *   the moments of dst are kept).  exp_avg / exp_avg_sq may be NULL without zero_moments.
+ * qed_mcmc_noise: means += R diag(s)^2 R^T (n * sigmoid(100 ((1 - o) - 0.995)) * scaler) with n = three Box-Muller normals
+ *   of counter (i, step, 0, 0), s = exp(log-scales), R of the normalised quaternion.
+ * qed_mcmc_reg: loss[0] = opacity_reg * mean_N o, loss[1] = scale_reg * mean_3N exp(log-scale) (device floats); their
+ *   gradients opacity_reg / N * o (1 - o) and scale_reg / (3 N) * exp(log-scale) are ADDED to grad (same layout).
+ *   workspace_bytes >= qed_mcmc_reg_workspace_bytes(), zeroed before the first call (every call leaves it zeroed).
+ *   Deterministic: fixed-order float64 sums. */
+size_t qed_mcmc_workspace_bytes(int64_t N);
+int qed_mcmc_census(int64_t N, const float* logit_opacities, float min_opacity, int32_t* dead_idx, int64_t* n_dead_dev, void* workspace,
+                    size_t workspace_bytes, qed_stream_t stream);
+int qed_mcmc_sample(int64_t N, const float* logit_opacities, float min_opacity, int zero_dead, int64_t n_draws, uint64_t seed, uint32_t step,
+                    uint32_t stream_id, int32_t* draws, int32_t* counts, int64_t* total_dev, void* workspace, size_t workspace_bytes,
+                    qed_stream_t stream);
+int qed_mcmc_relocate(int64_t N, const int32_t* counts, float min_opacity, int zero_moments, int64_t n_copies, const int32_t* src,
+                      const int32_t* dst, float* param, float* exp_avg, float* exp_avg_sq, const int64_t* group_starts, qed_stream_t stream);
+int qed_mcmc_noise(int64_t N, float* param, const int64_t* group_starts, float scaler, uint64_t seed, uint32_t step, qed_stream_t stream);
+size_t qed_mcmc_reg_workspace_bytes(void);
+int qed_mcmc_reg(int64_t N, const float* param, const int64_t* group_starts, float opacity_reg, float scale_reg, float* grad, float* loss,
+                 void* workspace, size_t workspace_bytes, qed_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * camera + data side (SURVEY.md section 8 rows a1 and f4)
  */

@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import c_double, c_float, c_int, c_int32, c_int64, c_size_t, c_void_p
+from ctypes import c_double, c_float, c_int, c_int32, c_int64, c_size_t, c_uint32, c_uint64, c_void_p
 from pathlib import Path
 
 _PKG = Path(__file__).resolve().parent
@@ -67,6 +67,13 @@ SIGNATURES = {
     "qed_comm_barrier": (c_int, [P, c_int, c_int, ctypes.c_uint32, P]),
     "qed_comm_allreduce_f32": (c_int, [P, P, P, c_int, c_int, c_int64, c_int64, ctypes.c_uint32, c_int, P]),
     "qed_arena_gather": (c_int, [c_int64, P, P, P, P, P, P, P, P, P, P, P, P, P, P]),
+    "qed_mcmc_workspace_bytes": (c_size_t, [c_int64]),
+    "qed_mcmc_census": (c_int, [c_int64, P, c_float, P, P, P, c_size_t, P]),
+    "qed_mcmc_sample": (c_int, [c_int64, P, c_float, c_int, c_int64, c_uint64, c_uint32, c_uint32, P, P, P, P, c_size_t, P]),
+    "qed_mcmc_relocate": (c_int, [c_int64, P, c_float, c_int, c_int64, P, P, P, P, P, P, P]),
+    "qed_mcmc_noise": (c_int, [c_int64, P, P, c_float, c_uint64, c_uint32, P]),
+    "qed_mcmc_reg_workspace_bytes": (c_size_t, []),
+    "qed_mcmc_reg": (c_int, [c_int64, P, P, c_float, c_float, P, P, P, c_size_t, P]),
     "qed_viewmat_from_c2w": (c_int, [c_int, c_int, P, P, P]),
     "qed_viewmat_from_c2w_bwd": (c_int, [c_int, c_int, P, P, P, P]),
     "qed_camera_opt_apply": (c_int, [c_int, c_int, c_int, P, P, P, P, P]),

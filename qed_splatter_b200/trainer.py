@@ -107,6 +107,15 @@ class TrainConfig:
     # (and qed-splatter's) is num_downscales = 2; it stays 0 (always full resolution) here so existing runs are unchanged.
     num_downscales: int = 0
     resolution_schedule: int = 3000
+    # densification strategy: "default" (gsplat DefaultStrategy: the fields above) or "mcmc" (gsplat MCMCStrategy, mcmc.py:
+    # relocation of dead Gaussians and capped growth every refine_every steps in (warmup_length, stop_split_at), position
+    # noise every step, no opacity reset; min_opacity = cull_alpha_thresh).  [UP] = nerfstudio 1.1.5 SplatfactoModelConfig
+    # defaults restated from memory of the upstream code.
+    strategy: str = "default"  # [UP]
+    max_gs_num: int = 1_000_000  # [UP] MCMC cap_max: the add step never grows past it
+    noise_lr: float = 5e5  # [UP] position noise scale = means lr * noise_lr
+    mcmc_opacity_reg: float = 0.01  # [UP] weight of mean(sigmoid(logit-opacities)) in the loss (MCMC only)
+    mcmc_scale_reg: float = 0.01  # [UP] weight of mean(exp(log-scales)) in the loss (MCMC only)
 
     def __post_init__(self):
         self.validate()
@@ -117,6 +126,17 @@ class TrainConfig:
 
         if self.camera_optimizer not in CAMERA_OPTIMIZER_MODES:
             raise ValueError(f"camera_optimizer must be one of {CAMERA_OPTIMIZER_MODES}, got {self.camera_optimizer!r}")
+        from .mcmc import MIN_OPACITY_FLOOR, STRATEGIES
+
+        if self.strategy not in STRATEGIES:
+            raise ValueError(f"strategy must be one of {STRATEGIES}, got {self.strategy!r}")
+        if self.max_gs_num < 1:
+            raise ValueError(f"max_gs_num >= 1 expected, got {self.max_gs_num}")
+        if self.noise_lr < 0 or self.mcmc_opacity_reg < 0 or self.mcmc_scale_reg < 0:
+            raise ValueError("noise_lr, mcmc_opacity_reg and mcmc_scale_reg must be >= 0")
+        if self.strategy == "mcmc" and not (MIN_OPACITY_FLOOR <= self.cull_alpha_thresh < 1.0):
+            # every alive Gaussian then has a positive sampling weight floor(o * 2^24) (mcmc.py)
+            raise ValueError(f"strategy='mcmc' needs 2^-23 <= cull_alpha_thresh < 1, got {self.cull_alpha_thresh}")
         if self.num_downscales < 0 or self.resolution_schedule < 1:
             raise ValueError(f"num_downscales >= 0 and resolution_schedule >= 1 expected, got {self.num_downscales} and {self.resolution_schedule}")
         if self.use_bilateral_grid:
@@ -479,6 +499,14 @@ class SplatTrainer:
             self.bilagrid = BilateralGridOptimizer(num_cameras, self.device, shape=c.bilateral_grid_shape, lr=c.bilateral_grid_lr,
                                                    lr_final=c.bilateral_grid_lr_final, warmup_steps=c.bilateral_grid_warmup, max_steps=c.max_steps,
                                                    tv_weight=c.bilateral_grid_tv_weight, betas=c.adam_betas, eps=c.adam_eps, backend=backend)
+        self.mcmc = None
+        if self.cfg.strategy == "mcmc":
+            from .mcmc import MCMCStrategy
+
+            c = self.cfg
+            self.mcmc = MCMCStrategy(self.device, cap_max=c.max_gs_num, noise_lr=c.noise_lr, refine_start=c.warmup_length, refine_stop=c.stop_split_at,
+                                     refine_every=c.refine_every, min_opacity=c.cull_alpha_thresh, opacity_reg=c.mcmc_opacity_reg,
+                                     scale_reg=c.mcmc_scale_reg, seed=c.seed, impl="fused" if backend == "cuda" else "torch")
 
     @property
     def pose_adjustment(self) -> Optional[Tensor]:
@@ -500,6 +528,11 @@ class SplatTrainer:
         """The grids' total-variation loss of the last step (device scalar [1]); None when the grid is off."""
         return None if self.bilagrid is None else self.bilagrid.tv_loss
 
+    @property
+    def mcmc_reg_loss(self) -> Optional[Tensor]:
+        """The MCMC regularisers of the last step (device [2]: opacity term, scale term); None with strategy "default"."""
+        return None if self.mcmc is None else self.mcmc.reg_loss
+
     def _pick_comm(self) -> str:
         c = self.cfg.comm
         if self.world <= 1:
@@ -515,7 +548,8 @@ class SplatTrainer:
 
     def _exchange_for(self, views_per_rank: int):
         """The symmetric gradient arena + exchange buffers for the current Gaussian count (rebuilt, collectively, when a
-        refine step changed N: every rank refines at the same step)."""
+        refine step changed N: every rank refines at the same step).  With MCMC the set never grows past max_gs_num, so the
+        buffers are sized for that once and never rebuilt."""
         from .comm import ViewShardedGradients
 
         x = self._xg
@@ -525,8 +559,11 @@ class SplatTrainer:
 
             err = None
             try:
-                x = ViewShardedGradients(self.arena.N, views_per_rank, self.device, self.pg,
-                                         headroom=0.25 if self.step_count < self.cfg.stop_split_at else 0.0,
+                if self.mcmc is not None:  # room for max_gs_num Gaussians: MCMC never grows past it
+                    headroom = max(self.cfg.max_gs_num / self.arena.N - 1.0, 0.0)
+                else:
+                    headroom = 0.25 if self.step_count < self.cfg.stop_split_at else 0.0
+                x = ViewShardedGradients(self.arena.N, views_per_rank, self.device, self.pg, headroom=headroom,
                                          num_cameras=0 if self.camera_opt is None else self.camera_opt.num_cameras,
                                          bilagrid_row=0 if self.bilagrid is None else self.bilagrid.row)
             except Exception as e:  # noqa: BLE001  (no peer mappings / symmetric memory on this box)
@@ -576,6 +613,7 @@ class SplatTrainer:
         if not pipelined:
             if self.comm == "nccl":
                 self._all_reduce(a.grad)
+            self._mcmc_regularize()
             self.optimizer_step()
             return
         import torch.distributed as dist
@@ -590,7 +628,13 @@ class SplatTrainer:
             w.wait()
             self.optimizer_step(lo, hi)
         head.wait()
+        self._mcmc_regularize()  # opacities and scales lie in [0, sh0)
         self.optimizer_step(0, sh0)
+
+    def _mcmc_regularize(self) -> None:
+        """MCMC: the regularisers' gradients, added once to the gradients summed over the ranks (identical on every rank)."""
+        if self.mcmc is not None:
+            self.mcmc.regularize(self.arena)
 
     # -- pieces that the tests drive directly ---------------------------------------------------
     def sh_degree_to_use(self) -> int:
@@ -728,8 +772,12 @@ class SplatTrainer:
 
     def maybe_refine(self, step: int) -> Optional[Dict[str, int]]:
         """DefaultStrategy.step_post_backward schedule, called after the optimizer step of 0-based iteration
-        `step` (nerfstudio passes its 0-based step; note gsplat resets opacities at step 0 too)."""
+        `step` (nerfstudio passes its 0-based step; note gsplat resets opacities at step 0 too).
+        strategy "mcmc": MCMCStrategy.step_post_backward with the means lr after the scheduler step -> {"n_relocated",
+        "n_added", "n"} on refine steps, position noise on every step."""
         c = self.cfg
+        if self.mcmc is not None:
+            return self.mcmc.step_post_backward(self.arena, step, c.lr_means_at(step + 1))
         info = None
         if step >= c.stop_split_at:
             return None
@@ -807,7 +855,8 @@ class SplatTrainer:
                                activations=3,  # ACT_LOG_SCALES | ACT_LOGIT_OPACITIES (pipeline.py / include/qed_splat.h)
                                mask=mask, depth_unit_scale=c.depth_unit_scale, ssim_lambda=c.ssim_lambda, pose_gradients=cam is not None,
                                bilateral_grid=None if bl is None else (bg.grids, camera_ids, bl[3]), gt_downscale=d, **comm_args)
-        self.accumulate_stats(out.packed_grads, out.radii, width, height, packed=True, n_cameras=total)
+        if self.mcmc is None:  # MCMC uses no gradient statistics
+            self.accumulate_stats(out.packed_grads, out.radii, width, height, packed=True, n_cameras=total)
         self._gaussian_update(pipelined, chunked_bwd, works)
         if cam is not None:
             self._camera_opt_update(out.v_viewmats, camera_ids, camera_to_worlds, xg)

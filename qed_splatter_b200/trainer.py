@@ -25,9 +25,10 @@ NOT a rendering fallback — rendering always needs the CUDA library).
 """
 from __future__ import annotations
 
+import dataclasses
 import math
 from dataclasses import dataclass, field
-from typing import Dict, Optional, Tuple
+from typing import Any, Dict, Optional, Tuple
 
 import torch
 from torch import Tensor
@@ -36,6 +37,13 @@ GROUPS = ("means", "quats", "scales", "opacities", "sh")
 GROUP_SHAPES = {"means": (3,), "quats": (4,), "scales": (3,), "opacities": (), "sh": (16, 3)}  # per Gaussian
 GROUP_DIMS = {g: math.prod(GROUP_SHAPES[g]) for g in GROUPS}
 FLOATS_PER_GAUSSIAN = sum(GROUP_DIMS.values())  # 59
+
+# SplatTrainer.state_dict(): splatfacto's stored Gaussian parameters (and optimizer groups), per-Gaussian shapes
+CHECKPOINT_FORMAT_VERSION = 1
+SPLATFACTO_SHAPES = {"means": (3,), "scales": (3,), "quats": (4,), "features_dc": (3,), "features_rest": (15, 3), "opacities": (1,)}
+STRATEGY_STATS = ("grad2d", "count", "radii")
+# TrainConfig fields that decide which tables a state holds and their shapes: a resumed run cannot change them
+LAYOUT_FIELDS = ("strategy", "camera_optimizer", "use_bilateral_grid", "bilateral_grid_shape")
 
 
 @dataclass
@@ -210,6 +218,13 @@ class GaussianArena:
 
     def views(self, buf: Tensor) -> Dict[str, Tensor]:
         return {g: self.view(buf, g) for g in GROUPS}
+
+    def splatfacto_views(self, buf: Tensor) -> Dict[str, Tensor]:
+        """Views of `buf` in splatfacto's names and shapes (SPLATFACTO_SHAPES): the SH block as features_dc [N,3] and
+        features_rest [N,15,3], the opacities as [N,1]."""
+        v = self.views(buf)
+        return {"means": v["means"], "scales": v["scales"], "quats": v["quats"], "features_dc": v["sh"][:, 0, :],
+                "features_rest": v["sh"][:, 1:, :], "opacities": v["opacities"][:, None]}
 
 
 @dataclass
@@ -453,6 +468,26 @@ def rescaled_camera(Ks: Tensor, width: int, height: int, factor: int) -> Tuple[T
     return Ks, w, h
 
 
+def _owned_cpu(t: Tensor) -> Tensor:
+    """A contiguous CPU copy of `t` whose storage holds exactly its elements (torch.save of a view writes the whole buffer
+    behind it)."""
+    out = torch.empty(t.shape, dtype=t.dtype, device="cpu")
+    out.copy_(t.detach())
+    return out
+
+
+def _check_shape(what: str, t: Any, shape) -> None:
+    if not isinstance(t, Tensor) or tuple(t.shape) != tuple(shape):
+        got = tuple(t.shape) if isinstance(t, Tensor) else type(t).__name__
+        raise ValueError(f"state {what}: expected a tensor of shape {tuple(shape)}, got {got}")
+
+
+def _section(state: Dict, key: str) -> Dict:
+    if not isinstance(state.get(key), dict):
+        raise ValueError(f"state {key!r}: missing (the saved configuration needs it)")
+    return state[key]
+
+
 class SplatTrainer:
     """One process per GPU.  `step()` = render local views + loss + backward + gradient all-reduce + Adam
     (+ densify / opacity reset on schedule)."""
@@ -468,6 +503,7 @@ class SplatTrainer:
         self.pg = process_group
         self.backend = backend
         self.device = means.device
+        self.num_cameras = int(num_cameras)
         self.arena = GaussianArena(means, quats, log_scales, logit_opacities, sh)
         self.state = StrategyState.zeros(self.arena.N, self.device)
         self.step_count = 0
@@ -866,3 +902,136 @@ class SplatTrainer:
         info = self.maybe_refine(self.step_count)
         self.step_count += 1
         return loss, info
+
+    # -- checkpoints -----------------------------------------------------------------------------
+    def _gather_rows(self, t: Tensor) -> Tensor:
+        """[world, N] on the CPU: row r = rank r's `t` (a collective with world_size > 1)."""
+        if self.world <= 1:
+            return _owned_cpu(t)[None]
+        import torch.distributed as dist
+
+        rows = [torch.empty_like(t) for _ in range(self.world)]
+        dist.all_gather(rows, t.contiguous(), group=self.pg)
+        return _owned_cpu(torch.stack(rows))
+
+    @torch.no_grad()
+    def state_dict(self) -> Dict[str, Any]:
+        """Everything the run needs to continue (DESIGN.md section 0 lists it), as plain Python values and CPU tensors that own
+        their storage, so `torch.save` writes exactly them and `torch.load(weights_only=True)` reads them back.  Call it
+        between steps; with world_size > 1 it is collective (the strategy statistics of every rank are gathered) and every
+        rank gets the same dict.  The live trainer is left as it was.
+
+        Keys: format_version, config (dataclasses.asdict), step, num_cameras, world_size, gauss_params / exp_avg / exp_avg_sq
+        (splatfacto's names and shapes: means, scales (log), quats (as stored), features_dc, features_rest, opacities (logit)
+        [N,1]), strategy_state (strategy "default": grad2d, count, radii [world_size, N], row r from rank r),
+        camera_optimizer (pose_adjustment, exp_avg, exp_avg_sq [num_cameras, 6]) and bil_grids (grids, exp_avg, exp_avg_sq
+        [num_cameras, 12, L, Y, X]) when those are on."""
+        a = self.arena
+        out: Dict[str, Any] = dict(format_version=CHECKPOINT_FORMAT_VERSION, config=dataclasses.asdict(self.cfg), step=int(self.step_count),
+                                   num_cameras=self.num_cameras, world_size=int(self.world))
+        for key, buf in (("gauss_params", a.param), ("exp_avg", a.exp_avg), ("exp_avg_sq", a.exp_avg_sq)):
+            out[key] = {k: _owned_cpu(v) for k, v in a.splatfacto_views(buf).items()}
+        if self.mcmc is None:
+            out["strategy_state"] = {k: self._gather_rows(getattr(self.state, k)) for k in STRATEGY_STATS}
+        if self.camera_opt is not None:
+            n = self.camera_opt.num_cameras * 6
+            out["camera_optimizer"] = {k: _owned_cpu(getattr(self.camera_opt, b)[:n].view(-1, 6))
+                                       for k, b in (("pose_adjustment", "param"), ("exp_avg", "exp_avg"), ("exp_avg_sq", "exp_avg_sq"))}
+        if self.bilagrid is not None:
+            shape = self.bilagrid.grids.shape
+            out["bil_grids"] = {k: _owned_cpu(getattr(self.bilagrid, b).view(shape))
+                                for k, b in (("grids", "param"), ("exp_avg", "exp_avg"), ("exp_avg_sq", "exp_avg_sq"))}
+        return out
+
+    @classmethod
+    @torch.no_grad()
+    def from_state_dict(cls, state: Dict[str, Any], cfg: Optional[TrainConfig] = None, *, rank: int = 0, world_size: int = 1,
+                        process_group=None, backend: str = "cuda", device=None) -> "SplatTrainer":
+        """A trainer that continues the run `state` (from `state_dict()`, possibly through torch.save / torch.load) at step
+        state["step"]: the next `step()` is the one the saved run would have taken.
+
+        `cfg=None` uses the saved configuration; a `cfg` passed in may change hyper-parameters (max_steps, learning rates,
+        comm, ...) but not the layout fields (LAYOUT_FIELDS: ValueError naming the field).  ValueError also for an unknown
+        format_version, a tensor whose shape disagrees with N, num_cameras or the grid shape, and an MCMC state with more
+        than cfg.max_gs_num Gaussians.
+
+        Strategy statistics ("default"): at the saved world size rank r takes row r, so the run continues exactly.  At another
+        world size rank 0 takes the rows' sum (radii: their maximum) and the other ranks zeros; the next refine step reduces
+        them over the ranks to the same totals (grad2d up to the float summation order).
+
+        Nothing else needs loading: the multi-GPU exchange buffers are built by the first `step()` as for a new trainer.
+        `device`: default the current CUDA device with backend "cuda", the CPU with backend "torch" (which opens a
+        checkpoint of a CUDA run on a machine without a GPU)."""
+        version = state.get("format_version") if isinstance(state, dict) else None
+        if version != CHECKPOINT_FORMAT_VERSION:
+            raise ValueError(f"state format_version {version!r} unknown: this trainer reads version {CHECKPOINT_FORMAT_VERSION}")
+        saved = TrainConfig(**state["config"])
+        if cfg is None:
+            cfg = saved
+        for f in LAYOUT_FIELDS:
+            old, new = getattr(saved, f), getattr(cfg, f)
+            if f == "bilateral_grid_shape":
+                if not saved.use_bilateral_grid:
+                    continue
+                old, new = tuple(old), tuple(new)
+            if old != new:
+                raise ValueError(f"cfg.{f} = {new!r} would change the state's layout (saved with {old!r})")
+        cfg.validate()
+        if device is None:
+            device = torch.device("cuda", torch.cuda.current_device()) if backend == "cuda" else torch.device("cpu")
+        device = torch.device(device)
+        # shapes, before anything is allocated
+        num_cameras = int(state["num_cameras"])
+        saved_world = int(state["world_size"])
+        gp = _section(state, "gauss_params")
+        if not isinstance(gp.get("means"), Tensor) or gp["means"].dim() != 2:
+            raise ValueError("state gauss_params['means']: expected a tensor of shape (N, 3)")
+        N = gp["means"].shape[0]
+        for key in ("gauss_params", "exp_avg", "exp_avg_sq"):
+            sec = _section(state, key)
+            for k, shape in SPLATFACTO_SHAPES.items():
+                _check_shape(f"{key}[{k!r}]", sec.get(k), (N, *shape))
+        if cfg.strategy == "mcmc" and N > cfg.max_gs_num:
+            raise ValueError(f"state holds {N} Gaussians, more than cfg.max_gs_num = {cfg.max_gs_num} (strategy 'mcmc')")
+        if cfg.strategy == "default":
+            sec = _section(state, "strategy_state")
+            for k in STRATEGY_STATS:
+                _check_shape(f"strategy_state[{k!r}]", sec.get(k), (saved_world, N))
+        tables = []
+        if cfg.camera_optimizer != "off":
+            tables.append(("camera_optimizer", ("pose_adjustment", "exp_avg", "exp_avg_sq"), (num_cameras, 6)))
+        if cfg.use_bilateral_grid:
+            X, Y, L = cfg.bilateral_grid_shape
+            tables.append(("bil_grids", ("grids", "exp_avg", "exp_avg_sq"), (num_cameras, 12, L, Y, X)))
+        for key, names, shape in tables:
+            sec = _section(state, key)
+            for k in names:
+                _check_shape(f"{key}[{k!r}]", sec.get(k), shape)
+
+        sh = torch.cat([gp["features_dc"][:, None, :], gp["features_rest"]], dim=1)
+        tr = cls(gp["means"].to(device), gp["quats"].to(device), gp["scales"].to(device), gp["opacities"].reshape(N).to(device), sh.to(device),
+                 cfg=cfg, rank=rank, world_size=world_size, process_group=process_group, backend=backend, num_cameras=num_cameras)
+        a = tr.arena
+        for key, buf in (("exp_avg", a.exp_avg), ("exp_avg_sq", a.exp_avg_sq)):
+            for k, v in a.splatfacto_views(buf).items():
+                v.copy_(state[key][k])
+        tr.step_count = int(state["step"])
+        if tr.mcmc is None:
+            for k in STRATEGY_STATS:
+                rows = state["strategy_state"][k]
+                if saved_world == world_size:
+                    v = rows[rank]
+                elif rank == 0:
+                    v = rows.amax(0) if k == "radii" else rows.sum(0)
+                else:
+                    continue  # zeros, as built
+                getattr(tr.state, k).copy_(v)
+        if tr.camera_opt is not None:
+            sec, n = state["camera_optimizer"], num_cameras * 6
+            for k, b in (("pose_adjustment", "param"), ("exp_avg", "exp_avg"), ("exp_avg_sq", "exp_avg_sq")):
+                getattr(tr.camera_opt, b)[:n].copy_(sec[k].reshape(-1))
+        if tr.bilagrid is not None:
+            sec = state["bil_grids"]
+            for k, b in (("grids", "param"), ("exp_avg", "exp_avg"), ("exp_avg_sq", "exp_avg_sq")):
+                getattr(tr.bilagrid, b).copy_(sec[k].reshape(-1))
+        return tr

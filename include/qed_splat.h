@@ -308,6 +308,28 @@ int qed_downscale_ground_truth(int C, int width, int height, int factor, const v
                                int depth_is_u16, double depth_unit_scale, const void* mask, int mask_is_u8, float* out_rgb,
                                float* out_depth, float* out_mask, qed_stream_t stream);
 
+/* Held-out evaluation metrics of C rendered views (nerfstudio's eval: torchmetrics PSNR / SSIM, and qed-splatter's
+ * DepthMetrics, metrics.py:115-156), forward only.
+ *  render[C,height,width,4] (RGB + depth), alphas[C,height,width], gt_rgb / gt_depth / depth_unit_scale as for
+ *  qed_loss_fwd_bwd (u8 * (1.0f / 255.0f); float(double(u16) * depth_unit_scale)), bg[3].
+ *  Per view, with the prediction formed as qed_loss_fwd_bwd forms it: rgb = clamp(render.rgb + (1 - alpha) bg, 0, 1);
+ *  depth = the depth channel where alpha > 0, else the view's maximum rendered depth.  metrics_dev[c * QED_EVAL_METRICS + k]
+ *  (overwritten) holds, in this order:
+ *    psnr = 10 log10(1 / rgb_mse) (+inf for a perfect image); ssim = the loss's SSIM (11x11 Gaussian window, sigma 1.5,
+ *    valid windows, C1 = 1e-4, C2 = 9e-4, mean over channels and pixels, no mask); rgb_mse = mean over H*W*3 of
+ *    (rgb - gt)^2; then, over the pixels whose ground-truth depth g is finite and > depth_tolerance, with d the predicted
+ *    depth: abs_rel = mean |g - d| / g, sq_rel = mean (g - d)^2 / g, rmse = sqrt(mean (g - d)^2),
+ *    rmse_log = sqrt(mean (log g - log d)^2), a1 / a2 / a3 = mean [max(g / d, d / g) < 1.25^k], and n_depth = their
+ *    number.  With n_depth = 0 the seven depth values are NaN; non-finite values (d = 0) propagate.
+ *  Sums in float64, per-block partials summed in a fixed order: the same inputs give the same bits, and a view's row does
+ *  not depend on the other views.  workspace_bytes >= qed_eval_metrics_workspace_bytes (16-byte aligned).
+ *  QED_ERR_UNSUPPORTED when width or height <= 10 (no valid SSIM window) or C > 21845. */
+#define QED_EVAL_METRICS 11 /* psnr, ssim, rgb_mse, abs_rel, sq_rel, rmse, rmse_log, a1, a2, a3, n_depth */
+size_t qed_eval_metrics_workspace_bytes(int C, int width, int height);
+int qed_eval_metrics(int C, int width, int height, const float* render, const float* alphas, const void* gt_rgb, int gt_rgb_is_u8,
+                     const void* gt_depth, int gt_depth_is_u16, double depth_unit_scale, const float* bg, float depth_tolerance,
+                     double* metrics_dev, void* workspace, size_t workspace_bytes, qed_stream_t stream);
+
 /* Total-variation regulariser of the bilateral grids (splatfacto get_loss_dict while training):
  *  loss_out[1] = weight / G * sum_{axes d in L, Y, X} sum (x[.., i+1, ..] - x[.., i, ..])^2 / (elements of one grid's
  *  difference along d, i.e. 12 L Y X (n_d - 1) / n_d).  v_grids[G,12,L,Y,X] is OVERWRITTEN with its gradient;

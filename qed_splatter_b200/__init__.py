@@ -8,6 +8,7 @@ loss-gradient / trainer step built on the same kernels.  Hand-written CUDA behin
 from .rendering import rasterization  # noqa: F401
 from .losses import bilateral_grid_tv_loss, depth_supervised_loss  # noqa: F401
 from .data_side import get_viewmat  # noqa: F401
-from . import data_side, ops, scenes  # noqa: F401
+from .metrics import image_metrics, summarize  # noqa: F401
+from . import data_side, metrics, ops, scenes  # noqa: F401
 
 __version__ = "0.1.0"

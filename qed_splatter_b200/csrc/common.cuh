@@ -102,6 +102,9 @@ struct GtDepth {
     }
 };
 
+// Per-block partial sums of the held-out metrics pass (ssim.cu, SsimEval), summed per view by metrics.cu.
+constexpr int kEvalPartials = 10;
+
 // Optional per-pixel loss mask of the batch (`batch["mask"]`, qed_splatter/model.py:93-97; splatfacto multiplies the
 // RGB images by it too): float32 or uint8 / bool [C,H,W]; NULL = all ones.
 struct PixelMask {

@@ -8,6 +8,8 @@
 // forward kernel : one CTA per 32x32 tile of the valid output, separable 11-tap filter in shared memory (register sliding
 //                  windows, two adjacent outputs per FFMA2: the weight pair (w[k], w[k-1]) times a broadcast input), writes
 //                  the three partial-derivative maps d map/d(mu2, e2, e12) and accumulates sum(map).
+//                  Its EVAL instantiation (held-out metrics, metrics.cu) forms the prediction from the render itself and
+//                  writes per-block partial sums instead (see SsimEval).
 // backward kernel: dL/dY(p) = sum_q w(q-p) [Dmu(q) + 2 Y(p) De2(q) + X(p) De12(q)] * scale  (zero outside the
 //                  valid region), again separable.  HBM-bound: ~15 floats per pixel-channel moved in total.
 #include "common.cuh"
@@ -70,10 +72,31 @@ __device__ __forceinline__ void filter_taps(const GaussWin& win, f32x2 (&acc2)[N
     }
 }
 
+// The held-out metrics' view of the kernel (ssim_fwd_kernel<true>): the prediction is clamp(rgb + (1 - alpha) bg, 0, 1)
+// of the render, formed as loss_grad_kernel forms it, against the unmasked ground truth.  Each block owns the input pixels
+// [x0, x0 + 32) x [y0, y0 + 32) of its tile (the last tile of a row / column also the up to 10 pixels after them: together
+// every pixel once) and writes, in fixed order, partials[(cam * 3 + ch) * tiles + tile][kEvalPartials] =
+//   {sum SSIM map, sum (pred - gt)^2 of channel ch, then for ch == 0 (zeros otherwise) over its pixels with finite ground
+//    truth > depth_tol: n, sum |g - d| / g, sum (g - d)^2 / g, sum (g - d)^2, sum (log g - log d)^2, and the counts of
+//    max(g / d, d / g) < 1.25, 1.25^2, 1.25^3}
+// with d = the depth channel where alpha > 0, else the view's fill value fill[cam] (float bits).  Sums in float64.
+
+struct SsimEval {
+    const float4* render;  // [C,H,W,4]
+    const float* alphas;   // [C,H,W]
+    const float* bg;       // [3]
+    GtDepth gt_depth;
+    const int* fill;       // [C] the view's maximum rendered depth, as float bits
+    float depth_tol;
+    double* partials;
+};
+
 // grid (tiles_x, tiles_y, C*3); 256 threads.
+template <bool EVAL>
 __global__ void __launch_bounds__(kSsimThreads) ssim_fwd_kernel(int W, int H, const float* __restrict__ pred /*[C,H,W,3]*/,
                                                                 const GtImage gt, const PixelMask mask, const GaussWin win,
-                                                                float* __restrict__ dmaps /*[C*3][3][OH][OW]*/, double* __restrict__ stats) {
+                                                                float* __restrict__ dmaps /*[C*3][3][OH][OW]*/, double* __restrict__ stats,
+                                                                const SsimEval ev = SsimEval{}) {
     extern __shared__ __align__(16) float ssim_smem[];
     float(*sx)[kSsimIn + 1] = reinterpret_cast<float(*)[kSsimIn + 1]>(ssim_smem);            // [42][43]
     float(*sy)[kSsimIn + 1] = sx + kSsimIn;                                                   // [42][43]
@@ -92,14 +115,48 @@ __global__ void __launch_bounds__(kSsimThreads) ssim_fwd_kernel(int W, int H, co
             float a = 0.f, b = 0.f;
             if (y < H && x < W) {
                 const int64_t pix = img + (int64_t)y * W + x, o = pix * 3 + ch;
-                a = gt.at(o) * mask.at(pix);  // pred already carries the mask (loss_grad_kernel<WRITE_PRED>)
-                b = pred[o];
+                if constexpr (EVAL) {
+                    const float4 r4 = ev.render[pix];
+                    const float rc = ch == 0 ? r4.x : (ch == 1 ? r4.y : r4.z);
+                    a = gt.at(o);
+                    b = fminf(fmaxf(rc + (1.0f - ev.alphas[pix]) * ev.bg[ch], 0.0f), 1.0f);
+                } else {
+                    a = gt.at(o) * mask.at(pix);  // pred already carries the mask (loss_grad_kernel<WRITE_PRED>)
+                    b = pred[o];
+                }
             }
             sx[r][c] = a;
             sy[r][c] = b;
         }
     }
     __syncthreads();
+    double part[kEvalPartials - 1] = {};  // EVAL: this thread's share of the partials after the SSIM sum
+    if constexpr (EVAL) {
+        // the pixels this block owns (see SsimEval)
+        const int tiles_x = gridDim.x, tiles_y = gridDim.y;
+        const int nx = (int)blockIdx.x == tiles_x - 1 ? W - ox0 : kSsimTile, ny = (int)blockIdx.y == tiles_y - 1 ? H - oy0 : kSsimTile;
+        const float fill = __int_as_float(ev.fill[cam]);
+        for (int i = threadIdx.x; i < nx * ny; i += kSsimThreads) {
+            const int r = i / nx, c = i % nx;
+            const double e = (double)sy[r][c] - (double)sx[r][c];
+            part[0] += e * e;
+            if (ch != 0) continue;
+            const int64_t pix = img + (int64_t)(oy0 + r) * W + ox0 + c;
+            const float gf = ev.gt_depth.at(pix);
+            if (!(fabsf(gf) <= 3.402823466e38f && gf > ev.depth_tol)) continue;
+            const double g = gf, d = ev.alphas[pix] > 0.0f ? ev.render[pix].w : fill;
+            const double diff = g - d, lg = log(g) - log(d);
+            const double t = fmax(g / d, d / g);
+            part[1] += 1.0;
+            part[2] += fabs(diff) / g;
+            part[3] += diff * diff / g;
+            part[4] += diff * diff;
+            part[5] += lg * lg;
+            part[6] += t < 1.25 ? 1.0 : 0.0;
+            part[7] += t < 1.25 * 1.25 ? 1.0 : 0.0;
+            part[8] += t < 1.25 * 1.25 * 1.25 ? 1.0 : 0.0;
+        }
+    }
     // horizontal pass: 42 rows x (32 / kBlkH) column groups = 168 items
     if (threadIdx.x < kSsimIn * (kSsimTile / kBlkH)) {
         const int r = threadIdx.x / (kSsimTile / kBlkH), c0 = (threadIdx.x % (kSsimTile / kBlkH)) * kBlkH;
@@ -145,22 +202,45 @@ __global__ void __launch_bounds__(kSsimThreads) ssim_fwd_kernel(int W, int H, co
                 const float inv = rcp_approx(B1) * rB2;
                 const float map = A1 * A2 * inv;
                 local_f += map;
-                float* d = dmaps + ((int64_t)blockIdx.z * 3) * plane + (int64_t)oy * OW + ox;
-                d[0] = (2.f * m1 * (A2 - A1) - 2.f * m2 * map * (B2 - B1)) * inv;  // d map / d mu2 (e2, e12 fixed)
-                d[plane] = -map * rB2;                                             // d map / d e2
-                d[2 * plane] = 2.f * A1 * inv;                                     // d map / d e12
+                if constexpr (!EVAL) {
+                    float* d = dmaps + ((int64_t)blockIdx.z * 3) * plane + (int64_t)oy * OW + ox;
+                    d[0] = (2.f * m1 * (A2 - A1) - 2.f * m2 * map * (B2 - B1)) * inv;  // d map / d mu2 (e2, e12 fixed)
+                    d[plane] = -map * rB2;                                             // d map / d e2
+                    d[2 * plane] = 2.f * A1 * inv;                                     // d map / d e12
+                }
             }
         }
     }
     double local = (double)local_f;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) local += __shfl_xor_sync(0xffffffffu, local, o);
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = local;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double s = 0;
-        for (int i = 0; i < kSsimThreads / 32; ++i) s += red[i];
-        atomicAdd(stats + cam * 8 + 5, s);
+    if constexpr (EVAL) {
+        // fixed-order block sums: xor shuffles inside each warp, then the warps in order
+        __shared__ double red_p[kSsimThreads / 32][kEvalPartials - 1];
+#pragma unroll
+        for (int k = 0; k < kEvalPartials - 1; ++k) {
+            double v = part[k];
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+            if (lane == 0) red_p[warp][k] = v;
+        }
+        if (lane == 0) red[warp] = local;
+        __syncthreads();
+        if (threadIdx.x < kEvalPartials) {
+            const int k = threadIdx.x;
+            double s = 0;
+            for (int i = 0; i < kSsimThreads / 32; ++i) s += k == 0 ? red[i] : red_p[i][k - 1];
+            const int64_t tile = (int64_t)blockIdx.y * gridDim.x + blockIdx.x;
+            ev.partials[((int64_t)blockIdx.z * gridDim.x * gridDim.y + tile) * kEvalPartials + k] = s;
+        }
+    } else {
+        if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = local;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double s = 0;
+            for (int i = 0; i < kSsimThreads / 32; ++i) s += red[i];
+            atomicAdd(stats + cam * 8 + 5, s);
+        }
     }
 }
 
@@ -248,11 +328,29 @@ int qed_ssim_launch(int C, int W, int H, const float* pred, qed::GtImage gt, qed
     if (W <= kHalo || H <= kHalo) return QED_ERR_UNSUPPORTED;
     static const GaussWin win = make_window();
     const int OW = W - kHalo, OH = H - kHalo;
-    QED_CUDA_TRY(cudaFuncSetAttribute(ssim_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSsimFwdSmem));
+    QED_CUDA_TRY(cudaFuncSetAttribute(ssim_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSsimFwdSmem));
     QED_CUDA_TRY(cudaFuncSetAttribute(ssim_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSsimBwdSmem));
     dim3 g1((OW + kSsimTile - 1) / kSsimTile, (OH + kSsimTile - 1) / kSsimTile, C * 3);
-    QED_CUDA_TRY(launch_pdl(ssim_fwd_kernel, g1, dim3(kSsimThreads), kSsimFwdSmem, stream, W, H, pred, gt, mask, win, dmaps, stats));
+    QED_CUDA_TRY(launch_pdl(ssim_fwd_kernel<false>, g1, dim3(kSsimThreads), kSsimFwdSmem, stream, W, H, pred, gt, mask, win, dmaps, stats, SsimEval{}));
     dim3 g2((W + kSsimTile - 1) / kSsimTile, (H + kSsimTile - 1) / kSsimTile, C * 3);
     QED_CUDA_TRY(launch_pdl(ssim_bwd_kernel, g2, dim3(kSsimThreads), kSsimBwdSmem, stream, W, H, pred, gt, mask, win, dmaps, scale, v_pred));
+    return QED_OK;
+}
+
+// Tiles (blocks per view and channel) of qed_ssim_eval_launch: its partials are [C*3][tiles][kEvalPartials] doubles.
+int64_t qed_ssim_eval_tiles(int W, int H) {
+    return (int64_t)((W - kHalo + kSsimTile - 1) / kSsimTile) * ((H - kHalo + kSsimTile - 1) / kSsimTile);
+}
+
+// The held-out metrics' pass (ssim_fwd_kernel<true>, see SsimEval).  Internal to qed_eval_metrics (metrics.cu), declared there.
+int qed_ssim_eval_launch(int C, int W, int H, const float* render, const float* alphas, qed::GtImage gt, qed::GtDepth gt_depth, const float* bg,
+                         const int* fill, float depth_tol, double* partials, cudaStream_t stream) {
+    if (W <= kHalo || H <= kHalo) return QED_ERR_UNSUPPORTED;
+    static const GaussWin win = make_window();
+    QED_CUDA_TRY(cudaFuncSetAttribute(ssim_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSsimFwdSmem));
+    const SsimEval ev{reinterpret_cast<const float4*>(render), alphas, bg, gt_depth, fill, depth_tol, partials};
+    dim3 g((W - kHalo + kSsimTile - 1) / kSsimTile, (H - kHalo + kSsimTile - 1) / kSsimTile, C * 3);
+    QED_CUDA_TRY(launch_pdl(ssim_fwd_kernel<true>, g, dim3(kSsimThreads), kSsimFwdSmem, stream, W, H, (const float*)nullptr, gt, PixelMask{nullptr, 0}, win,
+                            (float*)nullptr, (double*)nullptr, ev));
     return QED_OK;
 }

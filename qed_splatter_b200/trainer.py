@@ -44,6 +44,8 @@ SPLATFACTO_SHAPES = {"means": (3,), "scales": (3,), "quats": (4,), "features_dc"
 STRATEGY_STATS = ("grad2d", "count", "radii")
 # TrainConfig fields that decide which tables a state holds and their shapes: a resumed run cannot change them
 LAYOUT_FIELDS = ("strategy", "camera_optimizer", "use_bilateral_grid", "bilateral_grid_shape")
+# SplatTrainer.evaluate renders the local views at most this many at a time, so its buffers do not grow with the eval set
+EVAL_CHUNK_VIEWS = 8
 
 
 @dataclass
@@ -902,6 +904,46 @@ class SplatTrainer:
         info = self.maybe_refine(self.step_count)
         self.step_count += 1
         return loss, info
+
+    # -- evaluation ------------------------------------------------------------------------------
+    @torch.no_grad()
+    def evaluate(self, viewmats: Tensor, Ks: Tensor, width: int, height: int, gt_rgb: Tensor, gt_depth: Tensor, background: Tensor, *,
+                 depth_tolerance: float = 0.1) -> Dict[str, Tensor]:
+        """Renders this rank's held-out views as splatfacto renders outside training and scores them (metrics.image_metrics)
+        -> {name: [world_size * C] float64 device tensor} for every name of metrics.METRIC_NAMES: the rows of every rank's views,
+        rank-major (rank r's C views in slots [r C, (r + 1) C)), identical on every rank.  With world_size > 1 it is collective,
+        and every rank must pass the same number C of views.
+
+        The views are rendered at full resolution (whatever num_downscales and the step), from the poses as given (viewmats
+        [C,4,4], e.g. get_viewmat(camera_to_worlds): the camera optimizer's table is not applied), without the bilateral grid,
+        with sh_degree_to_use(), cfg.rasterize_mode and cfg.render_mode, composited on `background` [3] (splatfacto's fixed
+        colour when training uses a random one).  Ks [C,3,3]; gt_rgb / gt_depth at full resolution as for step(), depth in
+        cfg.depth_unit_scale when raw uint16.  At most EVAL_CHUNK_VIEWS views are rendered at a time.
+        No training state changes: the next step() computes exactly what it would have computed without this call, and costs
+        what it would have cost.  The views are rendered by a FusedSplatStep of their own, dropped when the call returns: the
+        step's buffers and intersection-list capacity stay sized for the training views."""
+        if self._fused is None:
+            raise RuntimeError("rendering needs the CUDA library (backend='cuda'); there is no CPU fallback")
+        from .metrics import METRIC_NAMES, metric_rows
+        from .pipeline import FusedSplatStep
+
+        c, a = self.cfg, self.arena
+        C = viewmats.shape[0]
+        if Ks.shape[0] != C or gt_rgb.shape[0] != C or gt_depth.shape[0] != C:
+            raise ValueError("viewmats, Ks, gt_rgb and gt_depth must hold the same views")
+        rows = torch.zeros(self.world * C, len(METRIC_NAMES), dtype=torch.float64, device=self.device)
+        pv = a.views(a.param)
+        fused = FusedSplatStep(self.device)
+        for c0 in range(0, C, EVAL_CHUNK_VIEWS):
+            c1 = min(c0 + EVAL_CHUNK_VIEWS, C)
+            render, alphas = fused.forward(pv["means"], pv["quats"], pv["scales"], pv["opacities"], pv["sh"], viewmats[c0:c1].contiguous(),
+                                           Ks[c0:c1].contiguous(), width, height, self.sh_degree_to_use(), render_mode=c.render_mode,
+                                           rasterize_mode=c.rasterize_mode, activations=3)  # ACT_LOG_SCALES | ACT_LOGIT_OPACITIES
+            slot = self.rank * C
+            metric_rows(render, alphas, gt_rgb[c0:c1], gt_depth[c0:c1], background, depth_unit_scale=c.depth_unit_scale,
+                        depth_tolerance=depth_tolerance, out=rows[slot + c0:slot + c1])
+        self._all_reduce(rows)  # every slot has one non-zero contributor: the sum is exact, the same bits on every rank
+        return {name: rows[:, k] for k, name in enumerate(METRIC_NAMES)}
 
     # -- checkpoints -----------------------------------------------------------------------------
     def _gather_rows(self, t: Tensor) -> Tensor:
